@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic frame windows of
 BASELINE.json configs[1] shape (15 frames x 150 detections, k=50, 12 message-passing steps):
@@ -20,6 +21,10 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+if __name__ == '__main__':
+    # a benchmark run writes nothing into the source tree it runs from, bytecode caches of the modules it imports
+    # included, so that a shared or read-only checkout stays exactly as the build left it
+    sys.dont_write_bytecode = True
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -31,9 +36,10 @@ METRIC = 'edge-updates/s'
 UNIT = 'edge-updates/s'
 NUM_STEPS_MP = 12
 NUM_CLASS_STEPS = 11
+DUMP_BYTES = 64_000_000
 
 
-def parse():
+def parse(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
     ap.add_argument('--steps', type=int, default=20)
@@ -51,7 +57,15 @@ def parse():
     ap.add_argument('--mode', default='infer', choices=['infer', 'train'],
                     help="'train': BASELINE configs[3] -- KITTI-shaped training step (fwd+bwd, 12 MP steps, 11 classified) "
                          'with one NCCL all-reduce of the flat gradient bucket + Adam; extra to the headline contract')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step returned (edge_index, edge_attr, '
+                         f'logits, pair_ptr) as DIR/<name>.npy, at most {DUMP_BYTES // 10**6} MB in all (rank 0 only)')
+    a = ap.parse_args(argv)
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if a.dump_outputs and (a.impl != 'b200' or a.mode != 'infer'):
+        ap.error('--dump-outputs records the b200 inference step only')
+    return a
 
 
 def workload_name(a):
@@ -105,10 +119,58 @@ def make_windows(a, rank, world):
     return wins
 
 
+def job_inputs(a, rank, world, dev):
+    """This rank's windows, their node offsets ``node_ptr`` and inputs: the detection table ``cols``, its page-locked
+    copy ``host`` and device copy ``devin``, both with one node-feature tensor per window (seeded by the rank)."""
+    wins = make_windows(a, rank, world)
+    gen = torch.Generator(device=dev).manual_seed(rank)
+    node_ptr = [0]
+    for w in wins:
+        node_ptr.append(node_ptr[-1] + w.N)
+    # the job's detection table: one set of columns for all windows (the way the reference holds a
+    # sequence's graph_df) + one node-feature tensor per window
+    cols = {k: torch.cat([torch.from_numpy(synth.det_columns(w)[k]) for w in wins])
+            for k in ('frame', 'bb_height', 'bb_width', 'feet_x', 'feet_y')}
+    for g in range(len(wins)):                      # one table for the job: window g owns its own frame numbers
+        cols['frame'][node_ptr[g]:node_ptr[g + 1]] += g * (a.frames + 1)
+    cols['reid'] = torch.cat([w.reid for w in wins])
+    host = {k: v.pin_memory() for k, v in cols.items()}
+    devin = {k: v.to(dev) for k, v in host.items()}
+    host['x'], devin['x'] = [], []
+    for w in wins:
+        shape = (w.N, 2048) if a.pooled else (w.N, 2048, 8, 4)
+        x = torch.randn(shape, generator=gen, device=dev).abs_()
+        devin['x'].append(x)
+        host['x'].append(x.cpu().pin_memory())
+    return wins, node_ptr, cols, host, devin
+
+
 def model_and_params():
     mp = default_graph_model_params(NUM_STEPS_MP, NUM_CLASS_STEPS)
     P = synth.make_params(mp, seed=9, gain=1.25, core_only=True)
     return mp, P
+
+
+def dump_outputs(out_dir, batch, out, budget=DUMP_BYTES):
+    """Write one step's results as ``out_dir/<name>.npy``: the graph batch's ``edge_index`` [2,E], ``edge_attr``
+    [E,F] and ``pair_ptr``, and the classifier ``logits`` [num_class_steps,E].  Indices are stored as float64
+    (exact), the rest as the float32 it was computed in.  When the files would exceed ``budget`` bytes, every
+    per-edge array keeps the same seeded sample of edges; ``edge_sample.npy`` holds the sorted edge ids kept."""
+    edge_index = batch.edge_index.cpu().numpy().astype(np.float64)
+    edge_attr = batch.edge_attr.cpu().numpy()
+    logits = out.logits.cpu().numpy()
+    pair_ptr = np.asarray(batch.pair_ptr, dtype=np.float64)
+    num_edges = edge_index.shape[1]
+    per_edge = edge_index.itemsize * 2 + edge_attr.itemsize * edge_attr.shape[1] + logits.itemsize * logits.shape[0] + 8
+    headers = 5 * 1024                  # 1 KB per file for its .npy header (128 bytes for these shapes)
+    keep = min(num_edges, max(0, (budget - headers - pair_ptr.nbytes) // per_edge))
+    sample = np.arange(num_edges) if keep == num_edges else \
+        np.sort(np.random.default_rng(0).choice(num_edges, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = dict(edge_index=edge_index[:, sample], edge_attr=edge_attr[sample], logits=logits[:, sample],
+                  pair_ptr=pair_ptr, edge_sample=sample.astype(np.float64))
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), np.ascontiguousarray(arr))
 
 
 # ------------------------------------------------------------------ reference arm (CPU)
@@ -232,27 +294,8 @@ def run_b200(a):
     model = MOTMPNet(mp).to(dev).eval()
     model.load_state_dict(P, strict=False)      # core weights; the mask branch keeps its init
 
-    wins = make_windows(a, rank, world)
-    gen = torch.Generator(device=dev).manual_seed(rank)
+    wins, node_ptr, cols, host, devin = job_inputs(a, rank, world, dev)
     fps = wins[0].fps
-    node_ptr = [0]
-    for w in wins:
-        node_ptr.append(node_ptr[-1] + w.N)
-    # the job's detection table: one set of columns for all windows (the way the reference holds a
-    # sequence's graph_df) + one node-feature tensor per window
-    cols = {k: torch.cat([torch.from_numpy(synth.det_columns(w)[k]) for w in wins])
-            for k in ('frame', 'bb_height', 'bb_width', 'feet_x', 'feet_y')}
-    for g in range(len(wins)):                      # one table for the job: window g owns its own frame numbers
-        cols['frame'][node_ptr[g]:node_ptr[g + 1]] += g * (a.frames + 1)
-    cols['reid'] = torch.cat([w.reid for w in wins])
-    host = {k: v.pin_memory() for k, v in cols.items()}
-    devin = {k: v.to(dev) for k, v in host.items()}
-    host['x'], devin['x'] = [], []
-    for w in wins:
-        shape = (w.N, 2048) if a.pooled else (w.N, 2048, 8, 4)
-        x = torch.randn(shape, generator=gen, device=dev).abs_()
-        devin['x'].append(x)
-        host['x'].append(x.cpu().pin_memory())
     h2d_bytes = sum(t.numel() * t.element_size() for k, t in host.items() if k != 'x') + \
         sum(t.numel() * t.element_size() for t in host['x'])
 
@@ -374,11 +417,10 @@ def run_b200(a):
             dist.barrier()
             torch.cuda.synchronize()
 
+    # every loop keeps its last step's result alive, so the timed loop runs with the memory pool the warmup left
     for _ in range(a.warmup):
-        batch, _ = step(devin)
+        last = step(devin)
     torch.cuda.synchronize()
-    edges = batch.num_edges
-    nodes = batch.num_nodes
 
     # ---- timed region: device-resident inputs (Python's cyclic GC is paused: a gen-2 collection inside
     #      a 7 ms step shows up as a 20-40 ms outlier)
@@ -392,10 +434,12 @@ def run_b200(a):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(a.steps):
-        step(devin)
+        last = step(devin)
     ev1.record()
     sync_all()
     ms = ev0.elapsed_time(ev1)
+    edges = last[0].num_edges
+    nodes = last[0].num_nodes
     launches = lib.mpn_launch_count() - launches0
     import ctypes as C
     prof_ms = (C.c_double * 2)()
@@ -437,6 +481,8 @@ def run_b200(a):
         sync_all()
         ms_raw = t0.elapsed_time(t1)
     gc.enable()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, *last)
 
     from mpntrackseg_b200.sharding import reduce_step_stats
     ms, (all_edges, all_nodes, h2d_total, d2h_total, h2d_raw_total) = reduce_step_stats(

@@ -3,11 +3,18 @@ tests (readers, need only the committed .npz files).  Inputs and weights are reg
 from seeds through mpntrackseg_b200.synth; fixtures hold the reference's outputs."""
 import hashlib
 import os
+import zipfile
 
 import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+
+# fixtures that would be larger than 1 MB as plain .npz files; make_golden.py writes them with save_compact
+COMPACT = ('config1', 'kitti_shape', 'config5')
+# graph arrays of a compact fixture are stored as digests: the oracle rebuilds them bit for bit from the seeded inputs
+GRAPH_KEYS = ('edge_index', 'edge_attr', 'edge_attr_sample')
+_GRAPHS = {}
 
 CASES = {
     # name: window kwargs, dataset kwargs, model steps, weight seed/gain, extras
@@ -67,16 +74,63 @@ def checksum(*tensors):
     return h.hexdigest()
 
 
+def save_compact(path, **arrays):
+    """``np.savez_compressed`` for the COMPACT fixtures, without dropping anything.  A graph array (GRAPH_KEYS) is
+    stored as the SHA-256 of the reference's array (``<key>__sha256``); the loaders rebuild it with the oracle and
+    require the same digest.  A float32 array is stored as its four byte planes (``<key>__planes``, uint8
+    [4, *shape]), which LZMA compresses much better than interleaved bytes."""
+    with zipfile.ZipFile(path, 'w', zipfile.ZIP_LZMA) as zf:
+        for key, a in arrays.items():
+            a = np.asarray(a)
+            if key in GRAPH_KEYS:
+                key, a = f'{key}__sha256', np.array(checksum(a))
+            elif a.dtype == np.float32 and a.ndim:
+                key, a = f'{key}__planes', np.moveaxis(np.ascontiguousarray(a)[..., None].view(np.uint8), -1, 0)
+            with zf.open(f'{key}.npy', 'w') as f:
+                np.lib.format.write_array(f, a)
+
+
+def _load_gold(name):
+    """The arrays of ``<name>.npz``, float32 byte planes (see save_compact) joined back."""
+    gold = {}
+    with np.load(os.path.join(HERE, f'{name}.npz')) as z:
+        for key in z.files:
+            if key.endswith('__planes'):
+                gold[key[:-8]] = np.ascontiguousarray(np.moveaxis(z[key], 0, -1)).view(np.float32)[..., 0]
+            else:
+                gold[key] = z[key]
+    return gold
+
+
+def _rebuild_graph(name, gold, win, ds, max_frame_dist):
+    """Replace the ``<key>__sha256`` entries of a compact fixture by the oracle's graph arrays, which must have the
+    reference's digests (the oracle builds the graph with the reference's own torch ops, bit for bit)."""
+    for key in [k for k in gold if k.endswith('__sha256')]:
+        if name not in _GRAPHS:
+            from mpntrackseg_b200 import synth
+            from oracle import graph_ref
+            g = graph_ref.build_graph(win.frame, win.reid, synth.det_columns(win), win.fps, ds, inference_mode=False,
+                                      max_frame_dist=max_frame_dist)
+            ea = g['edge_attr'].numpy()
+            # dtypes and the feature sample stride as make_golden.py stores them
+            _GRAPHS[name] = dict(edge_index=g['edge_index'].numpy().astype(np.int32), edge_attr=ea,
+                                 edge_attr_sample=ea[::16])
+        arr = _GRAPHS[name][key[:-8]].copy()
+        assert checksum(arr) == str(gold.pop(key)), f"{name}: the oracle's {key[:-8]} differs from the reference's"
+        gold[key[:-8]] = arr
+
+
 def load_case(name):
     """Rebuild the seeded inputs / weights of a golden case and load its reference outputs."""
     from mpntrackseg_b200 import synth
     from mpntrackseg_b200.config import default_dataset_params, default_graph_model_params
     c = TRACKER_CASE if name == 'tracker_window' else CASES[name]
-    gold = dict(np.load(os.path.join(HERE, f'{name}.npz')))
+    gold = _load_gold(name)
     win = synth.make_window(**c['win'])
     assert checksum(win.frame, win.reid, win.x, win.bb_height, win.feet_x) == str(gold['input_checksum']), \
         'seeded inputs differ from the ones the fixture was generated with'
     ds = default_dataset_params(**c['ds'])
+    _rebuild_graph(name, gold, win, ds, c.get('max_frame_dist', 'max'))
     mp = case_model_params(c)
     P = synth.make_params(mp, seed=c['wseed'], gain=c['gain'])
     key = [k for k in P if k.startswith('classifier.edge_model') and k.endswith('bias')][-1]
@@ -91,12 +145,13 @@ def load_big_case(name):
     from mpntrackseg_b200 import synth
     from mpntrackseg_b200.config import default_dataset_params, default_graph_model_params
     c = BIG_CASES[name]
-    gold = dict(np.load(os.path.join(HERE, f'{name}.npz')))
+    gold = _load_gold(name)
     win = synth.make_window(**c['win'])
     ds = default_dataset_params(**c['ds'])
     out = dict(case=c, win=win, ds=ds, gold=gold)
     if 'steps' in c:
         assert checksum(win.frame, win.reid, win.x, win.bb_height, win.feet_x) == str(gold['input_checksum'])
+        _rebuild_graph(name, gold, win, ds, 'max')
         mp = default_graph_model_params(*c['steps'])
         P = synth.make_params(mp, seed=c['wseed'], gain=c['gain'])
         key = [k for k in P if k.startswith('classifier.edge_model') and k.endswith('bias')][-1]

@@ -35,7 +35,7 @@ from mot_neural_solver.utils.graph import (  # noqa: E402
 from mpntrackseg_b200 import synth  # noqa: E402
 from mpntrackseg_b200.config import default_dataset_params, default_graph_model_params  # noqa: E402
 
-from cases import BIG_CASES, CASES, TRACKER_CASE, case_model_params, checksum  # noqa: E402
+from cases import BIG_CASES, CASES, COMPACT, TRACKER_CASE, case_model_params, checksum, save_compact  # noqa: E402
 
 
 def det_df(win):
@@ -146,7 +146,7 @@ def run_case(name, c):
                  logit_std=float(logits[-1].std()) if logits.numel() else 0.0,
                  frac_pos=float((logits[-1] > 0).float().mean()) if logits.numel() else 0.0)
     print(name, stats)
-    np.savez_compressed(os.path.join(HERE, f'{name}.npz'), **out)
+    (save_compact if name in COMPACT else np.savez_compressed)(os.path.join(HERE, f'{name}.npz'), **out)
 
 
 def run_tracker_case():
@@ -336,12 +336,12 @@ def run_config5_case():
     logits = torch.stack([t.view(-1) for t in core['classified_edges']])
     print('config5', dict(N=win.N, E=edge_index.shape[1], cand=n_cand, logit_std=float(logits[-1].std()),
                           frac_pos=float((logits[-1] > 0).float().mean()), node_max=float(core['node_state'].max())))
-    np.savez_compressed(os.path.join(HERE, 'config5.npz'), n_candidates=np.int64(n_cand),
-                        edge_index=edge_index.numpy().astype(np.int32), edge_attr_sample=edge_attr[::16].numpy(),
-                        logits_last=logits[-1].numpy(), logits_first=logits[0].numpy(),
-                        logits_step_means=logits.double().mean(dim=1).numpy(), bias_shift=np.float64(shift),
-                        input_checksum=checksum(win.frame, win.reid, win.x, win.bb_height, win.feet_x),
-                        param_checksum=checksum(*P.values()))
+    save_compact(os.path.join(HERE, 'config5.npz'), n_candidates=np.int64(n_cand),
+                 edge_index=edge_index.numpy().astype(np.int32), edge_attr_sample=edge_attr[::16].numpy(),
+                 logits_last=logits[-1].numpy(), logits_first=logits[0].numpy(),
+                 logits_step_means=logits.double().mean(dim=1).numpy(), bias_shift=np.float64(shift),
+                 input_checksum=checksum(win.frame, win.reid, win.x, win.bb_height, win.feet_x),
+                 param_checksum=checksum(*P.values()))
 
 
 def run_big_window_case():
