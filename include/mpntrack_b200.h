@@ -296,8 +296,10 @@ int mpn_adam_step_dev(float* params, const float* grads, float* exp_avg, float* 
  * Range: step t runs on operands scaled by 2^-s_t, s_t chosen on the device from the previous step's largest
  * activation and the growth of the node state (exact power-of-two scaling of a piecewise-linear network;
  * s_t = 0 while values stay below 64), so node states far beyond the fp16 range stay on this path.
- * *status (device int32) is set non-zero only if a value still left the fp16 range (one-step growth beyond the
- * 1024x headroom); the outputs are then invalid and the caller must rerun with mpn_mp_forward (fp32 kernels).
+ * *status (device int32) is set non-zero only if a value still left the fp16 range (bit 1: one-step growth beyond the
+ * 1024x headroom) or a step ran at s_t > 17, where the absolute resolution 2^(s_t-34) no longer resolves rows of
+ * order 1, e.g. a quiet window batched with a loud one (bit 2); the outputs are then invalid and the caller must
+ * rerun with mpn_mp_forward (fp32 kernels).
  * workspace bytes: mpn_mp_tc_workspace(N, E). */
 int64_t mpn_mp_tc_workspace(int64_t num_nodes, int64_t num_edges);
 int mpn_mp_forward_tc(const mpn_core_weights* h_w, const mpn_edge_layout* h_g, const float* x_init,

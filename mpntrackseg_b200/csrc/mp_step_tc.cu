@@ -75,6 +75,12 @@ constexpr float SCALE_TARGET = 64.f;
 constexpr int INIT_SHIFT = 8;                // the constant x_init / e_init rows are stored x 2^-8, their weight slabs carry 2^(8 - s_t):
                                              // the slabs stay normal fp16 numbers for s_t up to 22 (values up to ~2.7e8); beyond that the
                                              // constant-row terms fade out (they are < 2^-22 of the latent terms there)
+// Resolution floor: a value carried as v x 2^-s keeps 22 bits only while its high half is a normal fp16 number; below
+// that both halves are subnormal and the absolute resolution is 2^(s - 34), the same for every row of the batch.  Above
+// s = 17 that floor, carried through the recurrence, reaches the 1e-3 parity bar for rows whose own values are of
+// order 1 (a quiet window batched with a loud one: its logit error triples at s = 19 and is 7x the bar at s = 22, on
+// a B200).  Such a step sets status bit 2, which sends engine 'auto' to the fp32 kernels like an fp16 overflow.
+constexpr int S_RESOLVED = 17;
 constexpr int FLOW_SHIFT = 7;                // a flow vector sums up to ~100 messages: operand scale 2^-(s_t + 7)
 __device__ __forceinline__ float pow2i(int e) { return __int_as_float((127 + e) << 23); }   // 2^e, |e| <= 126
 // s_{t+1} from what is known when the node kernel of step t starts: the edge kernel's activation maximum of step t
@@ -796,9 +802,9 @@ __global__ void __launch_bounds__(NTHREADS3, 1) mp_edge_tc3_kernel(TcArgs a, con
       dst[i] = v;
     }
     // s_cur > INIT_SHIFT + 14: the slab factor 2^(INIT_SHIFT - s) is a subnormal fp16 number (or 0 beyond 2^-24) and the
-    // constant-row terms lose bits / vanish -- by then the latent operands are > 2^22 times larger than the constant
-    // rows, so what is lost is below 1e-6 of the accumulators
+    // constant-row terms lose bits / vanish; such steps are already flagged by S_RESOLVED
   }
+  if (s_cur > S_RESOLVED && blockIdx.x == 0 && tid == 0) atomicOr(a.status, 2);
   if (tid == 0) {
     for (int i = 0; i < NG3; ++i) { mbar_init(&bars[i], 1); mbar_init(&bars[NG3 + i], 4); }
     mbar_fence_init();

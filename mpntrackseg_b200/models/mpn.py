@@ -463,9 +463,11 @@ class MOTMPNet(nn.Module):
             if not any(flags):
                 break
             if eng == 'tc':
-                raise OverflowError('a value left the fp16 range on the tensor-core path; use engine="fp32"')
+                raise OverflowError('a value left the fp16 range on the tensor-core path, or the step scale passed the '
+                                    'split operands\' resolution; use engine="fp32"')
             import warnings
-            warnings.warn('mpntrackseg_b200: value outside the fp16 range, rerunning the forward on the fp32 kernels')
+            warnings.warn('mpntrackseg_b200: value outside the fp16 range (or step scale beyond the split operands\' '
+                          'resolution), rerunning the forward on the fp32 kernels')
         del keep
         return res
 

@@ -346,7 +346,8 @@ def mp_forward(cw, layout, x_init, e_init, num_steps, first_class_step, want_sta
 
     engine: 'tc' = tcgen05 tensor-core kernels (fp16 hi/lo split operands in a per-step power-of-two
     scale, fp32 accumulate), 'fp32' = fp32 SIMT kernels, 'auto' (default) = 'tc', rerun on 'fp32' if an
-    activation still left the fp16 range (one-step growth beyond the 1024x headroom of the scale).  status: optional int32[1] device tensor: the overflow flag is left there for the
+    activation still left the fp16 range (one-step growth beyond the 1024x headroom of the scale) or a step's scale
+    passed 2^17, beyond which rows of order 1 -- a quiet window batched with a loud one -- lose the parity bar.  status: optional int32[1] device tensor: the overflow flag is left there for the
     caller (no host sync, no fallback here)."""
     engine = engine or default_engine()
     x_init = _req(x_init, torch.float32, 'x_init')
@@ -377,9 +378,10 @@ def mp_forward(cw, layout, x_init, e_init, num_steps, first_class_step, want_sta
         if int(status.item()) == 0:
             return (logits, x_out, e_out) if want_state else logits
         if engine == 'tc':
-            raise OverflowError('mp_forward_tc: an activation left the fp16 range; use engine="fp32"')
-        warnings.warn('mpntrackseg_b200: activation outside the fp16 range, rerunning the message-passing '
-                      'steps on the fp32 kernels')
+            raise OverflowError('mp_forward_tc: an activation left the fp16 range, or the step scale passed the split '
+                                'operands\' resolution; use engine="fp32"')
+        warnings.warn('mpntrackseg_b200: activation outside the fp16 range (or step scale beyond the split operands\' '
+                      'resolution), rerunning the message-passing steps on the fp32 kernels')
     ws = _bytes(lib().mpn_mp_workspace(n, e), dev)
     check(lib().mpn_mp_forward(C.byref(cw), C.byref(g), ptr(x_init), ptr(e_init), int(num_steps), int(first),
                                ptr(ws), ptr(logits), ptr(x_out), ptr(e_out), stream_ptr()), 'mp_forward')

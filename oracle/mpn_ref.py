@@ -160,10 +160,16 @@ def mpn_forward(P, model_params, x, edge_index, edge_attr, x_ext=None, return_st
     """MOTMPNet.forward.  With ``x_ext=None`` only the core path (the one the edge
     logits depend on) is evaluated and 'mask_predictions' stays empty.
     reference: models/mpn.py:333-394"""
+    x0, e0 = encode(P, x, edge_attr)
+    return mp_steps(P, model_params, x0, e0, edge_index, x_ext=x_ext, return_state=return_state)
+
+
+def mp_steps(P, model_params, x0, e0, edge_index, x_ext=None, return_state=False):
+    """The step loop of ``mpn_forward`` from the encoded node / edge states ``x0`` [N, dn], ``e0`` [E, de]
+    (edges in the caller's order).  reference: models/mpn.py:356-394"""
     steps = model_params['num_enc_steps']
     first_cls = steps - model_params['num_class_steps'] + 1
     agg = model_params['node_agg_fn']
-    x0, e0 = encode(P, x, edge_attr)
     xs, es = x0, e0
     ext = x_ext is not None
     if ext:

@@ -488,7 +488,8 @@ def test_tc_engine_scales_activations_beyond_the_fp16_range():
 def test_bench_workload_stays_on_the_tensor_core_path():
     """bench.py's windows (seeds 0..127 = what 8 ranks x 16 windows evaluate) with bench.py's weights run through
     engine='tc' without the fp16-range status (round 1 fell back to the fp32 kernels on seed 80: node state
-    7.5e4 after 12 steps); seed 80 is also checked against the oracle."""
+    7.5e4 after 12 steps); all 16 windows of the batch that starts at seed 80 are checked against the fp64 oracle, each
+    having run under the per-step scale its batch chose."""
     from mpntrackseg_b200.data.mot_graph import build_window_graphs
     ds = default_dataset_params(top_k_nns=50, frames_per_graph=15)
     mp = default_graph_model_params(12, 11)
@@ -508,14 +509,18 @@ def test_bench_workload_stays_on_the_tensor_core_path():
             out = model.forward_batch(batch)                             # engine='tc' raises OverflowError on status != 0
         assert torch.isfinite(out.logits).all()
         if lo == 80:
-            w, x = wins[0], tabs[0]['x'].cpu()
-            ref_g = graph_ref.build_graph(w.frame, w.reid, synth.det_columns(w), w.fps, ds)
-            with torch.no_grad():
-                ref = mpn_ref.mpn_forward(P, mp, x, ref_g['edge_index'], ref_g['edge_attr'], return_state=True)
-            assert float(ref['node_state'].max()) > 65504.0
-            got = out.graph_logits(0).cpu().numpy()
-            exp = torch.stack([t.view(-1) for t in ref['classified_edges']]).numpy()
-            assert_logits_close(got, exp, 'bench seed 80')
+            # every window of the batch ran under the batch's per-step scale, chosen for the largest of them
+            P64 = {k: v.double() for k, v in P.items()}
+            for i, w in enumerate(wins):
+                ref_g = graph_ref.build_graph(w.frame, w.reid, synth.det_columns(w), w.fps, ds)
+                with torch.no_grad():
+                    ref = mpn_ref.mpn_forward(P64, mp, tabs[i]['x'].cpu().double(), ref_g['edge_index'],
+                                              ref_g['edge_attr'].double(), return_state=True)
+                if i == 0:
+                    assert float(ref['node_state'].max()) > 65504.0
+                got = out.graph_logits(i).cpu().numpy()
+                exp = torch.stack([t.view(-1) for t in ref['classified_edges']]).numpy()
+                assert_logits_close(got, exp, f'bench seed {80 + i}')
 
 
 def test_tc_engine_reports_fp16_overflow_and_auto_falls_back():
@@ -663,11 +668,16 @@ def test_attn_aggregate_against_oracle_softmax():
 
 
 def test_node_encoder_tc_against_fp32():
+    """Also beyond one 128-node tile per CTA (n > 2 * SMs * 128: the mbarrier parities and the TMA weight stream carry
+    over to the next tile), with an odd number of 64-wide K chunks (k0 = 192)."""
     from mpntrackseg_b200 import ops
     g = torch.Generator().manual_seed(12)
-    for n in (1, 127, 300, 2250):
-        x = torch.randn(n, 2048, generator=g).abs()
-        w0, b0 = torch.randn(128, 2048, generator=g) / 45, torch.randn(128, generator=g) * 0.1
+    t = 2 * torch.cuda.get_device_properties(0).multi_processor_count * 128
+    cases = [(n, 2048) for n in (1, 127, 300, 2250)] + [(t + 1, 64), (t + 1, 192), (t + 1, 2048), (5 * t // 2 + 3, 64),
+                                                        (5 * t // 2 + 3, 192)]
+    for n, k0 in cases:
+        x = torch.randn(n, k0, generator=g).abs()
+        w0, b0 = torch.randn(128, k0, generator=g) / (k0 ** 0.5), torch.randn(128, generator=g) * 0.1
         w1, b1 = torch.randn(32, 128, generator=g) / 11, torch.randn(32, generator=g) * 0.1
         ref = torch.relu(torch.nn.functional.linear(torch.relu(torch.nn.functional.linear(x.double(), w0.double(), b0.double())),
                                                     w1.double(), b1.double())).float()
@@ -676,7 +686,8 @@ def test_node_encoder_tc_against_fp32():
         got_32 = ops.node_encoder(*args, engine='fp32').cpu()
         scale = float(ref.abs().max())
         assert float((got_32 - ref).abs().max()) <= 2e-5 * scale
-        assert float((got_tc - ref).abs().max()) <= 2e-5 * scale, n
+        assert float((got_tc - ref).abs().max()) <= 2e-5 * scale, (n, k0)
+    assert max(n for n, _ in cases) > 2 * t
 
 
 def test_weighted_bce_loss_and_gradient_against_oracle():
