@@ -120,8 +120,12 @@ int mpn_edge_feats_assemble(const int64_t* row, const int64_t* col, int64_t num_
  * use_tensor_cores != 0 (and dim a multiple of 64, top_k >= 0): the dense distances come from a tcgen05 Gram
  * contraction (fp16 hi/lo split) and only pre-rank; rows whose k-th / (k+1)-th neighbours lie within the error
  * band are recomputed with the exact fp32 formula and re-ranked, and the distances returned for the kept pairs
- * are always the exact ones -- the kept edge set equals the exact path's.  h_stats (host, may be NULL):
- * [0] = 1 if the tensor-core path ran, [1] = number of rows that needed the exact repair.
+ * are always the exact ones -- the kept edge set equals the exact path's at every embedding scale (each window is
+ * packed under a power-of-two pre-scale, so the band bounds the Gram error).  h_stats (host, may be NULL):
+ * [0] = the build that ran: 0 exact fp32 (also after a whole-call exact rerun: values of magnitude >= 65,000 or
+ * more flagged rows than scratch slots), 1 dense Gram blocks + fused row select, 2 thresholded candidate lists,
+ * 3 dense Gram blocks + general select (windows above 5,120 nodes); nonzero = tensor cores.
+ * [1] = number of rows that needed the exact repair.
  * workspace: mpn_knn_graph_workspace(N, sum_g N_g^2, G) bytes (dense fp32 distance blocks + packed embeddings). */
 int64_t mpn_knn_graph_workspace(int64_t num_nodes, int64_t sum_sq_nodes, int64_t num_graphs);
 int mpn_knn_graph_pairs(const int64_t* frame_num, const int64_t* node_graph_ptr,

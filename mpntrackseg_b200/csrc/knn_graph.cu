@@ -208,10 +208,12 @@ __global__ void knn_pairs_kernel(const float* __restrict__ dense, const int64_t*
       if (ok) {
         d = D[li * n + lj];
         if (prune) {
-          const uint32_t key = order_key_f(d);
+          // each row against its own threshold with its own entry: after the tensor-core repair a repaired row holds
+          // exact distances while its mirror entries in the other rows stay approximate
+          const uint32_t key = order_key_f(d), key_t = order_key_f(D[lj * n + li]);
           const bool a = key < ki || (key == ki && lj <= ti);
           const uint32_t kj = thr_key[n0 + lj];
-          const bool b = key < kj || (key == kj && li <= thr_idx[n0 + lj]);   // D is symmetric
+          const bool b = key_t < kj || (key_t == kj && li <= thr_idx[n0 + lj]);
           ok = reciprocal ? (a && b) : (a || b);
         }
       }
@@ -241,7 +243,7 @@ __global__ void __launch_bounds__(SEL_THREADS) row_select_kernel(
     const float* __restrict__ dense, const int64_t* __restrict__ gptr, int64_t num_graphs, const int64_t* __restrict__ doff,
     const int64_t* __restrict__ moff, int64_t k, const int32_t* __restrict__ row_mask, uint32_t* __restrict__ thr_key,
     int32_t* __restrict__ thr_idx, uint32_t* __restrict__ M, const float* __restrict__ norm2,
-    const float* __restrict__ win_nmax, float beta, int32_t* __restrict__ amb, int32_t* __restrict__ amb_count,
+    const float* __restrict__ win_nmax, float beta, float keps, int32_t* __restrict__ amb, int32_t* __restrict__ amb_count,
     int64_t scratch_ld, int64_t scratch_rows) {
   __shared__ int hist[256];
   __shared__ uint32_t s_prefix;
@@ -355,7 +357,7 @@ __global__ void __launch_bounds__(SEL_THREADS) row_select_kernel(
         const uint32_t u = (tau & 0x80000000u) ? (tau & 0x7fffffffu) : ~tau;
         const float vk = __uint_as_float(u);
         if (isfinite(vk) && isfinite(mn)) {
-          const float band = beta * (norm2[i] + win_nmax[lo]);            // absolute error bound on d^2
+          const float band = beta * (norm2[i] + win_nmax[lo] + keps);     // absolute error bound on d^2
           flag = (mn - vk) <= 2.f * band ? 1 : 0;                         // the approximate rows hold d^2
         }
       }
@@ -368,12 +370,12 @@ __global__ void __launch_bounds__(SEL_THREADS) row_select_kernel(
 template <bool kAmb>
 static void launch_row_select(int64_t max_n, int64_t n, cudaStream_t s, const float* dense, const int64_t* gptr, int64_t num_graphs,
                               const int64_t* doff, const int64_t* moff, int64_t k, const int32_t* row_mask, uint32_t* thr_key,
-                              int32_t* thr_idx, uint32_t* M, const float* norm2, const float* win_nmax, float beta, int32_t* amb,
-                              int32_t* amb_count, int64_t scratch_ld = 0, int64_t scratch_rows = 0) {
+                              int32_t* thr_idx, uint32_t* M, const float* norm2, const float* win_nmax, float beta, float keps,
+                              int32_t* amb, int32_t* amb_count, int64_t scratch_ld = 0, int64_t scratch_rows = 0) {
   const unsigned g = (unsigned)n;
 #define MPN_SEL(PER)                                                                                                     \
   row_select_kernel<kAmb, PER><<<g, SEL_THREADS, 0, s>>>(dense, gptr, num_graphs, doff, moff, k, row_mask, thr_key, thr_idx, M, \
-                                                         norm2, win_nmax, beta, amb, amb_count, scratch_ld, scratch_rows)
+                                                         norm2, win_nmax, beta, keps, amb, amb_count, scratch_ld, scratch_rows)
   if (max_n <= 5 * SEL_THREADS) MPN_SEL(5);
   else if (max_n <= 9 * SEL_THREADS) MPN_SEL(9);
   else if (max_n <= 12 * SEL_THREADS) MPN_SEL(12);
@@ -496,6 +498,7 @@ __global__ void graph_pair_ptr_kernel(const int64_t* __restrict__ gptr, int64_t 
 }
 
 int64_t gram_workspace_bytes(int64_t num_nodes, int64_t total_tiles, int64_t num_graphs, int64_t dim);
+float gram_band_keps(int64_t dim);
 int gram_dist_blocks(const float* reid, int64_t dim, const int64_t* frame, const int64_t* gptr, const int64_t* h_gptr,
                      int64_t num_graphs, const int64_t* doff, int64_t max_dist, void* ws, float* dense,
                      int32_t* status, float** norm2_out, int32_t** amb_out, int32_t** amb_count_out, int squared,
@@ -589,7 +592,7 @@ int mpn_knn_graph_pairs(const int64_t* frame, const int64_t* gptr, const int64_t
                             amb_count, 0, max_n, scratch_rows, s);
     if (rc) return rc;
     launch_row_select<false>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, amb, tk, ti, M, nullptr, nullptr, 0.f,
-                             nullptr, nullptr, max_n, scratch_rows);
+                             0.f, nullptr, nullptr, max_n, scratch_rows);
   } else if (tc) {
     rc = gram_dist_blocks(reid, dim, frame, gptr, h_gptr, num_graphs, doff, max_frame_dist,
                           static_cast<char*>(ws) + cv.off, dense, status, &norm2, &amb, &amb_count,
@@ -609,16 +612,16 @@ int mpn_knn_graph_pairs(const int64_t* frame, const int64_t* gptr, const int64_t
     } else if (tc) {
       window_max_kernel<<<(unsigned)num_graphs, 256, 0, s>>>(norm2, gptr, win_nmax); count_launch();
       launch_row_select<true>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, nullptr, tk, ti, M, norm2, win_nmax, 2e-6f,
-                              amb, amb_count);
+                              gram_band_keps(dim), amb, amb_count);
       // rows whose top-k set is not certain: exact fp32 distances, ranked again
       rc = gram_fix_ambiguous(reid, dim, frame, gptr, num_graphs, n, doff, max_frame_dist, dense, norm2, tk, ti, 2e-6f,
                               amb, amb_count, 0, 0, 0, s);
       if (rc) return rc;
       launch_row_select<false>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, amb, tk, ti, M, nullptr, nullptr, 0.f,
-                               nullptr, nullptr);
+                               0.f, nullptr, nullptr);
     } else {
       launch_row_select<false>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, nullptr, tk, ti, M, nullptr, nullptr, 0.f,
-                               nullptr, nullptr);
+                               0.f, nullptr, nullptr);
     }
     const int64_t max_words = (max_n + 31) >> 5;
     const unsigned tgrid = (unsigned)std::min<int64_t>(std::max<int64_t>(ceil_div(max_words * max_words * 32, 256), 1), 4096);
@@ -652,7 +655,8 @@ int mpn_knn_graph_pairs(const int64_t* frame, const int64_t* gptr, const int64_t
   if (tc && h_flags[0] != 0)                                        // embeddings beyond the fp16 range: exact kernel
     return mpn_knn_graph_pairs(frame, gptr, h_gptr, num_graphs, reid, dim, top_k, reciprocal, max_frame_dist, 0, ws,
                                capacity, out_row, out_col, out_dist, graph_pair_ptr, h_graph_pair_ptr, h_stats, stream);
-  if (h_stats != nullptr) { h_stats[0] = tc ? 1 : 0; h_stats[1] = h_flags[1]; }
+  // build code: 0 exact, 1 dense Gram + fused row select, 2 thresholded candidate lists, 3 dense Gram + general select
+  if (h_stats != nullptr) { h_stats[0] = tg ? 2 : (tc ? (fused ? 1 : 3) : 0); h_stats[1] = h_flags[1]; }
   const int64_t total = h_graph_pair_ptr[num_graphs];
   if (total > capacity) {
     set_error("knn_graph_pairs: %lld pairs exceed the output capacity %lld", (long long)total, (long long)capacity);

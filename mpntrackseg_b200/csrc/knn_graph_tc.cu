@@ -5,6 +5,10 @@
 // the exact fp32 formula of the reference (same kernel arithmetic as knn_graph.cu) and re-ranked, and the
 // distances attached to the kept pairs are always recomputed exactly.  The kept edge set is therefore the
 // one the exact path produces.
+// The band, beta * (||a_i||^2 + max_window ||a||^2 + K eps^2), is relative to the window's largest squared norm.
+// The split's error is relative too only while the values sit high in the fp16 range: below 2^-3 the low half
+// is subnormal and its error an absolute 2^-25.  So every window is packed times 2^p, p chosen from its largest
+// |v| (pack_shift), and the Gram result is multiplied by 2^-2p, both exact (DESIGN.md section 4).
 #include <limits.h>
 #include <math.h>
 #include <stdlib.h>
@@ -25,11 +29,40 @@ __device__ __forceinline__ int slab_off(int n, int k16) {
   return (n >> 3) * 256 + (k16 >> 3) * 128 + (n & 7) * 16 + (k16 & 7) * 2;
 }
 
-// warp per node: packed fp16 hi/lo image of its row inside its 128-row tile, ||a||^2 and sum(a).
+// Power-of-two pre-scale of a window whose largest |v| is `amax_bits` (fp32 bits): 2^p * max |v| lies in
+// [2^13, 2^14), so every split operand keeps a resolution of 2^-25 relative to 2^13 ... 2^14 of the window's
+// largest value, and hi stays far from the fp16 maximum.  |p| <= 62 keeps 2^-2p a normal fp32 number.
+constexpr int PACK_SHIFT_MAX = 62;
+__device__ __forceinline__ int pack_shift(uint32_t amax_bits) {
+  const float m = __uint_as_float(amax_bits);
+  if (!(m > 0.f) || !isfinite(m)) return 0;                      // all-zero window (or an overflow the caller reruns)
+  int e;
+  frexpf(m, &e);                                                 // m in [2^(e-1), 2^e)
+  return max(-PACK_SHIFT_MAX, min(PACK_SHIFT_MAX, 14 - e));
+}
+
+// warp per node: max |v| of its row into its window's entry (non-negative floats order like their bits).
+__global__ void window_absmax_kernel(const float* __restrict__ reid, int64_t dim, const int64_t* __restrict__ gptr,
+                                     int64_t num_graphs, int64_t num_nodes, uint32_t* __restrict__ win_amax) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t i = warp; i < num_nodes; i += nwarps) {
+    int64_t lo = 0, hi = num_graphs;
+    while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
+    float m = 0.f;
+    for (int64_t k = lane; k < dim; k += 32) m = fmaxf(m, fabsf(reid[i * dim + k]));
+    for (int d = 16; d > 0; d >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, d));
+    if (lane == 0) atomicMax(&win_amax[lo], __float_as_uint(m));
+  }
+}
+
+// warp per node: packed fp16 hi/lo image of its row (times 2^p of its window) inside its 128-row tile, ||a||^2 and
+// sum(a) (unscaled).
 __global__ void pack_reid_kernel(const float* __restrict__ reid, int64_t dim, const int64_t* __restrict__ gptr,
                                  int64_t num_graphs, const int64_t* __restrict__ tile_off, int64_t num_nodes,
-                                 uint8_t* __restrict__ img, float* __restrict__ norm2, float* __restrict__ sum1,
-                                 int32_t* __restrict__ status) {
+                                 const uint32_t* __restrict__ win_amax, uint8_t* __restrict__ img,
+                                 float* __restrict__ norm2, float* __restrict__ sum1, int32_t* __restrict__ status) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -40,14 +73,16 @@ __global__ void pack_reid_kernel(const float* __restrict__ reid, int64_t dim, co
     const int64_t li = i - gptr[lo];
     const int64_t tile = tile_off[lo] + li / TS;
     const int n = (int)(li % TS);
+    const float up = ldexpf(1.f, pack_shift(win_amax[lo]));
     float s2 = 0.f, s1 = 0.f;
     bool ovf = false;
     for (int64_t k = lane; k < dim; k += 32) {
       const float v = reid[i * dim + k];
-      ovf |= !(fabsf(v) < 65000.f);                              // outside the fp16 range: the caller reruns exactly
+      ovf |= !(fabsf(v) < 65000.f);                              // outside the build's range (or NaN): the caller reruns exactly
       s2 = fmaf(v, v, s2);
       s1 += v;
-      const __half h = __float2half_rn(v), l = __float2half_rn(v - __half2float(h));
+      const float vs = v * up;
+      const __half h = __float2half_rn(vs), l = __float2half_rn(vs - __half2float(h));
       uint8_t* base = img + (tile * nchunks + k / KC) * CHUNK_BYTES + ((k % KC) >> 4) * SLAB + slab_off(n, (int)(k & 15));
       *reinterpret_cast<__half*>(base) = h;
       *reinterpret_cast<__half*>(base + (KC / 16) * SLAB) = l;
@@ -68,7 +103,7 @@ __device__ __forceinline__ uint32_t okey(float f) {
 __global__ void __launch_bounds__(256) row_ambiguity_kernel(const float* __restrict__ dense, const int64_t* __restrict__ gptr,
                                                             int64_t num_graphs, const int64_t* __restrict__ doff,
                                                             const float* __restrict__ norm2, const uint32_t* __restrict__ thr_key,
-                                                            const int32_t* __restrict__ thr_idx, float beta,
+                                                            const int32_t* __restrict__ thr_idx, float beta, float keps,
                                                             int32_t* __restrict__ amb, int32_t* __restrict__ amb_count) {
   __shared__ float s_min[8];
   __shared__ float s_nmax[8];
@@ -98,7 +133,7 @@ __global__ void __launch_bounds__(256) row_ambiguity_kernel(const float* __restr
     const float vk = __uint_as_float(u);
     int flag = 0;
     if (isfinite(vk) && isfinite(mn)) {
-      const float band = beta * (norm2[i] + nmax);                           // absolute error bound on d^2
+      const float band = beta * (norm2[i] + nmax + keps);                    // absolute error bound on d^2
       flag = (mn * mn - vk * vk) <= 2.f * band ? 1 : 0;
     }
     amb[i] = flag;
@@ -177,6 +212,7 @@ constexpr int SAMPLE_COLS = 2 * TS, CAND_CAP = 512, TG_MIN_TILES = 8, TG_DEFAULT
 struct Gram2Args {
   const int64_t* frame; const int64_t* gptr; const int64_t* doff; const int64_t* tile_off; const int64_t* tri_off;
   const uint8_t* img; const float* norm2; const float* sum1;
+  const uint32_t* win_amax; // [G] largest |v| of each window: the image is packed times 2^pack_shift
   int64_t num_graphs, max_dist, dim; float* dense;
   int squared;      // store d^2 (the fused row select ranks each row on its own entries; saves the square root)
   float* sample;            // MODE 1: [N][SAMPLE_COLS]
@@ -297,6 +333,7 @@ __global__ void __launch_bounds__(G2_THREADS, 1) gram_blocks2_kernel(Gram2Args a
       int ti, tj, nt;
       cur.seek(a, t, ti, tj, nt);
       const int64_t n0 = a.gptr[cur.w], n = a.gptr[cur.w + 1] - n0;
+      const float down = ldexpf(1.f, -2 * pack_shift(a.win_amax[cur.w]));   // the packed Gram is the true one x 2^2p
       int64_t li = (int64_t)ti * TS + wq * 32 + lane;
       const bool valid = li < n;
       if (!valid) li = n - 1;
@@ -331,7 +368,7 @@ __global__ void __launch_bounds__(G2_THREADS, 1) gram_blocks2_kernel(Gram2Args a
           const bool conn = fj != INT_MIN && df > 0 && (a.max_dist < 0 || df <= a.max_dist);
           // ||a_lo - a_hi + eps||^2 with lo / hi = the smaller / larger node index of the pair (the reference's i < j)
           const float ds = li < lj ? sa - sb : sb - sa;
-          const float d2 = (na + nb) - 2.f * __uint_as_float(j < 16 ? acc0[j] : acc1[j - 16]) + 2.f * eps * ds + keps;
+          const float d2 = (na + nb) - 2.f * (__uint_as_float(j < 16 ? acc0[j] : acc1[j - 16]) * down) + 2.f * eps * ds + keps;
           const float d2c = fmaxf(d2, 0.f);
           const float v = conn ? (a.squared ? d2c : sqrtf(d2c)) : INFINITY;
           D[lj * n + li] = v;                                        // row lj, column li: lanes = consecutive floats
@@ -349,7 +386,7 @@ __global__ void __launch_bounds__(G2_THREADS, 1) gram_blocks2_kernel(Gram2Args a
           int df = fi - fj; df = df < 0 ? -df : df;
           const bool conn = fj != INT_MIN && lj != (int)li && df > 0 && (a.max_dist < 0 || df <= a.max_dist);
           const float ds = (int)li < lj ? sa - sb : sb - sa;
-          const float d2 = (na + nb) - 2.f * __uint_as_float(j < 16 ? acc0[j] : acc1[j - 16]) + 2.f * eps * ds + keps;
+          const float d2 = (na + nb) - 2.f * (__uint_as_float(j < 16 ? acc0[j] : acc1[j - 16]) * down) + 2.f * eps * ds + keps;
           v[j] = conn ? fmaxf(d2, 0.f) : INFINITY;
         }
         if (valid) {
@@ -373,7 +410,7 @@ __global__ void __launch_bounds__(G2_THREADS, 1) gram_blocks2_kernel(Gram2Args a
           const float nb = __shfl_sync(0xffffffffu, nb_l, j), sb = __shfl_sync(0xffffffffu, sb_l, j);
           const float tau_j = __shfl_sync(0xffffffffu, tau_l, j);
           const int lj = colbase + j;
-          d2v[j] = fmaxf((na + nb) - 2.f * __uint_as_float(j < 16 ? acc0[j] : acc1[j - 16]) + 2.f * eps * (sa - sb) + keps, 0.f);
+          d2v[j] = fmaxf((na + nb) - 2.f * (__uint_as_float(j < 16 ? acc0[j] : acc1[j - 16]) * down) + 2.f * eps * (sa - sb) + keps, 0.f);
           const bool live = valid && lj < (int)n && (!diag || lj > row_l);
           if (live && d2v[j] <= tau_i) rowmask |= 1u << j;
           const uint32_t vote = __ballot_sync(0xffffffffu, live && d2v[j] <= tau_j);
@@ -454,7 +491,7 @@ __global__ void __launch_bounds__(32 * CSEL_WARPS) cand_select_kernel(
     const uint2* __restrict__ cand, const int32_t* __restrict__ cand_cnt, const float* __restrict__ tau,
     const int64_t* __restrict__ frame, const int64_t* __restrict__ gptr, int64_t num_graphs, int64_t num_nodes,
     const int64_t* __restrict__ moff, int64_t k, int64_t max_dist, const float* __restrict__ norm2,
-    const float* __restrict__ win_nmax, float beta, uint32_t* __restrict__ M, int32_t* __restrict__ amb,
+    const float* __restrict__ win_nmax, float beta, float keps, uint32_t* __restrict__ M, int32_t* __restrict__ amb,
     int32_t* __restrict__ amb_count) {
   __shared__ int s_hist[CSEL_WARPS][256];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -541,7 +578,7 @@ __global__ void __launch_bounds__(32 * CSEL_WARPS) cand_select_kernel(
     for (int d = 16; d > 0; d >>= 1) mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, d));
     // everything that is not a candidate lies above tau: without an out-of-set candidate tau itself bounds them from below
     if (!isfinite(mn)) mn = tau[i];
-    const float band = beta * (norm2[i] + win_nmax[lo]);                            // absolute error bound on d^2
+    const float band = beta * (norm2[i] + win_nmax[lo] + keps);                     // absolute error bound on d^2
     if (isfinite(mn) && (mn - __uint_as_float(kth)) <= 2.f * band) fallback = true;
   }
   if (lane == 0) {
@@ -558,13 +595,17 @@ int64_t gram_workspace_bytes(int64_t num_nodes, int64_t total_tiles, int64_t num
          2 * align_up((num_graphs + 1) * 8, 256) + align_up(num_nodes * 4, 256) + 1024 +
          // thresholded path: sample, tau, candidate lists and their counters
          align_up(num_nodes * gram::SAMPLE_COLS * 4, 256) + 2 * align_up(num_nodes * 4, 256) +
-         align_up(num_nodes * (int64_t)gram::CAND_CAP * 8, 256);
+         align_up(num_nodes * (int64_t)gram::CAND_CAP * 8, 256) +
+         align_up(num_graphs * 4, 256);                       // largest |v| per window (pre-scale)
 }
+
+// K eps^2 of the d^2 formula: the band's floor, the size of the d^2 terms that do not scale with the embeddings
+float gram_band_keps(int64_t dim) { return (float)dim * 1e-6f * 1e-6f; }
 
 namespace {
 struct GramWs {
   uint8_t* img; float* norm2; float* sum1; int64_t* tile_off; int64_t* tri_off; int32_t* amb;
-  float* sample; float* tau; int32_t* cand_cnt; uint2* cand;
+  float* sample; float* tau; int32_t* cand_cnt; uint2* cand; uint32_t* win_amax;
 };
 GramWs carve_gram(void* ws, int64_t n, int64_t total_tiles, int64_t num_graphs, int64_t dim) {
   Carver cv(ws);
@@ -579,10 +620,12 @@ GramWs carve_gram(void* ws, int64_t n, int64_t total_tiles, int64_t num_graphs, 
   w.tau = cv.take<float>(n);
   w.cand_cnt = cv.take<int32_t>(n);
   w.cand = cv.take<uint2>(n * (int64_t)gram::CAND_CAP);
+  w.win_amax = cv.take<uint32_t>(num_graphs);
   return w;
 }
 
-// pack the embeddings into the tile image (+ norms / sums); shared by the dense and the thresholded path
+// pack the embeddings into the tile image, each window times its 2^p (+ unscaled norms / sums); shared by the dense and
+// the thresholded path
 int gram_pack(const float* reid, int64_t dim, const int64_t* gptr, const int64_t* h_gptr, int64_t num_graphs, const GramWs& w,
               int32_t* status, int64_t* total_tiles_out, cudaStream_t s) {
   using namespace gram;
@@ -591,9 +634,12 @@ int gram_pack(const float* reid, int64_t dim, const int64_t* gptr, const int64_t
   for (int64_t g = 0; g < num_graphs; ++g) total_tiles += ceil_div(h_gptr[g + 1] - h_gptr[g], TS);
   MPN_CUDA(cudaMemsetAsync(w.img, 0, total_tiles * (dim / KC) * CHUNK_BYTES, s));
   MPN_CUDA(cudaMemsetAsync(w.amb + n, 0, 4, s));
+  MPN_CUDA(cudaMemsetAsync(w.win_amax, 0, 4 * num_graphs, s));
   tile_offsets_kernel<<<1, 32, 0, s>>>(gptr, num_graphs, w.tile_off, w.tri_off, 0); count_launch();
-  pack_reid_kernel<<<(unsigned)std::min<int64_t>(ceil_div(n * 32, 256), (int64_t)sm_count() * 16), 256, 0, s>>>(
-      reid, dim, gptr, num_graphs, w.tile_off, n, w.img, w.norm2, w.sum1, status); count_launch();
+  const unsigned pgrid = (unsigned)std::min<int64_t>(ceil_div(n * 32, 256), (int64_t)sm_count() * 16);
+  window_absmax_kernel<<<pgrid, 256, 0, s>>>(reid, dim, gptr, num_graphs, n, w.win_amax); count_launch();
+  pack_reid_kernel<<<pgrid, 256, 0, s>>>(reid, dim, gptr, num_graphs, w.tile_off, n, w.win_amax, w.img, w.norm2, w.sum1,
+                                         status); count_launch();
   MPN_CUDA(cudaFuncSetAttribute(gram::gram_blocks2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, G2_SMEM_BYTES));
   MPN_CUDA(cudaFuncSetAttribute(gram::gram_blocks2_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, G2_SMEM_BYTES));
   MPN_CUDA(cudaFuncSetAttribute(gram::gram_blocks2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, G2_SMEM_BYTES));
@@ -626,7 +672,7 @@ int gram_dist_blocks(const float* reid, int64_t dim, const int64_t* frame, const
   }
   Gram2Args a2 = {};
   a2.frame = frame; a2.gptr = gptr; a2.doff = doff; a2.tile_off = w.tile_off; a2.tri_off = w.tri_off;
-  a2.img = w.img; a2.norm2 = w.norm2; a2.sum1 = w.sum1; a2.num_graphs = num_graphs; a2.max_dist = max_dist; a2.dim = dim;
+  a2.img = w.img; a2.norm2 = w.norm2; a2.sum1 = w.sum1; a2.win_amax = w.win_amax; a2.num_graphs = num_graphs; a2.max_dist = max_dist; a2.dim = dim;
   a2.dense = dense; a2.squared = squared;
   const unsigned grid2 = (unsigned)std::min<int64_t>(std::max<int64_t>(total_blocks, 1), (int64_t)sm_count());
   gram_blocks2_kernel<0><<<grid2, G2_THREADS, G2_SMEM_BYTES, s>>>(a2); count_launch();
@@ -662,7 +708,7 @@ int gram_thresholded_select(const float* reid, int64_t dim, const int64_t* frame
   window_max(w.norm2, gptr, num_graphs, win_nmax, s);
   Gram2Args a2 = {};
   a2.frame = frame; a2.gptr = gptr; a2.doff = nullptr; a2.tile_off = w.tile_off; a2.tri_off = w.tri_off;
-  a2.img = w.img; a2.norm2 = w.norm2; a2.sum1 = w.sum1; a2.num_graphs = num_graphs; a2.max_dist = max_dist; a2.dim = dim;
+  a2.img = w.img; a2.norm2 = w.norm2; a2.sum1 = w.sum1; a2.win_amax = w.win_amax; a2.num_graphs = num_graphs; a2.max_dist = max_dist; a2.dim = dim;
   a2.squared = 1; a2.sample = w.sample; a2.tau = w.tau; a2.cand = w.cand; a2.cand_cnt = w.cand_cnt;
   const int sms = sm_count();
   // 1. sample pass
@@ -678,7 +724,8 @@ int gram_thresholded_select(const float* reid, int64_t dim, const int64_t* frame
   gram_blocks2_kernel<2><<<(unsigned)std::min<int64_t>(tri, sms), G2_THREADS, G2_SMEM_BYTES, s>>>(a2); count_launch();
   // 4. exact top-k over the candidates
   cand_select_kernel<<<(unsigned)ceil_div(n, CSEL_WARPS), 32 * CSEL_WARPS, 0, s>>>(
-      w.cand, w.cand_cnt, w.tau, frame, gptr, num_graphs, n, moff, top_k, max_dist, w.norm2, win_nmax, beta, M, w.amb, w.amb + n);
+      w.cand, w.cand_cnt, w.tau, frame, gptr, num_graphs, n, moff, top_k, max_dist, w.norm2, win_nmax, beta, gram_band_keps(dim), M, w.amb,
+      w.amb + n);
   count_launch();
   MPN_LAUNCH_CHECK();
   *norm2_out = w.norm2; *amb_out = w.amb; *amb_count_out = w.amb + n;
@@ -692,7 +739,7 @@ int gram_fix_ambiguous(const float* reid, int64_t dim, const int64_t* frame, con
   using namespace gram;
   if (detect) {                                                     // (the fused row-select kernel flags rows itself)
     row_ambiguity_kernel<<<(unsigned)num_nodes, 256, 0, s>>>(dense, gptr, num_graphs, doff, norm2, thr_key, thr_idx, beta,
-                                                           amb, amb_count); count_launch();
+                                                           gram_band_keps(dim), amb, amb_count); count_launch();
   }
   exact_rows_kernel<<<(unsigned)num_nodes, 256, 0, s>>>(reid, dim, frame, gptr, num_graphs, doff, max_dist, amb, dense,
                                                         scratch_ld, scratch_rows);

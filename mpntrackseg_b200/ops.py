@@ -128,7 +128,9 @@ def edge_feats_assemble(pairs, frame_f32, bb_height, bb_width, feet_x, feet_y, f
     return attr, eidx
 
 
-LAST_KNN_STATS = [0, 0]      # [tensor-core path used, rows repaired exactly] of the last knn_graph_pairs call
+# [build code, rows repaired exactly] of the last knn_graph_pairs call.  Build code: 0 exact fp32, 1 dense Gram + fused
+# row select, 2 thresholded candidate lists, 3 dense Gram + general select (nonzero = tensor cores).
+LAST_KNN_STATS = [0, 0]
 
 
 def knn_graph_pairs(frame_num, node_graph_ptr_host, reid, top_k, reciprocal, max_frame_dist=-1, engine=None):
