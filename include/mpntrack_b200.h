@@ -123,8 +123,8 @@ int mpn_edge_feats_assemble(const int64_t* row, const int64_t* col, int64_t num_
  * are always the exact ones -- the kept edge set equals the exact path's at every embedding scale (each window is
  * packed under a power-of-two pre-scale, so the band bounds the Gram error).  h_stats (host, may be NULL):
  * [0] = the build that ran: 0 exact fp32 (also after a whole-call exact rerun: values of magnitude >= 65,000 or
- * more flagged rows than scratch slots), 1 dense Gram blocks + fused row select, 2 thresholded candidate lists,
- * 3 dense Gram blocks + general select (windows above 5,120 nodes); nonzero = tensor cores.
+ * more flagged rows than scratch slots), 1 dense Gram blocks + row select, 2 thresholded candidate lists; nonzero =
+ * tensor cores.
  * [1] = number of rows that needed the exact repair.
  * workspace: mpn_knn_graph_workspace(N, sum_g N_g^2, G) bytes (dense fp32 distance blocks + packed embeddings). */
 int64_t mpn_knn_graph_workspace(int64_t num_nodes, int64_t sum_sq_nodes, int64_t num_graphs);

@@ -5,27 +5,15 @@
 #include <math.h>
 
 #include "common.cuh"
+#include "knn_select.cuh"
 
 namespace mpn {
 
-constexpr unsigned kFull = 0xffffffffu;
-
 // ------------------------------------------------------------------ time-valid pairs
-__device__ __forceinline__ bool time_valid(int64_t fi, int64_t fj, int64_t max_dist) {
-  int64_t d = fi > fj ? fi - fj : fj - fi;
-  return d > 0 && (max_dist < 0 || d <= max_dist);
-}
-
 // Upper end of the node range that may pair with node i (its window).
 __device__ __forceinline__ int64_t window_end(const int64_t* __restrict__ gptr, int64_t g,
                                               int64_t n, int64_t i) {
-  if (gptr == nullptr || g <= 0) return n;
-  int64_t lo = 0, hi = g;                     // find window w with gptr[w] <= i < gptr[w+1]
-  while (hi - lo > 1) {
-    int64_t mid = (lo + hi) >> 1;
-    if (gptr[mid] <= i) lo = mid; else hi = mid;
-  }
-  return gptr[lo + 1];
+  return gptr == nullptr || g <= 0 ? n : gptr[window_of(gptr, g, i) + 1];
 }
 
 template <bool kFill>
@@ -42,8 +30,8 @@ __global__ void time_valid_kernel(const int64_t* __restrict__ frame, int64_t n,
     int64_t cursor = kFill ? row_cnt_or_start[i] : 0;
     for (int64_t j0 = i + 1; j0 < end; j0 += 32) {
       const int64_t j = j0 + lane;
-      const bool ok = j < end && time_valid(fi, frame[j], max_dist);
-      const unsigned m = __ballot_sync(kFull, ok);
+      const bool ok = j < end && frames_connect(fi, frame[j], max_dist);
+      const unsigned m = __ballot_sync(kFullMask, ok);
       if (kFill && ok) {
         const int64_t pos = cursor + __popc(m & ((1u << lane) - 1u));
         out_row[pos] = i;
@@ -86,18 +74,12 @@ __global__ void pair_dist_kernel(const float* __restrict__ reid, int64_t dim,
       }
     }
 #pragma unroll
-    for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(kFull, acc, s);
+    for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(kFullMask, acc, s);
     if (lane == 0) out[p] = sqrtf(acc);
   }
 }
 
 // ------------------------------------------------------------------ KNN keep mask
-__device__ __forceinline__ uint32_t order_key(float f) {
-  // monotone map float -> uint32 (ascending), NaN (positive) sorts last like torch.sort
-  uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 __global__ void fill_f32(float* __restrict__ p, int64_t n, float v) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
        i += (int64_t)gridDim.x * blockDim.x)
@@ -115,63 +97,18 @@ __global__ void dense_scatter(const float* __restrict__ d, const int64_t* __rest
   }
 }
 
-// One CTA per dense row: radix-select the k-th smallest (key, index) pair.
+// One CTA per dense row: its k-th smallest (key, index) pair (streamed select_kth).
 // thr_key[i], thr_idx[i]: entry (i, j) is within the top-k  <=>
 //   key(i,j) < thr_key[i]  ||  (key(i,j) == thr_key[i] && j <= thr_idx[i]).
-__global__ void __launch_bounds__(256) row_kth_kernel(const float* __restrict__ dense, int64_t n,
-                                                      int64_t k, uint32_t* __restrict__ thr_key,
-                                                      int32_t* __restrict__ thr_idx) {
-  __shared__ int hist[256];
-  __shared__ uint32_t s_prefix;
-  __shared__ int s_remaining;
-  const int64_t i = blockIdx.x;
-  const float* rowp = dense + i * n;
-  if (threadIdx.x == 0) { s_prefix = 0u; s_remaining = (int)k; }
-  uint32_t mask = 0u;
-  for (int shift = 24; shift >= 0; shift -= 8) {
-    hist[threadIdx.x] = 0;
-    __syncthreads();
-    const uint32_t prefix = s_prefix;
-    for (int64_t j = threadIdx.x; j < n; j += blockDim.x) {
-      const uint32_t key = order_key(rowp[j]);
-      if ((key & mask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      int rem = s_remaining, b = 0;
-      for (; b < 256; ++b) {
-        if (hist[b] >= rem) break;
-        rem -= hist[b];
-      }
-      s_remaining = rem;
-      s_prefix = prefix | ((uint32_t)b << shift);
-    }
-    mask |= 255u << shift;
-    __syncthreads();
-  }
-  // ties at the threshold: include the first `need` of them in index order
-  if (threadIdx.x < 32) {
-    const uint32_t tau = s_prefix;
-    const int need = s_remaining;
-    const int lane = threadIdx.x;
-    int seen = 0;
-    int32_t found = (int32_t)(n - 1);
-    for (int64_t j0 = 0; j0 < n; j0 += 32) {
-      const int64_t j = j0 + lane;
-      const bool eq = j < n && order_key(rowp[j]) == tau;
-      const unsigned m = __ballot_sync(kFull, eq);
-      const int c = __popc(m);
-      if (seen + c >= need) {
-        int want = need - seen;               // 1-based within this ballot
-        unsigned mm = m;
-        for (int q = 1; q < want; ++q) mm &= mm - 1;
-        found = (int32_t)(j0 + __ffs(mm) - 1);
-        break;
-      }
-      seen += c;
-    }
-    if (lane == 0) { thr_key[i] = tau; thr_idx[i] = found; }
-  }
+__global__ void __launch_bounds__(SEL_THREADS) keep_threshold_kernel(const float* __restrict__ dense, int64_t n, int64_t k,
+                                                                    uint32_t* __restrict__ thr_key,
+                                                                    int32_t* __restrict__ thr_idx) {
+  __shared__ SelectSmem sm;
+  const float* rowp = dense + (int64_t)blockIdx.x * n;
+  uint32_t tau;
+  int32_t found;
+  select_kth(RowKeys<0>(rowp, n), rowp, n, k, sm, tau, found);
+  if (threadIdx.x == 0) { thr_key[blockIdx.x] = tau; thr_idx[blockIdx.x] = found; }
 }
 
 __global__ void knn_gather_kernel(const float* __restrict__ dense, int64_t n,
@@ -310,7 +247,7 @@ int mpn_knn_mask(const float* d, const int64_t* row, const int64_t* col, int64_t
   if (!all_in && k > 0) {
     fill_f32<<<grid_for(n * n, 256), 256, 0, s>>>(dense, n * n, INFINITY); count_launch();
     dense_scatter<<<grid_for(e, 256), 256, 0, s>>>(d, row, col, e, n, symmetric_edges ? 0 : 1, dense); count_launch();
-    row_kth_kernel<<<(unsigned)n, 256, 0, s>>>(dense, n, k, tk, ti); count_launch();
+    keep_threshold_kernel<<<(unsigned)n, SEL_THREADS, 0, s>>>(dense, n, k, tk, ti); count_launch();
     knn_gather_kernel<<<grid_for(e, 256), 256, 0, s>>>(dense, n, row, col, e, tk, ti, reciprocal, 0, keep); count_launch();
   } else if (all_in) {
     knn_gather_kernel<<<grid_for(e, 256), 256, 0, s>>>(dense, n, row, col, e, tk, ti, reciprocal, 1, keep); count_launch();

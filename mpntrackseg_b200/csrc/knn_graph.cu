@@ -9,22 +9,12 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "knn_select.cuh"
 
 namespace mpn {
 
-constexpr unsigned kFullMask = 0xffffffffu;
 constexpr int DT = 64;        // distance tile (rows x cols per CTA)
 constexpr int DK = 32;        // feature slab
-
-__device__ __forceinline__ uint32_t order_key_f(float f) {
-  uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
-__device__ __forceinline__ bool frames_connect(int64_t fi, int64_t fj, int64_t max_dist) {
-  const int64_t d = fi > fj ? fi - fj : fj - fi;
-  return d > 0 && (max_dist < 0 || d <= max_dist);
-}
 
 // blockIdx.y = window, blockIdx.x = upper-triangular tile id inside the window.
 __global__ void __launch_bounds__(256) dist_blocks_kernel(const float* __restrict__ reid, int64_t dim,
@@ -91,132 +81,57 @@ __global__ void __launch_bounds__(256) dist_blocks_kernel(const float* __restric
   }
 }
 
-// One CTA per node (batch-global row): radix-select the k-th smallest (key, local index) of its row.
-__global__ void __launch_bounds__(256) batch_row_kth_kernel(const float* __restrict__ dense,
-                                                            const int64_t* __restrict__ gptr, int64_t num_graphs,
-                                                            const int64_t* __restrict__ doff, int64_t k,
-                                                            const int32_t* __restrict__ row_mask,
-                                                            uint32_t* __restrict__ thr_key,
-                                                            int32_t* __restrict__ thr_idx) {
-  __shared__ int hist[256];
-  __shared__ uint32_t s_prefix;
-  __shared__ int s_remaining, s_count;
-  __shared__ int32_t s_found;
+// Exact row of each flagged node (amb[i] != 0) of the tensor-core builds, same arithmetic as dist_blocks_kernel
+// (sequential over the feature dimension).  scratch_ld > 0: `dense` is a scratch area of rows and amb[i] - 1 is this
+// row's slot (the thresholded build writes no dense blocks).
+__global__ void __launch_bounds__(256) exact_rows_kernel(const float* __restrict__ reid, int64_t dim,
+                                                         const int64_t* __restrict__ frame, const int64_t* __restrict__ gptr,
+                                                         int64_t num_graphs, const int64_t* __restrict__ doff, int64_t max_dist,
+                                                         const int32_t* __restrict__ amb, float* __restrict__ dense,
+                                                         int64_t scratch_ld, int64_t scratch_rows) {
   const int64_t i = blockIdx.x;
-  if (row_mask != nullptr && row_mask[i] == 0) return;
-  int64_t lo = 0, hi = num_graphs;                                  // window of node i
-  while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-  const int64_t n0 = gptr[lo], n = gptr[lo + 1] - n0;
-  const float* rowp = dense + doff[lo] + (i - n0) * n;
-  if (k >= n) {                                                     // every rank < k
-    if (threadIdx.x == 0) { thr_key[i] = 0xffffffffu; thr_idx[i] = (int32_t)n; }
-    return;
-  }
-  if (threadIdx.x == 0) { s_prefix = 0u; s_remaining = (int)k; s_found = (int32_t)(n - 1); }
-  uint32_t mask = 0u;
-  const int lane = threadIdx.x & 31;
-  for (int shift = 24; shift >= 0; shift -= 8) {
-    hist[threadIdx.x] = 0;
-    __syncthreads();
-    const uint32_t prefix = s_prefix;
-    for (int64_t j = threadIdx.x; j < n; j += blockDim.x) {
-      const uint32_t key = order_key_f(rowp[j]);
-      if ((key & mask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1);
+  if (!amb[i]) return;
+  const int64_t g = window_of(gptr, num_graphs, i);
+  const int64_t n0 = gptr[g], n = gptr[g + 1] - n0, li = i - n0;
+  if (scratch_ld > 0 && amb[i] > scratch_rows) return;
+  float* rowp = scratch_ld > 0 ? dense + (int64_t)(amb[i] - 1) * scratch_ld : dense + doff[g] + li * n;
+  const int64_t fi = frame[i];
+  const float eps = 1e-6f;
+  for (int64_t lj = threadIdx.x; lj < n; lj += blockDim.x) {
+    float v = INFINITY;
+    if (lj != li && frames_connect(fi, frame[n0 + lj], max_dist)) {
+      // the reference evaluates pairs as (row = smaller index, col = larger index)
+      const float* pa = reid + (n0 + (li < lj ? li : lj)) * dim;
+      const float* pb = reid + (n0 + (li < lj ? lj : li)) * dim;
+      float acc = 0.f;
+      for (int64_t k = 0; k < dim; ++k) { const float d = (pa[k] - pb[k]) + eps; acc = fmaf(d, d, acc); }
+      v = sqrtf(acc);
     }
-    __syncthreads();
-    if (threadIdx.x < 32) {
-      // bin holding the `remaining`-th element: lane l owns bins 8l..8l+7, warp scan over the lane totals
-      int h[8], tot = 0;
-#pragma unroll
-      for (int q = 0; q < 8; ++q) { h[q] = hist[8 * lane + q]; tot += h[q]; }
-      int incl = tot;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) { const int v = __shfl_up_sync(kFullMask, incl, d); if (lane >= d) incl += v; }
-      const int rem0 = s_remaining;
-      const bool here = incl >= rem0 && incl - tot < rem0;              // exactly one lane
-      if (here) {
-        int rem = rem0 - (incl - tot), b = 0;
-#pragma unroll
-        for (int q = 0; q < 8; ++q) { if (h[q] >= rem) { b = q; break; } rem -= h[q]; }
-        s_remaining = rem;
-        s_prefix = prefix | ((uint32_t)(8 * lane + b) << shift);
-        s_count = h[b];
-      }
-    }
-    mask |= 255u << shift;
-    __syncthreads();
-  }
-  const uint32_t tau = s_prefix;
-  const int need = s_remaining;
-  if (s_count == need) {
-    // no tie straddles the boundary: the k-th element (ties by ascending index) is the LAST element equal to tau
-    if (threadIdx.x == 0) s_found = -1;
-    __syncthreads();
-    int32_t mine = -1;
-    for (int64_t j = threadIdx.x; j < n; j += blockDim.x)
-      if (order_key_f(rowp[j]) == tau) mine = (int32_t)j;                // ascending j per thread
-    if (mine >= 0) atomicMax(&s_found, mine);
-    __syncthreads();
-    if (threadIdx.x == 0) { thr_key[i] = tau; thr_idx[i] = s_found; }
-    return;
-  }
-  if (threadIdx.x < 32) {                                           // a tie straddles the boundary: first `need` in index order
-    int seen = 0;
-    int32_t found = (int32_t)(n - 1);
-    for (int64_t j0 = 0; j0 < n; j0 += 32) {
-      const int64_t j = j0 + lane;
-      const bool eq = j < n && order_key_f(rowp[j]) == tau;
-      const unsigned m = __ballot_sync(kFullMask, eq);
-      const int c = __popc(m);
-      if (seen + c >= need) {
-        unsigned mm = m;
-        for (int q = 1; q < need - seen; ++q) mm &= mm - 1;
-        found = (int32_t)(j0 + __ffs(mm) - 1);
-        break;
-      }
-      seen += c;
-    }
-    if (lane == 0) { thr_key[i] = tau; thr_idx[i] = found; }
+    rowp[lj] = v;
   }
 }
 
-// warp per node i: kept pairs (i, j>i) of its window; kFill=false counts, true writes at row_start.
+// warp per node i: every time-valid pair (i, j>i) of its window with its distance (no KNN pruning);
+// kFill=false counts, true writes at row_start.
 template <bool kFill>
-__global__ void knn_pairs_kernel(const float* __restrict__ dense, const int64_t* __restrict__ gptr,
-                                 int64_t num_graphs, const int64_t* __restrict__ doff,
-                                 const int64_t* __restrict__ frame, int64_t num_nodes, int64_t max_dist,
-                                 const uint32_t* __restrict__ thr_key, const int32_t* __restrict__ thr_idx,
-                                 int prune, int reciprocal, int64_t* __restrict__ row_cnt_or_start,
-                                 int64_t* __restrict__ out_row, int64_t* __restrict__ out_col,
-                                 float* __restrict__ out_dist) {
+__global__ void time_valid_pairs_kernel(const float* __restrict__ dense, const int64_t* __restrict__ gptr,
+                                        int64_t num_graphs, const int64_t* __restrict__ doff,
+                                        const int64_t* __restrict__ frame, int64_t num_nodes, int64_t max_dist,
+                                        int64_t* __restrict__ row_cnt_or_start, int64_t* __restrict__ out_row,
+                                        int64_t* __restrict__ out_col, float* __restrict__ out_dist) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t i = warp; i < num_nodes; i += nwarps) {
-    int64_t lo = 0, hi = num_graphs;
-    while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-    const int64_t n0 = gptr[lo], n = gptr[lo + 1] - n0, li = i - n0;
-    const float* D = dense + doff[lo];
+    const int64_t g = window_of(gptr, num_graphs, i);
+    const int64_t n0 = gptr[g], n = gptr[g + 1] - n0, li = i - n0;
+    const float* D = dense + doff[g];
     const int64_t fi = frame[i];
-    const uint32_t ki = prune ? thr_key[i] : 0u;
-    const int32_t ti = prune ? thr_idx[i] : 0;
     int64_t cursor = kFill ? row_cnt_or_start[i] : 0;
     for (int64_t j0 = li + 1; j0 < n; j0 += 32) {
       const int64_t lj = j0 + lane;
-      bool ok = lj < n && frames_connect(fi, frame[n0 + lj], max_dist);
-      float d = 0.f;
-      if (ok) {
-        d = D[li * n + lj];
-        if (prune) {
-          // each row against its own threshold with its own entry: after the tensor-core repair a repaired row holds
-          // exact distances while its mirror entries in the other rows stay approximate
-          const uint32_t key = order_key_f(d), key_t = order_key_f(D[lj * n + li]);
-          const bool a = key < ki || (key == ki && lj <= ti);
-          const uint32_t kj = thr_key[n0 + lj];
-          const bool b = key_t < kj || (key_t == kj && li <= thr_idx[n0 + lj]);
-          ok = reciprocal ? (a && b) : (a || b);
-        }
-      }
+      const bool ok = lj < n && frames_connect(fi, frame[n0 + lj], max_dist);
+      const float d = ok ? D[li * n + lj] : 0.f;
       const unsigned m = __ballot_sync(kFullMask, ok);
       if (kFill && ok) {
         const int64_t pos = cursor + __popc(m & ((1u << lane) - 1u));
@@ -231,12 +146,13 @@ __global__ void knn_pairs_kernel(const float* __restrict__ dense, const int64_t*
 }
 
 
-// ------------------------------------------------------------------ fused row select (windows of up to 5,120 nodes)
-// One CTA per node: the row's keys are read ONCE into registers; radix-select of the k-th (key, index), the row of
-// the "is among my k nearest" bit matrix M, and (tensor-core path) the ambiguity test of the approximate distances
-// all come from those registers.  Every row is ranked on ITS OWN entries, so nothing downstream assumes that the
-// distance matrix is symmetric (repaired rows are exact, their mirror entries stay approximate).
-constexpr int SEL_THREADS = 256, SEL_MAX_N = 20 * SEL_THREADS;
+// ------------------------------------------------------------------ row select
+// One CTA per node: select_kth ranks the row, then the row of the "is among my k nearest" bit matrix M and
+// (tensor-core path) the ambiguity test of the approximate distances.  Windows of up to SEL_MAX_N nodes keep the row's
+// keys in registers (SEL_PER per thread); larger windows re-read the row (SEL_PER = 0).  Every row is ranked on ITS OWN
+// entries, so nothing downstream assumes that the distance matrix is symmetric (repaired rows are exact, their mirror
+// entries stay approximate).
+constexpr int SEL_MAX_N = 20 * SEL_THREADS;
 
 template <bool kAmb, int SEL_PER>
 __global__ void __launch_bounds__(SEL_THREADS) row_select_kernel(
@@ -245,105 +161,36 @@ __global__ void __launch_bounds__(SEL_THREADS) row_select_kernel(
     int32_t* __restrict__ thr_idx, uint32_t* __restrict__ M, const float* __restrict__ norm2,
     const float* __restrict__ win_nmax, float beta, float keps, int32_t* __restrict__ amb, int32_t* __restrict__ amb_count,
     int64_t scratch_ld, int64_t scratch_rows) {
-  __shared__ int hist[256];
-  __shared__ uint32_t s_prefix;
-  __shared__ int s_remaining, s_count;
-  __shared__ int32_t s_found;
+  __shared__ SelectSmem sm;
   __shared__ float s_min[SEL_THREADS / 32];
   const int64_t i = blockIdx.x;
   if (row_mask != nullptr && row_mask[i] == 0) return;
-  int64_t lo = 0, hi = num_graphs;
-  while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-  const int64_t n0 = gptr[lo], n = gptr[lo + 1] - n0, li = i - n0;
+  const int64_t g = window_of(gptr, num_graphs, i);
+  const int64_t n0 = gptr[g], n = gptr[g + 1] - n0, li = i - n0;
   // scratch_ld > 0: `dense` holds exact rows of the flagged nodes only, row_mask[i] - 1 is the row's slot
   if (scratch_ld > 0 && row_mask[i] > scratch_rows) return;
-  const float* rowp = scratch_ld > 0 ? dense + (int64_t)(row_mask[i] - 1) * scratch_ld : dense + doff[lo] + li * n;
+  const float* rowp = scratch_ld > 0 ? dense + (int64_t)(row_mask[i] - 1) * scratch_ld : dense + doff[g] + li * n;
   const int words = (int)((n + 31) >> 5);
-  uint32_t* mrow = M + moff[lo] + li * words;
+  uint32_t* mrow = M + moff[g] + li * words;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  uint32_t key[SEL_PER];
-#pragma unroll
-  for (int q = 0; q < SEL_PER; ++q) {
-    const int64_t j = tid + q * SEL_THREADS;
-    key[q] = j < n ? order_key_f(rowp[j]) : 0xffffffffu;
-  }
-  uint32_t tau = 0xffffffffu;
-  int32_t found = (int32_t)n;
-  if (k < n) {
-    if (tid == 0) { s_prefix = 0u; s_remaining = (int)k; s_found = -1; }
-    uint32_t mask = 0u;
-    for (int shift = 24; shift >= 0; shift -= 8) {
-      hist[tid] = 0;
-      __syncthreads();
-      const uint32_t prefix = s_prefix;
-#pragma unroll
-      for (int q = 0; q < SEL_PER; ++q)
-        if (tid + q * SEL_THREADS < n && (key[q] & mask) == prefix) atomicAdd(&hist[(key[q] >> shift) & 255u], 1);
-      __syncthreads();
-      if (tid < 32) {
-        int h[8], tot = 0;
-#pragma unroll
-        for (int q = 0; q < 8; ++q) { h[q] = hist[8 * lane + q]; tot += h[q]; }
-        int incl = tot;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) { const int v = __shfl_up_sync(kFullMask, incl, d); if (lane >= d) incl += v; }
-        const int rem0 = s_remaining;
-        if (incl >= rem0 && incl - tot < rem0) {                          // exactly one lane
-          int rem = rem0 - (incl - tot), b = 0;
-#pragma unroll
-          for (int q = 0; q < 8; ++q) { if (h[q] >= rem) { b = q; break; } rem -= h[q]; }
-          s_remaining = rem;
-          s_prefix = prefix | ((uint32_t)(8 * lane + b) << shift);
-          s_count = h[b];
-        }
-      }
-      mask |= 255u << shift;
-      __syncthreads();
-    }
-    tau = s_prefix;
-    const int need = s_remaining;
-    if (s_count == need) {                                                // no tie straddles the boundary: last equal element
-      int32_t mine = -1;
-#pragma unroll
-      for (int q = 0; q < SEL_PER; ++q)
-        if (tid + q * SEL_THREADS < n && key[q] == tau) mine = tid + q * SEL_THREADS;
-      if (mine >= 0) atomicMax(&s_found, mine);
-    } else if (tid < 32) {                                                // first `need` equal elements in index order
-      int seen = 0;
-      int32_t f = (int32_t)(n - 1);
-      for (int64_t j0 = 0; j0 < n; j0 += 32) {
-        const int64_t j = j0 + lane;
-        const bool eq = j < n && order_key_f(rowp[j]) == tau;
-        const unsigned m = __ballot_sync(kFullMask, eq);
-        const int c = __popc(m);
-        if (seen + c >= need) {
-          unsigned mm = m;
-          for (int q = 1; q < need - seen; ++q) mm &= mm - 1;
-          f = (int32_t)(j0 + __ffs(mm) - 1);
-          break;
-        }
-        seen += c;
-      }
-      if (lane == 0) s_found = f;
-    }
-    __syncthreads();
-    found = s_found;
-  }
+  const RowKeys<SEL_PER> keys(rowp, n);
+  uint32_t tau;
+  int32_t found;
+  select_kth(keys, rowp, n, k, sm, tau, found);
   if (tid == 0) { thr_key[i] = tau; thr_idx[i] = found; }
   // row of M and the smallest value left outside the top-k
   float mn = INFINITY;
+  const int nq = keys.chunks(n);
 #pragma unroll
-  for (int q = 0; q < SEL_PER; ++q) {
-    const int j = tid + q * SEL_THREADS;
-    if (q * SEL_THREADS < n) {                                            // uniform per warp group
-      const bool in = j < n && (key[q] < tau || (key[q] == tau && j <= found));
+  for (int q = 0; q < nq; ++q) {
+    const int64_t j = tid + (int64_t)q * SEL_THREADS;
+    if ((int64_t)q * SEL_THREADS < n) {                                   // uniform per warp group
+      const uint32_t key = keys[q];
+      const bool in = j < n && (key < tau || (key == tau && j <= found));
       const unsigned m = __ballot_sync(kFullMask, in);
       const int w = q * (SEL_THREADS / 32) + warp;
       if (lane == 0 && w < words) mrow[w] = m;
-      if (kAmb && j < n && !in) {
-        const uint32_t u = (key[q] & 0x80000000u) ? (key[q] & 0x7fffffffu) : ~key[q];
-        mn = fminf(mn, __uint_as_float(u));
-      }
+      if (kAmb && j < n && !in) mn = fminf(mn, key_value(key));
     }
   }
   if (kAmb) {
@@ -354,10 +201,9 @@ __global__ void __launch_bounds__(SEL_THREADS) row_select_kernel(
       for (int q = 1; q < SEL_THREADS / 32; ++q) mn = fminf(mn, s_min[q]);
       int flag = 0;
       if (tau != 0xffffffffu) {
-        const uint32_t u = (tau & 0x80000000u) ? (tau & 0x7fffffffu) : ~tau;
-        const float vk = __uint_as_float(u);
+        const float vk = key_value(tau);
         if (isfinite(vk) && isfinite(mn)) {
-          const float band = beta * (norm2[i] + win_nmax[lo] + keps);     // absolute error bound on d^2
+          const float band = beta * (norm2[i] + win_nmax[g] + keps);      // absolute error bound on d^2
           flag = (mn - vk) <= 2.f * band ? 1 : 0;                         // the approximate rows hold d^2
         }
       }
@@ -379,7 +225,8 @@ static void launch_row_select(int64_t max_n, int64_t n, cudaStream_t s, const fl
   if (max_n <= 5 * SEL_THREADS) MPN_SEL(5);
   else if (max_n <= 9 * SEL_THREADS) MPN_SEL(9);
   else if (max_n <= 12 * SEL_THREADS) MPN_SEL(12);
-  else MPN_SEL(20);
+  else if (max_n <= SEL_MAX_N) MPN_SEL(20);
+  else MPN_SEL(0);
 #undef MPN_SEL
   count_launch();
 }
@@ -431,12 +278,11 @@ __global__ void mask_pairs_kernel(const uint32_t* __restrict__ M, const uint32_t
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t i = warp; i < num_nodes; i += nwarps) {
-    int64_t lo = 0, hi = num_graphs;
-    while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-    const int64_t n0 = gptr[lo], n = gptr[lo + 1] - n0, li = i - n0;
+    const int64_t g = window_of(gptr, num_graphs, i);
+    const int64_t n0 = gptr[g], n = gptr[g + 1] - n0, li = i - n0;
     const int words = (int)((n + 31) >> 5);
-    const uint32_t* mi = M + moff[lo] + li * words;
-    const uint32_t* mti = MT + moff[lo] + li * words;
+    const uint32_t* mi = M + moff[g] + li * words;
+    const uint32_t* mti = MT + moff[g] + li * words;
     const int64_t fi = frame[i];
     int64_t cursor = kFill ? row_cnt_or_start[i] : 0;
     for (int c0 = (int)((li + 1) >> 5); c0 < words; c0 += 32) {
@@ -465,7 +311,7 @@ __global__ void mask_pairs_kernel(const uint32_t* __restrict__ M, const uint32_t
           const int64_t lj = (int64_t)c * 32 + b;
           out_row[pos] = i;
           out_col[pos] = n0 + lj;
-          out_dist[pos] = dense != nullptr ? dense[doff[lo] + li * n + lj] : 0.f;   // (recomputed exactly by the caller)
+          out_dist[pos] = dense != nullptr ? dense[doff[g] + li * n + lj] : 0.f;   // (recomputed exactly by the caller)
           ++pos;
         }
       }
@@ -501,12 +347,7 @@ int64_t gram_workspace_bytes(int64_t num_nodes, int64_t total_tiles, int64_t num
 float gram_band_keps(int64_t dim);
 int gram_dist_blocks(const float* reid, int64_t dim, const int64_t* frame, const int64_t* gptr, const int64_t* h_gptr,
                      int64_t num_graphs, const int64_t* doff, int64_t max_dist, void* ws, float* dense,
-                     int32_t* status, float** norm2_out, int32_t** amb_out, int32_t** amb_count_out, int squared,
-                     cudaStream_t s);
-int gram_fix_ambiguous(const float* reid, int64_t dim, const int64_t* frame, const int64_t* gptr, int64_t num_graphs,
-                       int64_t num_nodes, const int64_t* doff, int64_t max_dist, float* dense, const float* norm2,
-                       const uint32_t* thr_key, const int32_t* thr_idx, float beta, int32_t* amb, int32_t* amb_count,
-                       int detect, int64_t scratch_ld, int64_t scratch_rows, cudaStream_t s);
+                     int32_t* status, float** norm2_out, int32_t** amb_out, int32_t** amb_count_out, cudaStream_t s);
 bool gram_thresholded_applies(const int64_t* h_gptr, int64_t num_graphs, int64_t top_k);
 int gram_thresholded_select(const float* reid, int64_t dim, const int64_t* frame, const int64_t* gptr, const int64_t* h_gptr,
                             int64_t num_graphs, const int64_t* moff, int64_t max_dist, int64_t top_k, void* ws,
@@ -580,6 +421,7 @@ int mpn_knn_graph_pairs(const int64_t* frame, const int64_t* gptr, const int64_t
   const bool force_dense = getenv("MPN_KNN_DENSE") != nullptr;          // read per call: tests toggle it
   const bool tg = tc && max_n <= SEL_MAX_N && !force_dense && gram_thresholded_applies(h_gptr, num_graphs, top_k);
   int64_t scratch_rows = 0;
+  // pruned builds: per-row select into the bit matrix M -> transpose -> pairs (i, j > i) kept by M[i][j] and / or M[j][i]
   if (tg) {
     rc = gram_thresholded_select(reid, dim, frame, gptr, h_gptr, num_graphs, moff, max_frame_dist, top_k,
                                  static_cast<char*>(ws) + cv.off, win_nmax, 2e-6f, M, status, &norm2, &amb, &amb_count,
@@ -588,58 +430,40 @@ int mpn_knn_graph_pairs(const int64_t* frame, const int64_t* gptr, const int64_t
     // flagged rows (uncertain top-k set, list overflow, too few candidates): exact fp32 row into a scratch slot of the
     // (otherwise unused) dense area, ranked by the dense row select
     scratch_rows = sum_sq / max_n;
-    rc = gram_fix_ambiguous(reid, dim, frame, gptr, num_graphs, n, doff, max_frame_dist, dense, norm2, tk, ti, 2e-6f, amb,
-                            amb_count, 0, max_n, scratch_rows, s);
-    if (rc) return rc;
+    exact_rows_kernel<<<(unsigned)n, 256, 0, s>>>(reid, dim, frame, gptr, num_graphs, doff, max_frame_dist, amb, dense, max_n,
+                                                  scratch_rows); count_launch();
     launch_row_select<false>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, amb, tk, ti, M, nullptr, nullptr, 0.f,
                              0.f, nullptr, nullptr, max_n, scratch_rows);
   } else if (tc) {
     rc = gram_dist_blocks(reid, dim, frame, gptr, h_gptr, num_graphs, doff, max_frame_dist,
-                          static_cast<char*>(ws) + cv.off, dense, status, &norm2, &amb, &amb_count,
-                          max_n <= SEL_MAX_N ? 1 : 0, s);
+                          static_cast<char*>(ws) + cv.off, dense, status, &norm2, &amb, &amb_count, s);
     if (rc) return rc;
+    window_max_kernel<<<(unsigned)num_graphs, 256, 0, s>>>(norm2, gptr, win_nmax); count_launch();
+    launch_row_select<true>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, nullptr, tk, ti, M, norm2, win_nmax, 2e-6f,
+                            gram_band_keps(dim), amb, amb_count);
+    // rows whose top-k set is not certain: exact fp32 distances, ranked again
+    exact_rows_kernel<<<(unsigned)n, 256, 0, s>>>(reid, dim, frame, gptr, num_graphs, doff, max_frame_dist, amb, dense, 0, 0);
+    count_launch();
+    launch_row_select<false>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, amb, tk, ti, M, nullptr, nullptr, 0.f,
+                             0.f, nullptr, nullptr);
   } else {
     const int64_t nt = ceil_div(max_n, DT);
     dim3 grid((unsigned)(nt * (nt + 1) / 2), (unsigned)num_graphs);
     dist_blocks_kernel<<<grid, 256, 0, s>>>(reid, dim, frame, gptr, doff, max_frame_dist, dense); count_launch();
-  }
-  const unsigned wgrid = (unsigned)std::min<int64_t>(ceil_div(n * 32, 256), (int64_t)sm_count() * 16);
-  // windows of up to SEL_MAX_N nodes: fused row select -> bit matrices -> pairs; larger windows: the general kernels
-  const bool fused = prune && max_n <= SEL_MAX_N;
-  if (fused) {
-    if (tg) {
-      // bit matrix rows are already in place
-    } else if (tc) {
-      window_max_kernel<<<(unsigned)num_graphs, 256, 0, s>>>(norm2, gptr, win_nmax); count_launch();
-      launch_row_select<true>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, nullptr, tk, ti, M, norm2, win_nmax, 2e-6f,
-                              gram_band_keps(dim), amb, amb_count);
-      // rows whose top-k set is not certain: exact fp32 distances, ranked again
-      rc = gram_fix_ambiguous(reid, dim, frame, gptr, num_graphs, n, doff, max_frame_dist, dense, norm2, tk, ti, 2e-6f,
-                              amb, amb_count, 0, 0, 0, s);
-      if (rc) return rc;
-      launch_row_select<false>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, amb, tk, ti, M, nullptr, nullptr, 0.f,
-                               0.f, nullptr, nullptr);
-    } else {
+    if (prune)
       launch_row_select<false>(max_n, n, s, dense, gptr, num_graphs, doff, moff, top_k, nullptr, tk, ti, M, nullptr, nullptr, 0.f,
                                0.f, nullptr, nullptr);
-    }
+  }
+  const unsigned wgrid = (unsigned)std::min<int64_t>(ceil_div(n * 32, 256), (int64_t)sm_count() * 16);
+  if (prune) {
     const int64_t max_words = (max_n + 31) >> 5;
     const unsigned tgrid = (unsigned)std::min<int64_t>(std::max<int64_t>(ceil_div(max_words * max_words * 32, 256), 1), 4096);
     bit_transpose_kernel<<<dim3(tgrid, (unsigned)num_graphs), 256, 0, s>>>(M, MT, gptr, moff); count_launch();
     mask_pairs_kernel<false><<<wgrid, 256, 0, s>>>(M, MT, tg ? nullptr : dense, gptr, num_graphs, doff, moff, frame, n, max_frame_dist, reciprocal,
                                                   row_start, nullptr, nullptr, nullptr); count_launch();
   } else {
-    if (prune) {
-      batch_row_kth_kernel<<<(unsigned)n, 256, 0, s>>>(dense, gptr, num_graphs, doff, top_k, nullptr, tk, ti); count_launch();
-      if (tc) {                                                       // repair rows whose top-k set is not certain
-        rc = gram_fix_ambiguous(reid, dim, frame, gptr, num_graphs, n, doff, max_frame_dist, dense, norm2, tk, ti, 2e-6f,
-                                amb, amb_count, 1, 0, 0, s);
-        if (rc) return rc;
-        batch_row_kth_kernel<<<(unsigned)n, 256, 0, s>>>(dense, gptr, num_graphs, doff, top_k, amb, tk, ti); count_launch();
-      }
-    }
-    knn_pairs_kernel<false><<<wgrid, 256, 0, s>>>(dense, gptr, num_graphs, doff, frame, n, max_frame_dist, tk, ti, prune,
-                                                 reciprocal, row_start, nullptr, nullptr, nullptr); count_launch();
+    time_valid_pairs_kernel<false><<<wgrid, 256, 0, s>>>(dense, gptr, num_graphs, doff, frame, n, max_frame_dist, row_start,
+                                                        nullptr, nullptr, nullptr); count_launch();
   }
   MPN_LAUNCH_CHECK();
   rc = exclusive_scan_i64(row_start, row_start, n, s);
@@ -655,19 +479,19 @@ int mpn_knn_graph_pairs(const int64_t* frame, const int64_t* gptr, const int64_t
   if (tc && h_flags[0] != 0)                                        // embeddings beyond the fp16 range: exact kernel
     return mpn_knn_graph_pairs(frame, gptr, h_gptr, num_graphs, reid, dim, top_k, reciprocal, max_frame_dist, 0, ws,
                                capacity, out_row, out_col, out_dist, graph_pair_ptr, h_graph_pair_ptr, h_stats, stream);
-  // build code: 0 exact, 1 dense Gram + fused row select, 2 thresholded candidate lists, 3 dense Gram + general select
-  if (h_stats != nullptr) { h_stats[0] = tg ? 2 : (tc ? (fused ? 1 : 3) : 0); h_stats[1] = h_flags[1]; }
+  // build code: 0 exact, 1 dense Gram + row select, 2 thresholded candidate lists
+  if (h_stats != nullptr) { h_stats[0] = tg ? 2 : (tc ? 1 : 0); h_stats[1] = h_flags[1]; }
   const int64_t total = h_graph_pair_ptr[num_graphs];
   if (total > capacity) {
     set_error("knn_graph_pairs: %lld pairs exceed the output capacity %lld", (long long)total, (long long)capacity);
     return MPN_ENOSPC;
   }
-  if (fused) {
+  if (prune) {
     mask_pairs_kernel<true><<<wgrid, 256, 0, s>>>(M, MT, tg ? nullptr : dense, gptr, num_graphs, doff, moff, frame, n, max_frame_dist, reciprocal,
                                                  row_start, out_row, out_col, out_dist); count_launch();
   } else {
-    knn_pairs_kernel<true><<<wgrid, 256, 0, s>>>(dense, gptr, num_graphs, doff, frame, n, max_frame_dist, tk, ti, prune,
-                                                reciprocal, row_start, out_row, out_col, out_dist); count_launch();
+    time_valid_pairs_kernel<true><<<wgrid, 256, 0, s>>>(dense, gptr, num_graphs, doff, frame, n, max_frame_dist, row_start,
+                                                       out_row, out_col, out_dist); count_launch();
   }
   MPN_LAUNCH_CHECK();
   if (tc && total > 0)                                              // the edge feature is always the exact distance

@@ -5,7 +5,7 @@
 // the exact fp32 formula of the reference (same kernel arithmetic as knn_graph.cu) and re-ranked, and the
 // distances attached to the kept pairs are always recomputed exactly.  The kept edge set is therefore the
 // one the exact path produces.
-// The band, beta * (||a_i||^2 + max_window ||a||^2 + K eps^2), is relative to the window's largest squared norm.
+// The band, beta * (||a_i||^2 + max_window ||a||^2 + K eps^2), is relative to the window's largest ||a||^2.
 // The split's error is relative too only while the values sit high in the fp16 range: below 2^-3 the low half
 // is subnormal and its error an absolute 2^-25.  So every window is packed times 2^p, p chosen from its largest
 // |v| (pack_shift), and the Gram result is multiplied by 2^-2p, both exact (DESIGN.md section 4).
@@ -14,6 +14,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "knn_select.cuh"
 #include "tc_ptx.cuh"
 
 namespace mpn {
@@ -48,12 +49,11 @@ __global__ void window_absmax_kernel(const float* __restrict__ reid, int64_t dim
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t i = warp; i < num_nodes; i += nwarps) {
-    int64_t lo = 0, hi = num_graphs;
-    while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
+    const int64_t g = window_of(gptr, num_graphs, i);
     float m = 0.f;
     for (int64_t k = lane; k < dim; k += 32) m = fmaxf(m, fabsf(reid[i * dim + k]));
     for (int d = 16; d > 0; d >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, d));
-    if (lane == 0) atomicMax(&win_amax[lo], __float_as_uint(m));
+    if (lane == 0) atomicMax(&win_amax[g], __float_as_uint(m));
   }
 }
 
@@ -68,12 +68,11 @@ __global__ void pack_reid_kernel(const float* __restrict__ reid, int64_t dim, co
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const int nchunks = (int)(dim / KC);
   for (int64_t i = warp; i < num_nodes; i += nwarps) {
-    int64_t lo = 0, hi = num_graphs;
-    while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-    const int64_t li = i - gptr[lo];
-    const int64_t tile = tile_off[lo] + li / TS;
+    const int64_t g = window_of(gptr, num_graphs, i);
+    const int64_t li = i - gptr[g];
+    const int64_t tile = tile_off[g] + li / TS;
     const int n = (int)(li % TS);
-    const float up = ldexpf(1.f, pack_shift(win_amax[lo]));
+    const float up = ldexpf(1.f, pack_shift(win_amax[g]));
     float s2 = 0.f, s1 = 0.f;
     bool ovf = false;
     for (int64_t k = lane; k < dim; k += 32) {
@@ -90,86 +89,6 @@ __global__ void pack_reid_kernel(const float* __restrict__ reid, int64_t dim, co
     for (int d = 16; d > 0; d >>= 1) { s2 += __shfl_xor_sync(0xffffffffu, s2, d); s1 += __shfl_xor_sync(0xffffffffu, s1, d); }
     if (lane == 0) { norm2[i] = s2; sum1[i] = s1; }
     if (ovf) atomicOr(status, 1);
-  }
-}
-
-__device__ __forceinline__ uint32_t okey(float f) {
-  uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
-// One CTA per row: is the top-k SET of this row certain given the error band of the Gram distances?
-// ambiguous <=> an entry outside the top-k lies within the band above the k-th value (in d^2).
-__global__ void __launch_bounds__(256) row_ambiguity_kernel(const float* __restrict__ dense, const int64_t* __restrict__ gptr,
-                                                            int64_t num_graphs, const int64_t* __restrict__ doff,
-                                                            const float* __restrict__ norm2, const uint32_t* __restrict__ thr_key,
-                                                            const int32_t* __restrict__ thr_idx, float beta, float keps,
-                                                            int32_t* __restrict__ amb, int32_t* __restrict__ amb_count) {
-  __shared__ float s_min[8];
-  __shared__ float s_nmax[8];
-  const int64_t i = blockIdx.x;
-  int64_t lo = 0, hi = num_graphs;
-  while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-  const int64_t n0 = gptr[lo], n = gptr[lo + 1] - n0;
-  const float* rowp = dense + doff[lo] + (i - n0) * n;
-  const uint32_t tk = thr_key[i];
-  const int32_t ti = thr_idx[i];
-  if (tk == 0xffffffffu) { if (threadIdx.x == 0) amb[i] = 0; return; }      // k >= row length: everything is in
-  float mn = INFINITY, nmax = 0.f;
-  for (int64_t j = threadIdx.x; j < n; j += blockDim.x) {
-    const float v = rowp[j];
-    const uint32_t key = okey(v);
-    const bool outside = key > tk || (key == tk && j > ti);
-    if (outside) mn = fminf(mn, v);
-    nmax = fmaxf(nmax, norm2[n0 + j]);
-  }
-  for (int d = 16; d > 0; d >>= 1) { mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, d)); nmax = fmaxf(nmax, __shfl_xor_sync(0xffffffffu, nmax, d)); }
-  if ((threadIdx.x & 31) == 0) { s_min[threadIdx.x >> 5] = mn; s_nmax[threadIdx.x >> 5] = nmax; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int q = 1; q < 8; ++q) { mn = fminf(mn, s_min[q]); nmax = fmaxf(nmax, s_nmax[q]); }
-    // k-th value from its key
-    const uint32_t u = (tk & 0x80000000u) ? (tk & 0x7fffffffu) : ~tk;
-    const float vk = __uint_as_float(u);
-    int flag = 0;
-    if (isfinite(vk) && isfinite(mn)) {
-      const float band = beta * (norm2[i] + nmax + keps);                    // absolute error bound on d^2
-      flag = (mn * mn - vk * vk) <= 2.f * band ? 1 : 0;
-    }
-    amb[i] = flag;
-    if (flag) atomicAdd(amb_count, 1);
-  }
-}
-
-// Exact fp32 row (reference formula, sequential over the feature dimension) for the flagged rows.
-__global__ void __launch_bounds__(256) exact_rows_kernel(const float* __restrict__ reid, int64_t dim,
-                                                         const int64_t* __restrict__ frame, const int64_t* __restrict__ gptr,
-                                                         int64_t num_graphs, const int64_t* __restrict__ doff, int64_t max_dist,
-                                                         const int32_t* __restrict__ amb, float* __restrict__ dense,
-                                                         int64_t scratch_ld, int64_t scratch_rows) {
-  const int64_t i = blockIdx.x;
-  if (!amb[i]) return;
-  int64_t lo = 0, hi = num_graphs;
-  while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-  const int64_t n0 = gptr[lo], n = gptr[lo + 1] - n0, li = i - n0;
-  // scratch_ld > 0: `dense` is a scratch area of rows, amb[i] - 1 is this row's slot (thresholded path: no dense blocks)
-  if (scratch_ld > 0 && amb[i] > scratch_rows) return;
-  float* rowp = scratch_ld > 0 ? dense + (int64_t)(amb[i] - 1) * scratch_ld : dense + doff[lo] + li * n;
-  const int64_t fi = frame[i];
-  const float eps = 1e-6f;
-  for (int64_t lj = threadIdx.x; lj < n; lj += blockDim.x) {
-    const int64_t fj = frame[n0 + lj];
-    const int64_t df = fi > fj ? fi - fj : fj - fi;
-    float v = INFINITY;
-    if (lj != li && df > 0 && (max_dist < 0 || df <= max_dist)) {
-      // the reference evaluates pairs as (row = smaller index, col = larger index)
-      const float* pa = reid + (n0 + (li < lj ? li : lj)) * dim;
-      const float* pb = reid + (n0 + (li < lj ? lj : li)) * dim;
-      float acc = 0.f;
-      for (int64_t k = 0; k < dim; ++k) { const float d = (pa[k] - pb[k]) + eps; acc = fmaf(d, d, acc); }
-      v = sqrtf(acc);
-    }
-    rowp[lj] = v;
   }
 }
 
@@ -213,8 +132,7 @@ struct Gram2Args {
   const int64_t* frame; const int64_t* gptr; const int64_t* doff; const int64_t* tile_off; const int64_t* tri_off;
   const uint8_t* img; const float* norm2; const float* sum1;
   const uint32_t* win_amax; // [G] largest |v| of each window: the image is packed times 2^pack_shift
-  int64_t num_graphs, max_dist, dim; float* dense;
-  int squared;      // store d^2 (the fused row select ranks each row on its own entries; saves the square root)
+  int64_t num_graphs, max_dist, dim; float* dense;  // MODE 0: [sum N_g^2] approximate d^2 (+inf where not time-valid)
   float* sample;            // MODE 1: [N][SAMPLE_COLS]
   const float* tau;         // MODE 2: [N] thresholds on d^2
   uint2* cand;              // MODE 2: [N][CAND_CAP] (column index inside the window, d^2 bits)
@@ -370,7 +288,7 @@ __global__ void __launch_bounds__(G2_THREADS, 1) gram_blocks2_kernel(Gram2Args a
           const float ds = li < lj ? sa - sb : sb - sa;
           const float d2 = (na + nb) - 2.f * (__uint_as_float(j < 16 ? acc0[j] : acc1[j - 16]) * down) + 2.f * eps * ds + keps;
           const float d2c = fmaxf(d2, 0.f);
-          const float v = conn ? (a.squared ? d2c : sqrtf(d2c)) : INFINITY;
+          const float v = conn ? d2c : INFINITY;
           D[lj * n + li] = v;                                        // row lj, column li: lanes = consecutive floats
           if (ti == tj) D[li * n + lj] = v;
         }
@@ -454,9 +372,8 @@ __global__ void __launch_bounds__(256) row_threshold_kernel(const float* __restr
   const int lane = threadIdx.x & 31;
   const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (i >= num_nodes) return;
-  int64_t lo = 0, hi = num_graphs;
-  while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-  const int64_t n = gptr[lo + 1] - gptr[lo];
+  const int64_t g = window_of(gptr, num_graphs, i);
+  const int64_t n = gptr[g + 1] - gptr[g];
   float v[8];
   int nv = 0;
 #pragma unroll
@@ -498,11 +415,10 @@ __global__ void __launch_bounds__(32 * CSEL_WARPS) cand_select_kernel(
   const int64_t i = (int64_t)blockIdx.x * CSEL_WARPS + wib;
   if (i >= num_nodes) return;
   int* hist = s_hist[wib];
-  int64_t lo = 0, hi = num_graphs;
-  while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (gptr[mid] <= i) lo = mid; else hi = mid; }
-  const int64_t n0 = gptr[lo], n = gptr[lo + 1] - n0, li = i - n0;
+  const int64_t g = window_of(gptr, num_graphs, i);
+  const int64_t n0 = gptr[g], n = gptr[g + 1] - n0, li = i - n0;
   const int words = (int)((n + 31) >> 5);
-  uint32_t* mrow = M + moff[lo] + li * words;
+  uint32_t* mrow = M + moff[g] + li * words;
   for (int w = lane; w < words; w += 32) mrow[w] = 0u;
   const int cnt = cand_cnt[i];
   bool fallback = cnt > CAND_CAP;
@@ -517,9 +433,7 @@ __global__ void __launch_bounds__(32 * CSEL_WARPS) cand_select_kernel(
     key[q] = 0xffffffffu; idx[q] = -1;
     if (!fallback && c < cnt) {
       const uint2 e = cand[i * CAND_CAP + c];
-      const int64_t fj = frame[n0 + e.x];
-      const int64_t df = fi > fj ? fi - fj : fj - fi;
-      if ((int64_t)e.x != li && df > 0 && (max_dist < 0 || df <= max_dist)) { key[q] = e.y; idx[q] = (int32_t)e.x; ++nvalid; }
+      if ((int64_t)e.x != li && frames_connect(fi, frame[n0 + e.x], max_dist)) { key[q] = e.y; idx[q] = (int32_t)e.x; ++nvalid; }
     }
   }
   for (int d = 16; d > 0; d >>= 1) nvalid += __shfl_xor_sync(0xffffffffu, nvalid, d);
@@ -578,7 +492,7 @@ __global__ void __launch_bounds__(32 * CSEL_WARPS) cand_select_kernel(
     for (int d = 16; d > 0; d >>= 1) mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, d));
     // everything that is not a candidate lies above tau: without an out-of-set candidate tau itself bounds them from below
     if (!isfinite(mn)) mn = tau[i];
-    const float band = beta * (norm2[i] + win_nmax[lo] + keps);                     // absolute error bound on d^2
+    const float band = beta * (norm2[i] + win_nmax[g] + keps);                      // absolute error bound on d^2
     if (isfinite(mn) && (mn - __uint_as_float(kth)) <= 2.f * band) fallback = true;
   }
   if (lane == 0) {
@@ -653,12 +567,10 @@ int64_t count_tiles(const int64_t* h_gptr, int64_t num_graphs) {
 }
 }  // namespace
 
-// Fills the dense blocks with Gram distances, ranks, then repairs ambiguous rows exactly.
-// `rank_rows(mask)` is provided by knn_graph.cu (batch_row_kth_kernel launcher).
+// Fills the dense blocks with approximate d^2 from the Gram kernel; the caller ranks the rows and repairs the flagged ones.
 int gram_dist_blocks(const float* reid, int64_t dim, const int64_t* frame, const int64_t* gptr, const int64_t* h_gptr,
                      int64_t num_graphs, const int64_t* doff, int64_t max_dist, void* ws, float* dense,
-                     int32_t* status, float** norm2_out, int32_t** amb_out, int32_t** amb_count_out, int squared,
-                     cudaStream_t s) {
+                     int32_t* status, float** norm2_out, int32_t** amb_out, int32_t** amb_count_out, cudaStream_t s) {
   using namespace gram;
   const int64_t n = h_gptr[num_graphs];
   GramWs w = carve_gram(ws, n, count_tiles(h_gptr, num_graphs), num_graphs, dim);
@@ -673,7 +585,7 @@ int gram_dist_blocks(const float* reid, int64_t dim, const int64_t* frame, const
   Gram2Args a2 = {};
   a2.frame = frame; a2.gptr = gptr; a2.doff = doff; a2.tile_off = w.tile_off; a2.tri_off = w.tri_off;
   a2.img = w.img; a2.norm2 = w.norm2; a2.sum1 = w.sum1; a2.win_amax = w.win_amax; a2.num_graphs = num_graphs; a2.max_dist = max_dist; a2.dim = dim;
-  a2.dense = dense; a2.squared = squared;
+  a2.dense = dense;
   const unsigned grid2 = (unsigned)std::min<int64_t>(std::max<int64_t>(total_blocks, 1), (int64_t)sm_count());
   gram_blocks2_kernel<0><<<grid2, G2_THREADS, G2_SMEM_BYTES, s>>>(a2); count_launch();
   MPN_LAUNCH_CHECK();
@@ -709,7 +621,7 @@ int gram_thresholded_select(const float* reid, int64_t dim, const int64_t* frame
   Gram2Args a2 = {};
   a2.frame = frame; a2.gptr = gptr; a2.doff = nullptr; a2.tile_off = w.tile_off; a2.tri_off = w.tri_off;
   a2.img = w.img; a2.norm2 = w.norm2; a2.sum1 = w.sum1; a2.win_amax = w.win_amax; a2.num_graphs = num_graphs; a2.max_dist = max_dist; a2.dim = dim;
-  a2.squared = 1; a2.sample = w.sample; a2.tau = w.tau; a2.cand = w.cand; a2.cand_cnt = w.cand_cnt;
+  a2.sample = w.sample; a2.tau = w.tau; a2.cand = w.cand; a2.cand_cnt = w.cand_cnt;
   const int sms = sm_count();
   // 1. sample pass
   tile_offsets_kernel<<<1, 32, 0, s>>>(gptr, num_graphs, w.tile_off, w.tri_off, 1); count_launch();
@@ -729,22 +641,6 @@ int gram_thresholded_select(const float* reid, int64_t dim, const int64_t* frame
   count_launch();
   MPN_LAUNCH_CHECK();
   *norm2_out = w.norm2; *amb_out = w.amb; *amb_count_out = w.amb + n;
-  return MPN_OK;
-}
-
-int gram_fix_ambiguous(const float* reid, int64_t dim, const int64_t* frame, const int64_t* gptr, int64_t num_graphs,
-                       int64_t num_nodes, const int64_t* doff, int64_t max_dist, float* dense, const float* norm2,
-                       const uint32_t* thr_key, const int32_t* thr_idx, float beta, int32_t* amb, int32_t* amb_count,
-                       int detect, int64_t scratch_ld, int64_t scratch_rows, cudaStream_t s) {
-  using namespace gram;
-  if (detect) {                                                     // (the fused row-select kernel flags rows itself)
-    row_ambiguity_kernel<<<(unsigned)num_nodes, 256, 0, s>>>(dense, gptr, num_graphs, doff, norm2, thr_key, thr_idx, beta,
-                                                           gram_band_keps(dim), amb, amb_count); count_launch();
-  }
-  exact_rows_kernel<<<(unsigned)num_nodes, 256, 0, s>>>(reid, dim, frame, gptr, num_graphs, doff, max_dist, amb, dense,
-                                                        scratch_ld, scratch_rows);
-  count_launch();
-  MPN_LAUNCH_CHECK();
   return MPN_OK;
 }
 

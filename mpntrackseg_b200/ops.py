@@ -128,8 +128,8 @@ def edge_feats_assemble(pairs, frame_f32, bb_height, bb_width, feet_x, feet_y, f
     return attr, eidx
 
 
-# [build code, rows repaired exactly] of the last knn_graph_pairs call.  Build code: 0 exact fp32, 1 dense Gram + fused
-# row select, 2 thresholded candidate lists, 3 dense Gram + general select (nonzero = tensor cores).
+# [build code, rows repaired exactly] of the last knn_graph_pairs call.  Build code: 0 exact fp32, 1 dense Gram + row
+# select, 2 thresholded candidate lists (nonzero = tensor cores).
 LAST_KNN_STATS = [0, 0]
 
 

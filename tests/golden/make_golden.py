@@ -345,7 +345,7 @@ def run_config5_case():
 
 
 def run_big_window_case():
-    """A window of 5,400 detections (> 5,120: the batched builder's general select path): kept pairs only."""
+    """A window of 5,400 detections (> 5,120: the batched builder's streamed row select): kept pairs only."""
     c = BIG_CASES['big_window']
     win = synth.make_window(**c['win'])
     ds = default_dataset_params(**c['ds'])

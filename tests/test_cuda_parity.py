@@ -1011,7 +1011,7 @@ def test_config5_dense_crowd_window_matches_reference_golden(engine):
 @pytest.mark.parametrize('k', [25, 50, 100, 128])
 def test_thresholded_and_dense_knn_builds_keep_the_same_pairs(k, monkeypatch):
     """The two tensor-core graph builds (thresholded candidate lists: default up to k = 64, forced up to k = 128 with
-    MPN_KNN_THRESHOLDED; dense blocks + fused row select: MPN_KNN_DENSE) and the exact fp32 build return identical pairs on
+    MPN_KNN_THRESHOLDED; dense blocks + row select: MPN_KNN_DENSE) and the exact fp32 build return identical pairs on
     the configs[4] window (N = 4,500) next to a configs[1]-sized one."""
     from mpntrackseg_b200.data.mot_graph import build_window_graphs
     c = load_big_case('config5')
@@ -1036,10 +1036,11 @@ def test_thresholded_and_dense_knn_builds_keep_the_same_pairs(k, monkeypatch):
 
 
 @pytest.mark.parametrize('engine', ENGINES)
-def test_window_beyond_5120_nodes_takes_the_general_select_path(engine):
-    """A window of 5,400 detections is above the fused row-select limit (5,120): batch_row_kth_kernel / knn_pairs_kernel
-    (csrc/knn_graph.cu) must produce the reference's kept pairs (tests/golden/big_window.npz), alone and next to a
-    small window in the same batch."""
+def test_window_beyond_5120_nodes_takes_the_streamed_row_select(engine):
+    """A window of 5,400 detections is above the limit (5,120) of the register-held row select: row_select_kernel
+    re-reads its rows (csrc/knn_graph.cu) and must produce the reference's kept pairs (tests/golden/big_window.npz),
+    alone and next to a small window in the same batch; on the tensor cores through the dense Gram build (code 1)."""
+    from mpntrackseg_b200 import ops
     from mpntrackseg_b200.data.mot_graph import build_window_graphs
     c = load_big_case('big_window')
     win, ds, gold = c['win'], c['ds'], c['gold']
@@ -1051,6 +1052,8 @@ def test_window_beyond_5120_nodes_takes_the_general_select_path(engine):
     ref_small = graph_ref.build_graph(small.frame, small.reid, synth.det_columns(small), small.fps, ds)
     for tabs in ([tab], [stab, tab]):
         batch = build_window_graphs(tabs, ds, win.fps, device=dev(), engine=engine)
+        if engine == 'tc':
+            assert ops.LAST_KNN_STATS[0] == 1, ops.LAST_KNN_STATS
         gi = len(tabs) - 1
         g = batch.graph(gi)
         p = g.edge_index.shape[1] // 2

@@ -1,11 +1,11 @@
 """GPU tests of the batched KNN graph build (csrc/knn_graph.cu, csrc/knn_graph_tc.cu) across embedding scale,
 dimension, build gates and degenerate windows, against the exact fp32 build and an fp64 oracle.
 
-The build has four routes; ``ops.LAST_KNN_STATS[0]`` reports which one ran:
+The build has three routes; ``ops.LAST_KNN_STATS[0]`` reports which one ran:
 0 exact fp32 (``engine='fp32'``, a gate that rules the tensor cores out, or the whole-call exact rerun),
-1 dense Gram blocks + fused row select (windows of up to SEL_MAX_N = 5,120 nodes),
-2 thresholded candidate lists (every window >= TG_MIN_TILES * 128 = 1,024 nodes, k <= 64, or k <= CAND_CAP / 4 = 128
-  with MPN_KNN_THRESHOLDED), 3 dense Gram blocks + general select (a window above 5,120 nodes).
+1 dense Gram blocks + row select (its keys in registers up to SEL_MAX_N = 5,120 nodes, re-read from the row above),
+2 thresholded candidate lists (every window >= TG_MIN_TILES * 128 = 1,024 nodes, at most SEL_MAX_N, k <= 64, or
+  k <= CAND_CAP / 4 = 128 with MPN_KNN_THRESHOLDED).
 Each tensor-core route pre-ranks with approximate Gram distances and recomputes exactly every row whose k-th and
 (k+1)-th distances fall inside an error band, so its kept edge set must equal the exact build's.  Every test asserts
 that its case reached the route, gate, fallback or rerun it names.
@@ -27,13 +27,13 @@ import torch.nn.functional as F
 from mpntrackseg_b200 import ops, synth
 from oracle import graph_ref
 
-EXACT, DENSE, THRESHOLDED, GENERAL = 0, 1, 2, 3
+EXACT, DENSE, THRESHOLDED = 0, 1, 2
 EPS = 1e-6                  # the reference's F.pairwise_distance eps
 GAP = 1e-5                  # fp64 relative k-th / (k+1)-th gap above which a row's top-k set is decided
 K = 50
 TS = 128                    # csrc/knn_graph_tc.cu: rows per Gram tile
 TG_MIN_N = 8 * TS           # TG_MIN_TILES * TS: smallest window of the thresholded build
-SEL_MAX_N = 20 * 256        # csrc/knn_graph.cu: largest window of the fused row select
+SEL_MAX_N = 20 * 256        # csrc/knn_graph.cu: largest window whose row select keeps its keys in registers
 CAND_CAP = 512              # candidate list slots per row
 TG_DEFAULT_MAX_K = 64
 MAX_WINDOWS = 65535         # gridDim.y of bit_transpose_kernel / dist_blocks_kernel
@@ -245,15 +245,15 @@ def test_embedding_scale_thresholded_and_dense(norm, monkeypatch):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize('norm', ['raw', 'l2'])
-def test_embedding_scale_general_select(norm, monkeypatch):
-    """A window of 5,200 nodes (above SEL_MAX_N): Gram blocks + the general select, at a few scales."""
+def test_embedding_scale_streamed_row_select(norm, monkeypatch):
+    """A window of 5,200 nodes (above SEL_MAX_N): Gram blocks + the streamed row select, at a few scales."""
     reid, frame = bench_window(seed=12, T=26, D=200)
     assert reid.shape[0] > SEL_MAX_N
     if norm == 'l2':
         reid = F.normalize(reid, dim=1)
     reid, frame, ptr = batch([(reid, frame)])
     report, failed = sweep(reid, frame, ptr, [2.0 ** -20, 2.0 ** -13, 2.0 ** -8, 1.0, 2.0 ** 13],
-                           [('general', None, GENERAL)], monkeypatch)
+                           [('dense', None, DENSE)], monkeypatch)
     assert not failed, '\n'.join(report)
 
 
@@ -304,7 +304,7 @@ def test_unaligned_embeddings_run_exact():
 # ------------------------------------------------------------------ C. build selection
 @pytest.mark.gpu
 @pytest.mark.parametrize('n, code', [(TG_MIN_N - 1, DENSE), (TG_MIN_N, THRESHOLDED), (TG_MIN_N + 1, THRESHOLDED),
-                                     (SEL_MAX_N, THRESHOLDED), (SEL_MAX_N + 1, GENERAL)])
+                                     (SEL_MAX_N, THRESHOLDED), (SEL_MAX_N + 1, DENSE)])
 def test_window_size_gates(n, code):
     reid, frame = sized_window(n, seed=n)
     _, _, ptr = batch([(reid, frame)])
@@ -350,21 +350,27 @@ def test_partial_last_tiles_on_the_thresholded_build():
 
 # ------------------------------------------------------------------ D. degenerate windows on the thresholded build
 @pytest.mark.gpu
+@pytest.mark.parametrize('sizes, code', [((TG_MIN_N,), THRESHOLDED), ((5400, K - 20), DENSE)])
 @pytest.mark.parametrize('recip', [True, False])
-def test_all_identical_embeddings(recip):
-    """Every distance ties: every candidate list overflows CAND_CAP and every row is flagged; the result is the
-    reference's index-ordered top-k (graph_ref on the same inputs)."""
-    reid, frame = sized_window(TG_MIN_N, seed=40)
-    reid = reid[:1].expand_as(reid).contiguous()
-    _, _, ptr = batch([(reid, frame)])
-    got = against_exact(reid, frame, ptr, K, recip, THRESHOLDED)
-    assert got[3][1] == reid.shape[0], got[3]
-    pairs = graph_ref.time_valid_pairs(frame)
-    d = graph_ref.pair_reid_dist(reid.double(), pairs)
-    assert float(d.max()) == float(d.min())
-    keep = graph_ref.knn_keep_mask(d, pairs, reid.shape[0], K, recip, symmetric_edges=False)
-    assert torch.equal(got[0], pairs[:, keep])
+def test_all_identical_embeddings(recip, sizes, code):
+    """Every distance of a window ties and every row with more than k nodes in its window is flagged.  One 1,024-node
+    window: every candidate list overflows CAND_CAP; the result is the reference's index-ordered top-k (graph_ref on
+    the same inputs).  A 5,400-node window next to one smaller than k: the row select that re-reads rows above
+    SEL_MAX_N resolves the ties straddling k by index."""
+    wins = []
+    for i, n in enumerate(sizes):
+        r, f = sized_window(n, seed=40 + i)
+        wins.append((r[:1].expand_as(r).contiguous(), f))
+    reid, frame, ptr = batch(wins)
+    got = against_exact(reid, frame, ptr, K, recip, code)
+    assert got[3][1] == sum(n for n in sizes if n > K), got[3]
     assert torch.equal(got[0], index_order_keep(frame, ptr, K, recip))
+    if len(sizes) == 1:
+        pairs = graph_ref.time_valid_pairs(frame)
+        d = graph_ref.pair_reid_dist(reid.double(), pairs)
+        assert float(d.max()) == float(d.min())
+        keep = graph_ref.knn_keep_mask(d, pairs, reid.shape[0], K, recip, symmetric_edges=False)
+        assert torch.equal(got[0], pairs[:, keep])
 
 
 @pytest.mark.gpu

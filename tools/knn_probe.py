@@ -21,4 +21,4 @@ for it in range(3):
     e1.record()
     torch.cuda.synchronize()
     print('dense' if os.environ.get('MPN_KNN_DENSE') else 'thresholded', 'iter', it, 'ms', round(e0.elapsed_time(e1), 3),
-          'pairs', pairs.shape[1], 'stats [build code (0 exact, 1 dense, 2 thresholded, 3 general), repaired rows]', ops.LAST_KNN_STATS)
+          'pairs', pairs.shape[1], 'stats [build code (0 exact, 1 dense, 2 thresholded), repaired rows]', ops.LAST_KNN_STATS)
