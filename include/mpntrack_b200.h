@@ -160,8 +160,9 @@ int mpn_linear(const float* in, int64_t m, int64_t k, const float* w, const floa
                int64_t o, int relu, float* out, void* stream);
 
 /* models/mpn.py:355 encoder.node_model for the shipped widths K -> 128 -> 32 (K a multiple of 64) on the
- * tcgen05 tensor cores: x [N,K] (already pooled) -> out [N,32] = ReLU(W1 ReLU(W0 x + b0) + b1), fp16
- * hi/lo split operands, fp32 accumulation.  *status != 0: a value left the fp16 range, rerun with
+ * tcgen05 tensor cores: x [N,K] (already pooled, 16-byte aligned) -> out [N,32] = ReLU(W1 ReLU(W0 x + b0) + b1),
+ * fp16 hi/lo split operands, each row of x, W0, W1 and the hidden layer at its own power-of-two scale, fp32
+ * accumulation.  *status != 0: a non-finite value in x or the weights (or an x row beyond 2^73), rerun with
  * mpn_linear.  workspace: mpn_node_encoder_tc_workspace(K) bytes (packed weight image). */
 int64_t mpn_node_encoder_tc_workspace(int64_t k0);
 int mpn_node_encoder_tc(const float* x, int64_t n, int64_t k0, const float* w0, const float* b0,

@@ -9,6 +9,15 @@
 // bytes on an mbarrier); 12 MMAs (128 x 128 x 16, hi*hi + hi*lo + lo*hi) per chunk
 // accumulate in TMEM while the next chunk is being loaded.  The 128 -> 32 layer reuses the accumulator
 // in place as its operand.
+//
+// Every operand row is split at its own power-of-two scale (pack_shift): each output row of W0 and W1 (pack_kernel)
+// and each row of the hidden h (epilogue 1) with its largest |v| in [2^13, 2^14); each row of x with the largest |v|
+// seen so far in [2^10, 2^11): the shift is set by the first nonzero chunk and lowered when a later chunk would pass
+// 2^15, the row's accumulator then rescaled in TMEM by the same power of two (rare: a 16x jump within the row).
+// Unscaled, the low half of a value below 2^-3 is subnormal and carries an absolute error of 2^-25, which the
+// default weights (|w| ~ 0.02 .. 0.1) and small features already reach.  The epilogues multiply the accumulators
+// by the inverse powers of two before adding the biases, so every scaling is exact, the error is relative to
+// ||x_r|| ||w_o|| whatever the magnitudes, and out(x 2^p, b 2^p) = 2^p out(x, b) bit for bit (DESIGN.md section 4).
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -23,8 +32,9 @@ constexpr int SLAB1 = H * 32;                                         // one K=1
 constexpr int CHUNK_BYTES = 2 * (KC / 16) * SLAB1;                    // hi + lo, 4 k-steps = 32 KB
 constexpr int SLAB2 = O * 32;                                         // one K=16 step of W1: 32 rows x 32 B
 constexpr int W2_BYTES = 2 * (H / 16) * SLAB2;                        // 16 KB
-constexpr int F_B0 = 0, F_B1 = H, F_COUNT = H + O;
-constexpr int TAIL_BYTES = W2_BYTES + F_COUNT * 4;                    // W1 image + biases
+// tail floats: biases, then 2^-e of each output row of W0 and W1 (the row was packed times 2^e)
+constexpr int F_B0 = 0, F_B1 = H, F_S0 = H + O, F_S1 = 2 * H + O, F_COUNT = 2 * (H + O);
+constexpr int TAIL_BYTES = W2_BYTES + F_COUNT * 4;                    // W1 image + biases + row scales
 
 constexpr int C_A = 0;            // A operand double buffer: [buf][hi 32 cols | lo 32 cols]
 constexpr int C_D1 = 128;         // 128 accumulator columns, reused in place as the layer-2 operand
@@ -40,31 +50,54 @@ __device__ __forceinline__ int slab_off(int n, int k16) {
   return (n >> 3) * 256 + (k16 >> 3) * 128 + (n & 7) * 16 + (k16 & 7) * 2;
 }
 
-// global image: [K0/64 chunks][hi: 4 slabs | lo: 4 slabs] then the tail (W1 hi slabs, lo slabs, b0, b1)
-__global__ void pack_kernel(const float* __restrict__ w0, const float* __restrict__ b0, const float* __restrict__ w1,
-                            const float* __restrict__ b1, int64_t k0, uint8_t* __restrict__ img) {
-  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nt = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i = tid; i < (int64_t)H * k0; i += nt) {
-    const int n = (int)(i / k0);
-    const int64_t k = i % k0;
-    const float v = w0[i];
-    const __half h = __float2half_rn(v), l = __float2half_rn(v - __half2float(h));
-    const int64_t off = (k / KC) * CHUNK_BYTES + ((k % KC) >> 4) * SLAB1 + slab_off(n, (int)(k & 15));
-    *reinterpret_cast<__half*>(img + off) = h;
-    *reinterpret_cast<__half*>(img + off + (KC / 16) * SLAB1) = l;
+// global image: [K0/64 chunks][hi: 4 slabs | lo: 4 slabs] then the tail (W1 hi slabs, lo slabs, b0, b1, row scales).
+// One CTA per output row (W0 rows 0..127, then W1 rows 0..31): the row's largest |w| gives its shift e, the row is
+// packed times 2^e and 2^-e goes to the tail.  A non-finite weight or bias sets status bit 1.
+__global__ void __launch_bounds__(256) pack_kernel(const float* __restrict__ w0, const float* __restrict__ b0,
+                                                   const float* __restrict__ w1, const float* __restrict__ b1, int64_t k0,
+                                                   uint8_t* __restrict__ img, int32_t* __restrict__ status) {
+  __shared__ float s_max[8];
+  __shared__ int s_fin[8];
+  const int tid = threadIdx.x, lane = tid & 31;
+  const bool layer0 = blockIdx.x < H;
+  const int n = layer0 ? (int)blockIdx.x : (int)blockIdx.x - H;
+  const int64_t len = layer0 ? k0 : H;
+  const float* w = layer0 ? w0 + (int64_t)n * k0 : w1 + (int64_t)n * H;
+  float m = 0.f;
+  bool fin = true;
+  for (int64_t k = tid; k < len; k += 256) {
+    const float a = fabsf(w[k]);
+    m = fmaxf(m, a);
+    fin &= a <= 3.402823466e38f;                                     // false for inf and NaN
   }
+  for (int d = 16; d > 0; d >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, d));
+  fin = __all_sync(0xffffffffu, fin);
+  if (lane == 0) { s_max[tid >> 5] = m; s_fin[tid >> 5] = fin; }
+  __syncthreads();
+  for (int i = 0; i < 8; ++i) { m = fmaxf(m, s_max[i]); fin &= s_fin[i] != 0; }
+  const float bias = layer0 ? b0[n] : b1[n];
+  if (tid == 0 && !(fin && fabsf(bias) <= 3.402823466e38f)) atomicOr(status, 1);
+  const int e = pack_shift(__float_as_uint(m));
+  const float up = pow2i(e);
   uint8_t* tail = img + (k0 / KC) * CHUNK_BYTES;
-  for (int64_t i = tid; i < O * H; i += nt) {
-    const int n = (int)(i / H), k = (int)(i % H);
-    const float v = w1[i];
+  for (int64_t k = tid; k < len; k += 256) {
+    const float v = w[k] * up;
     const __half h = __float2half_rn(v), l = __float2half_rn(v - __half2float(h));
-    const int off = (k >> 4) * SLAB2 + slab_off(n, k & 15);
-    *reinterpret_cast<__half*>(tail + off) = h;
-    *reinterpret_cast<__half*>(tail + off + (H / 16) * SLAB2) = l;
+    const int64_t off = layer0 ? (k / KC) * CHUNK_BYTES + ((k % KC) >> 4) * SLAB1 + slab_off(n, (int)(k & 15))
+                               : (k >> 4) * SLAB2 + slab_off(n, (int)(k & 15));
+    uint8_t* dst = layer0 ? img + off : tail + off;
+    *reinterpret_cast<__half*>(dst) = h;
+    *reinterpret_cast<__half*>(dst + (layer0 ? (KC / 16) * SLAB1 : (H / 16) * SLAB2)) = l;
   }
-  float* ft = reinterpret_cast<float*>(tail + W2_BYTES);
-  for (int64_t i = tid; i < F_COUNT; i += nt) ft[i] = i < H ? b0[i] : b1[i - H];
+  if (tid == 0) {
+    float* ft = reinterpret_cast<float*>(tail + W2_BYTES);
+    ft[(layer0 ? F_B0 : F_B1) + n] = bias;
+    ft[(layer0 ? F_S0 : F_S1) + n] = pow2i(-e);
+  }
 }
+
+constexpr int X_HEADROOM = 3;            // x rows are packed with their largest |v| so far in [2^10, 2^11) ...
+constexpr float X_RESCALE_AT = 32768.f;  // ... until a chunk would reach 2^15
 
 __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const float* __restrict__ x, int64_t n, int64_t k0,
                                                                      const uint8_t* __restrict__ img,
@@ -103,6 +136,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const floa
     int64_t row = t * TS + gt;
     const bool valid = row < n;
     if (!valid) row = n - 1;
+    int sx = 0;                                                      // the row's shift so far
+    float xmax = 0.f;                                                // its largest |x| so far
+    bool early = false;                                              // MMAs of chunk c-1 already waited for
     const float4* xr = reinterpret_cast<const float4*>(x + row * k0);
     auto load_w = [&](int c) {                                       // 32 KB weight chunk: one TMA bulk copy
       if (gt == 0) {
@@ -117,16 +153,29 @@ __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const floa
     for (int c = 0; c < nchunks; ++c) {
       // ---- this chunk's A operand: split the 64 values and store them to TMEM buffer c&1
       const uint32_t abuf = tlane + C_A + (c & 1) * 64;
+      float cmax = 0.f;
+#pragma unroll
+      for (int j = 0; j < KC / 4; ++j)
+        cmax = fmaxf(cmax, fmaxf(fmaxf(fabsf(xv[j].x), fabsf(xv[j].y)), fmaxf(fabsf(xv[j].z), fabsf(xv[j].w))));
+      // the first nonzero chunk sets the shift (the accumulator is still exactly 0); a chunk that would pass 2^15
+      // lowers it, and the accumulator of the chunks before is rescaled to match
+      const bool first = !(xmax > 0.f) && cmax > 0.f;
+      const bool rescale = xmax > 0.f && cmax * pow2i(sx) >= X_RESCALE_AT;
+      const int snew = first || rescale ? pack_shift(__float_as_uint(cmax)) - X_HEADROOM : sx;
+      const float fix = pow2i(snew - sx);
+      sx = snew;
+      xmax = fmaxf(xmax, cmax);
+      const float up = pow2i(sx);
 #pragma unroll
       for (int q = 0; q < KC / 16; ++q) {
         uint32_t hi[8], lo[8];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const float4 v = xv[4 * q + j];
-          split2(v.x, v.y, hi[2 * j], lo[2 * j]);
-          split2(v.z, v.w, hi[2 * j + 1], lo[2 * j + 1]);
-          vmax = __hmax2(vmax, __habs2(*reinterpret_cast<const __half2*>(&hi[2 * j])));
-          vmax = __hmax2(vmax, __habs2(*reinterpret_cast<const __half2*>(&hi[2 * j + 1])));
+          split2(v.x * up, v.y * up, hi[2 * j], lo[2 * j]);
+          split2(v.z * up, v.w * up, hi[2 * j + 1], lo[2 * j + 1]);
+          vmax = __hmax2_nan(vmax, __habs2(*reinterpret_cast<const __half2*>(&hi[2 * j])));
+          vmax = __hmax2_nan(vmax, __habs2(*reinterpret_cast<const __half2*>(&hi[2 * j + 1])));
         }
         tmem_st8(abuf + 8 * q, hi);
         tmem_st8(abuf + 32 + 8 * q, lo);
@@ -134,7 +183,28 @@ __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const floa
       mbar_wait(&wbars[c & 1], wpar[c & 1]); wpar[c & 1] ^= 1;       // this chunk's weights have landed
       tc_wait_st();
       tc_fence_before();
-      named_barrier(1 + g, TS);
+      early = named_barrier_or(1 + g, TS, rescale);                   // never at c = 0: no accumulator yet
+      if (early) {                                                     // wait for chunk c-1, rescale the rows that ask
+        mbar_wait(&bars[(c - 1) & 1], par[(c - 1) & 1]); par[(c - 1) & 1] ^= 1;
+        tc_fence_after();
+        const float f = rescale ? fix : 1.f;
+#pragma unroll 1
+        for (int ch = 0; ch < H / 16; ++ch) {
+          uint32_t acc[16], a[8], b[8];
+          tmem_ld16(tlane + C_D1 + 16 * ch, acc);
+          tc_wait_ld();
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            a[j] = __float_as_uint(__uint_as_float(acc[j]) * f);
+            b[j] = __float_as_uint(__uint_as_float(acc[j + 8]) * f);
+          }
+          tmem_st8(tlane + C_D1 + 16 * ch, a);
+          tmem_st8(tlane + C_D1 + 16 * ch + 8, b);
+        }
+        tc_wait_st();
+        tc_fence_before();
+        named_barrier(1 + g, TS);
+      }
       if (wq == 0) {
         tc_fence_after();
         if (elect_one()) {
@@ -154,17 +224,31 @@ __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const floa
       }
       // ---- next chunk: its buffers were last read by the MMAs of chunk c-1
       if (c + 1 < nchunks) {
-        if (c >= 1) { mbar_wait(&bars[(c - 1) & 1], par[(c - 1) & 1]); par[(c - 1) & 1] ^= 1; }
+        if (c >= 1 && !early) { mbar_wait(&bars[(c - 1) & 1], par[(c - 1) & 1]); par[(c - 1) & 1] ^= 1; }
         load_w(c + 1);
 #pragma unroll
         for (int j = 0; j < KC / 4; ++j) xv[j] = __ldcs(xr + (c + 1) * (KC / 4) + j);
       }
     }
     // drain: the last two commits
-    if (nchunks >= 2) { mbar_wait(&bars[(nchunks - 2) & 1], par[(nchunks - 2) & 1]); par[(nchunks - 2) & 1] ^= 1; }
+    if (nchunks >= 2 && !early) { mbar_wait(&bars[(nchunks - 2) & 1], par[(nchunks - 2) & 1]); par[(nchunks - 2) & 1] ^= 1; }
     mbar_wait(&bars[(nchunks - 1) & 1], par[(nchunks - 1) & 1]); par[(nchunks - 1) & 1] ^= 1;
     tc_fence_after();
-    // ---- epilogue 1: h = ReLU(D1 + b0) -> layer-2 operand in place
+    // ---- epilogue 1: h = ReLU(D1 * 2^-(sx + e_o) + b0) -> layer-2 operand in place, split at the row's own shift.
+    // Sweep 1 finds the row's largest h, sweep 2 recomputes the same values, scales them by 2^sh and splits them.
+    const float down = pow2i(-sx);
+    float hmax = 0.f;
+#pragma unroll 1
+    for (int ch = 0; ch < H / 16; ++ch) {
+      uint32_t acc[16];
+      tmem_ld16(tlane + C_D1 + 16 * ch, acc);
+      tc_wait_ld();
+#pragma unroll
+      for (int j = 0; j < 16; ++j)
+        hmax = fmaxf(hmax, fmaf(__uint_as_float(acc[j]), down * s_f[F_S0 + 16 * ch + j], s_f[F_B0 + 16 * ch + j]));
+    }
+    const int sh = pack_shift(__float_as_uint(hmax));
+    const float hup = pow2i(sh), hdown = pow2i(-sh);
 #pragma unroll
     for (int ch = 0; ch < H / 16; ++ch) {
       uint32_t acc[16];
@@ -173,9 +257,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const floa
       uint32_t hi[8], lo[8];
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
-        split2_relu(__uint_as_float(acc[2 * j]) + s_f[F_B0 + 16 * ch + 2 * j],
-                    __uint_as_float(acc[2 * j + 1]) + s_f[F_B0 + 16 * ch + 2 * j + 1], hi[j], lo[j]);
-        vmax = __hmax2(vmax, *reinterpret_cast<const __half2*>(&hi[j]));
+        const int o = 16 * ch + 2 * j;
+        split2_relu(fmaf(__uint_as_float(acc[2 * j]), down * s_f[F_S0 + o], s_f[F_B0 + o]) * hup,
+                    fmaf(__uint_as_float(acc[2 * j + 1]), down * s_f[F_S0 + o + 1], s_f[F_B0 + o + 1]) * hup, hi[j], lo[j]);
+        vmax = __hmax2_nan(vmax, *reinterpret_cast<const __half2*>(&hi[j]));
       }
       tmem_st8(tlane + C_D1 + 16 * ch, hi);
       tmem_st8(tlane + C_D1 + 16 * ch + 8, lo);
@@ -202,7 +287,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const floa
     }
     mbar_wait(&bars[0], par[0]); par[0] ^= 1;
     tc_fence_after();
-    // ---- epilogue 2: x_init = ReLU(D2 + b1)
+    // ---- epilogue 2: x_init = ReLU(D2 * 2^-(sh + e_o) + b1)
 #pragma unroll
     for (int ch = 0; ch < O / 16; ++ch) {
       uint32_t acc[16];
@@ -210,18 +295,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) node_encoder_tc_kernel(const floa
       tc_wait_ld();
       if (valid) {
         float4* dst = reinterpret_cast<float4*>(out + (t * TS + gt) * O + 16 * ch);
+        float v[16];
 #pragma unroll
-        for (int j = 0; j < 4; ++j)
-          dst[j] = make_float4(fmaxf(__uint_as_float(acc[4 * j]) + s_f[F_B1 + 16 * ch + 4 * j], 0.f),
-                               fmaxf(__uint_as_float(acc[4 * j + 1]) + s_f[F_B1 + 16 * ch + 4 * j + 1], 0.f),
-                               fmaxf(__uint_as_float(acc[4 * j + 2]) + s_f[F_B1 + 16 * ch + 4 * j + 2], 0.f),
-                               fmaxf(__uint_as_float(acc[4 * j + 3]) + s_f[F_B1 + 16 * ch + 4 * j + 3], 0.f));
+        for (int j = 0; j < 16; ++j)
+          v[j] = fmaxf(fmaf(__uint_as_float(acc[j]), hdown * s_f[F_S1 + 16 * ch + j], s_f[F_B1 + 16 * ch + j]), 0.f);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) dst[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
       }
     }
     tc_fence_before();
     named_barrier(1 + g, TS);                                        // D2 / A buffers are free for the next tile
   }
   {
+    // scaled operands stay below 2^15 and the max keeps NaN: only a non-finite x (or a row beyond the shift's reach,
+    // |v| >= 2^73) gets here
     const uint32_t w = *reinterpret_cast<const uint32_t*>(&vmax);
     if ((w & 0x7FFFu) >= 0x7BFFu || ((w >> 16) & 0x7FFFu) >= 0x7BFFu) atomicOr(status, 1);
   }
@@ -254,7 +341,7 @@ int mpn_node_encoder_tc(const float* x, int64_t n, int64_t k0, const float* w0, 
   uint8_t* img = static_cast<uint8_t*>(ws);
   MPN_CUDA(cudaFuncSetAttribute(enc::node_encoder_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 enc::SMEM_BYTES));
-  enc::pack_kernel<<<64, 256, 0, s>>>(w0, b0, w1, b1, k0, img); count_launch();
+  enc::pack_kernel<<<enc::H + enc::O, 256, 0, s>>>(w0, b0, w1, b1, k0, img, status); count_launch();
   const int64_t tiles = ceil_div(n, enc::TS);
   int grid = (int)std::min<int64_t>(ceil_div(tiles, 2), sm_count());
   enc::node_encoder_tc_kernel<<<grid, enc::NTHREADS, enc::SMEM_BYTES, s>>>(x, n, k0, img, out, status); count_launch();

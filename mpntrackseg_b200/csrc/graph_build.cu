@@ -45,6 +45,12 @@ __global__ void time_valid_kernel(const int64_t* __restrict__ frame, int64_t n,
 
 // ------------------------------------------------------------------ per-pair ReID distance
 // One warp per pair; lane-strided partial sums of ((a-b)+eps)^2, then a fixed xor tree.
+// dim % 4 == 0: lane q sums the groups of four 4q..4q+3, q += 32, read as float4 when `reid` is 16-byte aligned and
+// as four scalars otherwise (a contiguous view at an odd element offset), in the same order: the same bits either way.
+__device__ __forceinline__ float4 load4(const float* p, bool aligned) {
+  return aligned ? __ldg(reinterpret_cast<const float4*>(p)) : make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3));
+}
+
 __global__ void pair_dist_kernel(const float* __restrict__ reid, int64_t dim,
                                  const int64_t* __restrict__ row, const int64_t* __restrict__ col,
                                  int64_t npairs, float* __restrict__ out) {
@@ -52,15 +58,14 @@ __global__ void pair_dist_kernel(const float* __restrict__ reid, int64_t dim,
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const float eps = 1e-6f;
+  const bool aligned = (reinterpret_cast<uintptr_t>(reid) & 15) == 0;
   for (int64_t p = warp; p < npairs; p += nwarps) {
     const float* a = reid + row[p] * dim;
     const float* b = reid + col[p] * dim;
     float acc = 0.f;
     if ((dim & 3) == 0) {
-      const float4* a4 = reinterpret_cast<const float4*>(a);
-      const float4* b4 = reinterpret_cast<const float4*>(b);
       for (int64_t q = lane; q < (dim >> 2); q += 32) {
-        const float4 u = __ldg(a4 + q), v = __ldg(b4 + q);
+        const float4 u = load4(a + 4 * q, aligned), v = load4(b + 4 * q, aligned);
         float d;
         d = (u.x - v.x) + eps; acc = fmaf(d, d, acc);
         d = (u.y - v.y) + eps; acc = fmaf(d, d, acc);

@@ -30,18 +30,6 @@ __device__ __forceinline__ int slab_off(int n, int k16) {
   return (n >> 3) * 256 + (k16 >> 3) * 128 + (n & 7) * 16 + (k16 & 7) * 2;
 }
 
-// Power-of-two pre-scale of a window whose largest |v| is `amax_bits` (fp32 bits): 2^p * max |v| lies in
-// [2^13, 2^14), so every split operand keeps a resolution of 2^-25 relative to 2^13 ... 2^14 of the window's
-// largest value, and hi stays far from the fp16 maximum.  |p| <= 62 keeps 2^-2p a normal fp32 number.
-constexpr int PACK_SHIFT_MAX = 62;
-__device__ __forceinline__ int pack_shift(uint32_t amax_bits) {
-  const float m = __uint_as_float(amax_bits);
-  if (!(m > 0.f) || !isfinite(m)) return 0;                      // all-zero window (or an overflow the caller reruns)
-  int e;
-  frexpf(m, &e);                                                 // m in [2^(e-1), 2^e)
-  return max(-PACK_SHIFT_MAX, min(PACK_SHIFT_MAX, 14 - e));
-}
-
 // warp per node: max |v| of its row into its window's entry (non-negative floats order like their bits).
 __global__ void window_absmax_kernel(const float* __restrict__ reid, int64_t dim, const int64_t* __restrict__ gptr,
                                      int64_t num_graphs, int64_t num_nodes, uint32_t* __restrict__ win_amax) {

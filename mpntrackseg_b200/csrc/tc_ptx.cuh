@@ -159,6 +159,15 @@ __device__ __forceinline__ bool elect_one() {
 __device__ __forceinline__ void named_barrier(int id, int threads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
 }
+// named barrier that also returns whether `v` was true in any participating thread
+__device__ __forceinline__ bool named_barrier_or(int id, int threads, bool v) {
+  uint32_t r;
+  asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.u32 q, %1, 0;\n\tbar.red.or.pred p, %2, %3, q;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+               : "=r"(r)
+               : "r"((uint32_t)v), "r"(id), "r"(threads)
+               : "memory");
+  return r != 0;
+}
 
 // ---------------------------------------------------------------- fp16 hi/lo split
 // v ~= hi + lo with hi = fp16(v), lo = fp16(v - hi): 22 significant bits.
@@ -176,6 +185,20 @@ __device__ __forceinline__ void split2_relu(float a, float b, uint32_t& hi, uint
   const float2 hf = __half22float2(*reinterpret_cast<const __half2*>(&hi));
   asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(b - hf.y), "f"(a - hf.x));
 }
+
+// Power-of-two pre-scale of an operand row (or block) whose largest |v| is `amax_bits` (fp32 bits): 2^p * max |v|
+// lies in [2^13, 2^14), so every split2 operand keeps a resolution of 2^-25 relative to 2^13 ... 2^14 of the
+// largest value, and hi stays far from the fp16 maximum.  |p| <= 62 keeps 2^-2p a normal fp32 number.
+constexpr int PACK_SHIFT_MAX = 62;
+__device__ __forceinline__ int pack_shift(uint32_t amax_bits) {
+  const float m = __uint_as_float(amax_bits);
+  if (!(m > 0.f) || !isfinite(m)) return 0;                      // all zero (or non-finite: the caller's status says so)
+  int e;
+  frexpf(m, &e);                                                 // m in [2^(e-1), 2^e)
+  return max(-PACK_SHIFT_MAX, min(PACK_SHIFT_MAX, 14 - e));
+}
+// 2^e for -126 <= e <= 127 (exact)
+__device__ __forceinline__ float pow2i(int e) { return __int_as_float((e + 127) << 23); }
 
 // ---------------------------------------------------------------- fp16 hi/lo split with a lifted low part
 // v ~= hi + lo' * 2^-LO_SHIFT with lo' = fp16((v - hi) * 2^LO_SHIFT).  The low part is then a NORMAL fp16 number whenever

@@ -238,9 +238,10 @@ def linear(inp, weight, bias, relu):
 
 def node_encoder(x, weights, biases, engine=None, status=None):
     """encoder.node_model on pooled features x [N, K].  The shipped K -> 128 -> 32 stack runs as one
-    tcgen05 kernel (engine 'tc' / 'auto'); other widths, engine 'fp32' and fp16-range overflow use the
-    fp32 Linear kernel chain.  models/mpn.py:355
-    status: optional int32[1] device tensor; if given the overflow flag is left there for the caller to
+    tcgen05 kernel (engine 'tc' / 'auto'; every operand row split at its own power-of-two scale, so the error is
+    relative at any magnitude); other widths, x off 16-byte alignment, engine 'fp32' and non-finite features or
+    weights use the fp32 Linear kernel chain.  models/mpn.py:355
+    status: optional int32[1] device tensor; if given the non-finite flag is left there for the caller to
     check (no host sync here) and no fallback is attempted."""
     engine = engine or default_engine()
     x = _req(x, torch.float32, 'x')
@@ -260,8 +261,8 @@ def node_encoder(x, weights, biases, engine=None, status=None):
         if deferred or (engine == 'tc' and not STRICT_TC_STATUS) or int(status.item()) == 0:
             return out
         if engine == 'tc':
-            raise OverflowError('node_encoder_tc: a value left the fp16 range; use engine="fp32"')
-        warnings.warn('mpntrackseg_b200: node features outside the fp16 range, rerunning the encoder on the fp32 kernels')
+            raise OverflowError('node_encoder_tc: non-finite node features or encoder weights; use engine="fp32"')
+        warnings.warn('mpntrackseg_b200: non-finite node features or encoder weights, rerunning the encoder on the fp32 kernels')
     h = x
     for w, b in zip(ws_, bs_):
         h = linear(h, w, b, relu=w.shape[0] != 1)
