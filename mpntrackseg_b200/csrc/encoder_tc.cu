@@ -46,10 +46,6 @@ constexpr int SM_BAR = (SM_TAIL + TAIL_BYTES + 127) / 128 * 128;      // u64 bar
 constexpr int SM_TMEM = SM_BAR + 8 * 8;
 constexpr int SMEM_BYTES = SM_TMEM + 16;
 
-__device__ __forceinline__ int slab_off(int n, int k16) {
-  return (n >> 3) * 256 + (k16 >> 3) * 128 + (n & 7) * 16 + (k16 & 7) * 2;
-}
-
 // global image: [K0/64 chunks][hi: 4 slabs | lo: 4 slabs] then the tail (W1 hi slabs, lo slabs, b0, b1, row scales).
 // One CTA per output row (W0 rows 0..127, then W1 rows 0..31): the row's largest |w| gives its shift e, the row is
 // packed times 2^e and 2^-e goes to the tail.  A non-finite weight or bias sets status bit 1.

@@ -26,10 +26,6 @@ constexpr int TS = 128, KC = 64;
 constexpr int SLAB = TS * 32;                               // one K=16 step of a 128-row B tile
 constexpr int CHUNK_BYTES = 2 * (KC / 16) * SLAB;           // hi + lo: 32 KB
 
-__device__ __forceinline__ int slab_off(int n, int k16) {
-  return (n >> 3) * 256 + (k16 >> 3) * 128 + (n & 7) * 16 + (k16 & 7) * 2;
-}
-
 // warp per node: max |v| of its row into its window's entry (non-negative floats order like their bits).
 __global__ void window_absmax_kernel(const float* __restrict__ reid, int64_t dim, const int64_t* __restrict__ gptr,
                                      int64_t num_graphs, int64_t num_nodes, uint32_t* __restrict__ win_amax) {

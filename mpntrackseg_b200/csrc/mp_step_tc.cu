@@ -2,8 +2,9 @@
 //
 // One 128-edge tile = one M=128 MMA tile: TMEM lane i <-> edge slot i <-> epilogue thread i.
 // The four dense layers of a step (edge MLP 160->80->16, flow MLP 80->56->32) run as
-// tcgen05.mma kind::f16 with the ACTIVATIONS in TMEM (A operand, written by the epilogue
-// threads with tcgen05.st) and the WEIGHTS resident in shared memory (B operand, K-major).
+// tcgen05.mma kind::f16 with the ACTIVATIONS as the A operand (in TMEM, written by the epilogue
+// threads with tcgen05.st; the gathered x[col] rows in shared memory, written by TMA) and the
+// WEIGHTS resident in shared memory (B operand, K-major).
 // Precision: every operand is split v ~= hi + lo in fp16 (22 significant bits; the low part is stored lifted by
 // 2^10 so that it stays a normal number, tc_ptx.cuh "lifted low part") and each layer issues lo*hi + hi*lo for
 // all K steps, folds them in with the accumulator input scale 2^-10, then hi*hi, with fp32 accumulation in TMEM -- single-pass bf16/tf32 breaks
@@ -15,18 +16,18 @@
 //   (fp32, computed by the node kernel), added in the first epilogue.
 //
 // State lives in HBM already split: per node 128 B = [hi(32 halfs) | lo(32 halfs)], per edge
-// 64 B = [hi(16) | lo(16)], so loads are plain copies into TMEM and the bytes per edge-update
-// stay at 200.
+// 64 B = [hi(16) | lo(16)], so loads are plain copies into the operands and the bytes per
+// edge-update stay at 200.
 //
-// Warp roles (512 threads, 1 CTA / SM): two groups of 8 warps; each group keeps one tile in flight
-// and owns 256 of the 512 TMEM columns.  Every edge row is served by two threads (halves A and B of
-// the group) that split the columns of each epilogue.  After the group's 256 threads have written a
-// layer's operand, an elected lane of the group's first warp issues that layer's MMAs and commits
-// them to the group's mbarrier; while one group runs an epilogue the tensor core runs the other
-// group's layer.  Operand rows of the next tile are staged with cp.async during the current one,
-// the per-row message sums of the previous tile run under the current tile's first layer.
+// Warp roles (768 threads, 1 CTA / SM): three groups of 8 warps; each group keeps one tile in flight
+// and owns 144 of the 512 TMEM columns and 48 KB of shared memory.  Every edge row is served by two
+// threads (halves A and B of the group) that split the columns of each epilogue.  After the group's
+// 256 threads have written a layer's operand, an elected lane of the group's first warp issues that
+// layer's MMAs and commits them to the group's mbarrier; while one group runs an epilogue the tensor
+// core runs another group's layer.  The x[col] rows of the next tile are gathered by TMA during the
+// current one, and its layer 1 is issued as soon as the current tile's layer 4 has retired, so the
+// last epilogue and the per-row message sums run under it.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "tc_ptx.cuh"
@@ -60,10 +61,6 @@ constexpr int NOFF_PWH = NOFF_NWL + NW_KS * NW_SLAB, NOFF_PWL = NOFF_PWH + PW_KS
 constexpr int NOFF_F32 = NOFF_PWL + PW_KS * PW_SLAB;       // bn[32]
 constexpr int NIMG_BYTES = (NOFF_F32 + DN * 4 + 127) / 128 * 128;
 
-__device__ __forceinline__ int slab_off(int n, int k16) {           // byte offset inside a slab
-  return (n >> 3) * 256 + (k16 >> 3) * 128 + (n & 7) * 16 + (k16 & 7) * 2;
-}
-
 // =================================================================== range bookkeeping
 // Per forward: sched[t] = s_t (exponent of the step's scale), amax[t] = float bits of the largest true activation
 // the edge kernel of step t saw, xmax[t] = largest |x_lat| consumed by step t (t = 1..num_steps; all zeroed at start).
@@ -82,16 +79,15 @@ constexpr int INIT_SHIFT = 8;                // the constant x_init / e_init row
 // a B200).  Such a step sets status bit 2, which sends engine 'auto' to the fp32 kernels like an fp16 overflow.
 constexpr int S_RESOLVED = 17;
 constexpr int FLOW_SHIFT = 7;                // a flow vector sums up to ~100 messages: operand scale 2^-(s_t + 7)
-__device__ __forceinline__ float pow2i(int e) { return __int_as_float((127 + e) << 23); }   // 2^e, |e| <= 126
 // s_{t+1} from what is known when the node kernel of step t starts: the edge kernel's activation maximum of step t
 // and the node-state maxima of steps t and t-1 (their ratio predicts the growth of the state being produced).
-__device__ __forceinline__ int scale_for(float a_t, float x_t, float x_tm1, float target) {
+__device__ __forceinline__ int scale_for(float a_t, float x_t, float x_tm1) {
   float growth = x_tm1 > 0.f ? x_t / x_tm1 : 4.f;
   growth = fminf(fmaxf(growth, 1.f), 64.f);
   const float lag = fmaxf(a_t, x_t * growth);
-  if (!(lag > target)) return 0;
+  if (!(lag > SCALE_TARGET)) return 0;
   int e;
-  frexpf(lag / target, &e);             // lag / target = m * 2^e, m in [0.5, 1)
+  frexpf(lag / SCALE_TARGET, &e);       // lag / target = m * 2^e, m in [0.5, 1)
   return e > 100 ? 100 : e;
 }
 __device__ __forceinline__ void atomic_max_f32(uint32_t* addr, float v) {   // v >= 0: integer order = float order
@@ -102,7 +98,7 @@ __device__ __forceinline__ void atomic_max_f32(uint32_t* addr, float v) {   // v
 // =================================================================== weight packing (once per forward)
 // One image per direction (flow_out / flow_in); layers 1-2 and the classifier are shared.
 __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ img_out, uint8_t* __restrict__ img_in,
-                                    uint8_t* __restrict__ img_node, int cls_in_l3, int32_t* __restrict__ status) {
+                                    uint8_t* __restrict__ img_node, int32_t* __restrict__ status) {
   int bad = 0;                       // a weight whose fp16 image (x 2^INIT_SHIFT for the constant-row slabs) is not finite
   auto fits = [&](float v) { if (!(fabsf(v) * pow2i(INIT_SHIFT) < 65000.f)) bad = 1; };
   {
@@ -146,10 +142,10 @@ __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ im
     }
     for (int i = tid; i < FHP * 80; i += nt) {           // flow layer 0 (rows padded 56 -> 64)
       const int n = i / 80, k = i % 80;
-      // rows 56..63 are padding for the flow MLP; variant 3 puts the classifier's first layer there (it reads
+      // rows 56..63 are padding for the flow MLP; the edge kernel puts the classifier's first layer there (it reads
       // only the e' K step, columns 64..79)
       float v = n < FH ? f0[n * 80 + k] : 0.f;
-      if (cls_in_l3 && n >= FH && k >= 64) v = w.cls_w0[(n - FH) * DE + (k - 64)];
+      if (n >= FH && k >= 64) v = w.cls_w0[(n - FH) * DE + (k - 64)];
       put(OFF_L3H, OFF_L3L, L3_SLAB, n, k, v);
     }
     for (int i = tid; i < DN * FHP; i += nt) {           // flow layer 1 (K padded 56 -> 64)
@@ -231,188 +227,9 @@ __global__ void __launch_bounds__(256) prep_nodes_kernel(const float* __restrict
 // Per step: x' = ReLU(Wn [flow_in | flow_out] + bn)  (models/mpn.py:97-99), then the split copy of
 // x' for the next step's gathers and prow[r] = pinit[r] + W0[:, 32:64] x'.
 //
-// A warp takes NODE_NB = 8 consecutive nodes at a time, lane = output feature.  The 8 nodes' input vectors sit in a
-// per-warp shared-memory tile [input][node] and are read back as 16-byte broadcasts, so every weight (node Linear: in
-// registers; prow: one shared-memory load) is used for 8 nodes, and the products run as packed FFMA2 (two nodes per
-// instruction, the weight as the scalar operand): ~120 instructions per node instead of ~300 with a node per warp.
-constexpr int NODE_NB = 4;
-__device__ __forceinline__ float2 ffma2(float2 a, float w, float2 c) {
-  unsigned long long ra, rw, rc, rd;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a.x), "f"(a.y));
-  asm("mov.b64 %0, {%1, %1};" : "=l"(rw) : "f"(w));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(rc) : "f"(c.x), "f"(c.y));
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(rd) : "l"(ra), "l"(rw), "l"(rc));
-  float2 d;
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(d.x), "=f"(d.y) : "l"(rd));
-  return d;
-}
-
-__global__ void __launch_bounds__(256, 3) node_tc_kernel(const int32_t* __restrict__ out_ptr, const int32_t* __restrict__ in_ptr,
-                                                         int64_t num_nodes, int64_t num_out, int32_t chunks_out,
-                                                         int chunk_shift, const float* __restrict__ flow, const float* __restrict__ part,
-                                                         const float* __restrict__ node_w, const float* __restrict__ node_b,
-                                                         const float* __restrict__ w0, const float* __restrict__ pinit,
-                                                         __half* __restrict__ xl_next, float* __restrict__ prow,
-                                                         float* __restrict__ x_out, int32_t step, int32_t* __restrict__ sched,
-                                                         const uint32_t* __restrict__ amax, uint32_t* __restrict__ xmax,
-                                                         float scale_target, int32_t agg, int32_t* __restrict__ status) {
-  __shared__ float s_w0[DN * EH];                                   // [i][o] over W0 columns 32..63
-  __shared__ float s_wn[2 * DN * DN];                               // node Linear, [in][out]
-  __shared__ __align__(16) float s_in[8][2 * DN][NODE_NB];          // per warp: [input feature][node]
-  __shared__ __align__(16) float s_x[8][DN][NODE_NB];               // per warp: x' [feature][node]
-  for (int idx = threadIdx.x; idx < EH * DN; idx += blockDim.x) {
-    const int o = idx / DN, i = idx - o * DN;
-    s_w0[i * EH + o] = w0[o * 160 + 32 + i];
-  }
-  for (int idx = threadIdx.x; idx < 2 * DN * DN; idx += blockDim.x) {
-    const int o = idx / (2 * DN), i = idx - o * 2 * DN;
-    s_wn[i * DN + o] = node_w[idx];
-  }
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const float bn = node_b[lane];
-  __syncthreads();
-  const int64_t warp = (int64_t)blockIdx.x * 8 + wib;
-  const int64_t nwarps = (int64_t)gridDim.x * 8;
-  const int o2 = lane + 64 < EH ? lane + 64 : lane;                  // lanes >= 16 have no third output (result unused)
-  int ovf = 0;
-  // scale of the step that will consume this kernel's outputs (x_lat rows and prow are written pre-scaled)
-  const int s_next = scale_for(__uint_as_float(amax[step]), __uint_as_float(xmax[step]),
-                               step > 1 ? __uint_as_float(xmax[step - 1]) : 0.f, scale_target);
-  const float sig_next = pow2i(-s_next);
-  if (blockIdx.x == 0 && threadIdx.x == 0) sched[step + 1] = s_next;
-  float mx = 0.f;
-
-  // One direction's flow vector of a node: the row sum written by the edge kernel (row inside one 16-slot granule), or
-  // its granule partials added in granule order.  Branch-free: every piece is an unconditional load from a valid
-  // address (masked to 0 when absent), so the loads of all nodes of the group are in flight together; only rows that
-  // span more than four granules (degree > 48) take the loop.
-  struct FlowReq { float v0, v1, v2, v3, inv_cnt; int64_t ca, cb; };
-  const int64_t gmask = ((int64_t)1 << chunk_shift) - 1;
-  auto issue_flow = [&](int64_t r, int d, int64_t s0, int64_t s1, bool live) {
-    const int64_t seg_base = d == 0 ? num_out : 0;
-    const int64_t chunk_off = d == 0 ? chunks_out : 0;
-    const bool has = live && s1 > s0;
-    const int64_t rel0 = s0 - seg_base;
-    const int64_t ca = rel0 >> chunk_shift, cb = has ? (s1 - 1 - seg_base) >> chunk_shift : ca;
-    const int64_t more = cb - ca;
-    const bool single = more == 0;
-    const bool first_in_chunk = (rel0 & gmask) == 0;
-    const float* p0 = single ? flow + r * 2 * DN + d * DN : part + ((chunk_off + ca) * 2 + (first_in_chunk ? 0 : 1)) * DN;
-    const float* pp = part + ((chunk_off + ca + 1) * 2) * DN;
-    FlowReq q;
-    q.v0 = (has ? p0 : flow)[lane];
-    q.v1 = (has && more >= 1 ? pp : flow)[lane];
-    q.v2 = (has && more >= 2 ? pp + 2 * DN : flow)[lane];
-    q.v3 = (has && more >= 3 ? pp + 4 * DN : flow)[lane];
-    q.v0 = has ? q.v0 : 0.f;
-    q.v1 = has && more >= 1 ? q.v1 : 0.f;
-    q.v2 = has && more >= 2 ? q.v2 : 0.f;
-    q.v3 = has && more >= 3 ? q.v3 : 0.f;
-    q.ca = chunk_off + ca; q.cb = chunk_off + cb;
-    q.inv_cnt = has ? 1.f / (float)(s1 - s0) : 1.f;                    // scatter_mean: / max(count, 1)
-    return q;
-  };
-  auto finish_flow = [&](const FlowReq& q) {
-    // + 0.f / max(., 0.f) are exact on the non-negative messages: same results as the piecewise form
-    float v = agg == 2 ? fmaxf(fmaxf(q.v0, q.v1), fmaxf(q.v2, q.v3)) : ((q.v0 + q.v1) + q.v2) + q.v3;
-    for (int64_t t = q.ca + 4; t <= q.cb; ++t) { const float u = part[(t * 2) * DN + lane]; v = agg == 2 ? fmaxf(v, u) : v + u; }
-    return agg == 1 ? v * q.inv_cnt : v;
-  };
-  auto load_ptrs = [&](int64_t r0, int cnt) {
-    // row pointers of the group's nodes (+1): lanes 0..NB hold in_ptr, lanes 16..16+NB out_ptr
-    int32_t pv = 0;
-    if (r0 < num_nodes && (lane & 15) <= cnt) pv = lane < 16 ? in_ptr[r0 + lane] : out_ptr[r0 + lane - 16];
-    return pv;
-  };
-  auto group_cnt = [&](int64_t r0) { return (int)(num_nodes - r0 < NODE_NB ? (num_nodes - r0 > 0 ? num_nodes - r0 : 0) : NODE_NB); };
-
-  float (*vin)[NODE_NB] = s_in[wib];
-  float (*vx)[NODE_NB] = s_x[wib];
-  int32_t pv = load_ptrs(warp * NODE_NB, group_cnt(warp * NODE_NB));
-  for (int64_t r0 = warp * NODE_NB; r0 < num_nodes; r0 += nwarps * NODE_NB) {
-    const int cnt = group_cnt(r0);
-    FlowReq qi[NODE_NB], qo[NODE_NB];
-#pragma unroll
-    for (int j = 0; j < NODE_NB; ++j) {
-      const int32_t i0 = __shfl_sync(0xffffffffu, pv, j), i1 = __shfl_sync(0xffffffffu, pv, j + 1);
-      const int32_t q0 = __shfl_sync(0xffffffffu, pv, 16 + j), q1 = __shfl_sync(0xffffffffu, pv, 17 + j);
-      qi[j] = issue_flow(r0 + j, 0, i0, i1, j < cnt);                   // flow_in
-      qo[j] = issue_flow(r0 + j, 1, q0, q1, j < cnt);                   // flow_out
-    }
-    // hoisted-term inputs of the group's nodes (independent loads, in flight with the flow pieces)
-    float2 pa[3][NODE_NB / 2];
-#pragma unroll
-    for (int q = 0; q < 3; ++q) {
-      const int o = q < 2 ? lane + 32 * q : o2;
-#pragma unroll
-      for (int j = 0; j < NODE_NB; j += 2) {
-        pa[q][j >> 1].x = pinit[(j < cnt ? r0 + j : 0) * EH + o];
-        pa[q][j >> 1].y = pinit[(j + 1 < cnt ? r0 + j + 1 : 0) * EH + o];
-      }
-    }
-    pv = load_ptrs(r0 + nwarps * NODE_NB, group_cnt(r0 + nwarps * NODE_NB));   // next group's pointers, one group ahead
-    float fi[NODE_NB], fo[NODE_NB];
-#pragma unroll
-    for (int j = 0; j < NODE_NB; ++j) { fi[j] = finish_flow(qi[j]); fo[j] = finish_flow(qo[j]); }
-    __syncwarp();                                                       // the previous group's reads of the tiles are done
-    *reinterpret_cast<float4*>(&vin[lane][0]) = make_float4(fi[0], fi[1], fi[2], fi[3]);
-    *reinterpret_cast<float4*>(&vin[DN + lane][0]) = make_float4(fo[0], fo[1], fo[2], fo[3]);
-    __syncwarp();
-    // ---- node Linear 64 -> 32 for the group's nodes
-    float2 acc[NODE_NB / 2];
-#pragma unroll
-    for (int h = 0; h < NODE_NB / 2; ++h) acc[h] = make_float2(bn, bn);
-#pragma unroll
-    for (int i = 0; i < 2 * DN; ++i) {
-      const float4 va = *reinterpret_cast<const float4*>(&vin[i][0]);
-      const float w = s_wn[i * DN + lane];
-      acc[0] = ffma2(make_float2(va.x, va.y), w, acc[0]);
-      acc[1] = ffma2(make_float2(va.z, va.w), w, acc[1]);
-    }
-    float xn[NODE_NB];
-#pragma unroll
-    for (int h = 0; h < NODE_NB / 2; ++h) { xn[2 * h] = fmaxf(acc[h].x, 0.f); xn[2 * h + 1] = fmaxf(acc[h].y, 0.f); }
-    *reinterpret_cast<float4*>(&vx[lane][0]) = make_float4(xn[0], xn[1], xn[2], xn[3]);
-#pragma unroll
-    for (int j = 0; j < NODE_NB; ++j) {
-      if (j < cnt) {
-        if (x_out != nullptr) x_out[(r0 + j) * DN + lane] = xn[j];
-        mx = fmaxf(mx, xn[j]);
-        store_split_row(xl_next + (r0 + j) * 64, lane, xn[j] * sig_next, &ovf);
-      }
-    }
-    __syncwarp();
-    // ---- prow = pinit + W0[:, 32:64] x' for the group's nodes (80 outputs: lane, lane + 32, lane + 64)
-#pragma unroll 8
-    for (int i = 0; i < DN; ++i) {
-      const float4 va = *reinterpret_cast<const float4*>(&vx[i][0]);
-      const float w_0 = s_w0[i * EH + lane], w_1 = s_w0[i * EH + lane + 32], w_2 = s_w0[i * EH + o2];
-      const float ws[3] = {w_0, w_1, w_2};
-#pragma unroll
-      for (int q = 0; q < 3; ++q) {
-        pa[q][0] = ffma2(make_float2(va.x, va.y), ws[q], pa[q][0]);
-        pa[q][1] = ffma2(make_float2(va.z, va.w), ws[q], pa[q][1]);
-      }
-    }
-#pragma unroll
-    for (int q = 0; q < 3; ++q) {
-      const int o = lane + 32 * q;
-      if (o < EH) {
-#pragma unroll
-        for (int j = 0; j < NODE_NB; j += 2) {
-          if (j < cnt) prow[(r0 + j) * EH + o] = pa[q][j >> 1].x * sig_next;
-          if (j + 1 < cnt) prow[(r0 + j + 1) * EH + o] = pa[q][j >> 1].y * sig_next;
-        }
-      }
-    }
-  }
-  atomic_max_f32(xmax + step + 1, mx);
-  if (ovf) atomicOr(status, 1);
-}
-
-// ---- the same node update on the tensor cores (default).  Tile = 128 nodes, TMEM lane = node = thread; two groups of
-// 4 warps per CTA, one tile in flight each.  A thread gathers its node's two flow vectors (the row sum, or the granule
-// partials added in granule order), splits them into the A operand in TMEM, the node Linear runs as 12 MMAs (N = 32),
+// Tile = 128 nodes, TMEM lane = node = thread; two groups of 4 warps per CTA, one tile in flight each.  A thread
+// gathers its node's two flow vectors (the row sum, or the granule partials added in granule order), splits them
+// into the A operand in TMEM, the node Linear runs as 12 MMAs (N = 32),
 // the epilogue writes x' (fp32 on the last step, split rows in the next step's scale) and leaves the scaled split x'
 // in TMEM as the A operand of the hoisted row term (6 MMAs, N = 80), whose epilogue adds pinit and stores prow.
 constexpr int NT2_THREADS = 256;
@@ -424,7 +241,7 @@ __global__ void __launch_bounds__(NT2_THREADS, 1) node_tc2_kernel(
     int32_t chunks_out, int chunk_shift, const float* __restrict__ flow, const float* __restrict__ part,
     const uint8_t* __restrict__ wimg, const float* __restrict__ pinit, uint4* __restrict__ xl_next,
     float* __restrict__ prow, float* __restrict__ x_out, int32_t step, int32_t* __restrict__ sched,
-    const uint32_t* __restrict__ amax, uint32_t* __restrict__ xmax, float scale_target, int32_t agg, int32_t* __restrict__ status) {
+    const uint32_t* __restrict__ amax, uint32_t* __restrict__ xmax, int32_t agg, int32_t* __restrict__ status) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
@@ -442,7 +259,7 @@ __global__ void __launch_bounds__(NT2_THREADS, 1) node_tc2_kernel(
   __syncthreads();
   tc_fence_after();
   const uint32_t tbase = *tmem_slot;
-  const int s_next = scale_for(a_t, x_t, x_tm1, scale_target);
+  const int s_next = scale_for(a_t, x_t, x_tm1);
   const float sig_next = pow2i(-s_next);
   if (blockIdx.x == 0 && tid == 0) sched[step + 1] = s_next;
   // the flow vectors enter the node Linear in the scale of the step that produced the messages, 2^-FLOW_SHIFT lower
@@ -712,20 +529,7 @@ __device__ __forceinline__ void ld_f32x8(float (&d)[8], const float* __restrict_
   }
 }
 
-// relu(acc + add) for 16 values, split to fp16 hi/lo words; accumulates the overflow detector
-__device__ __forceinline__ void relu_split16(const uint32_t (&acc)[16], const float* add, uint32_t (&hi)[8],
-                                             uint32_t (&lo)[8], uint32_t& ovf) {
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const float a = fmaxf(__uint_as_float(acc[2 * j]) + add[2 * j], 0.f);
-    const float b = fmaxf(__uint_as_float(acc[2 * j + 1]) + add[2 * j + 1], 0.f);
-    split2s(a, b, hi[j], lo[j]);
-    ovf |= hi[j] + 0x04000400u;        // fp16 inf (0x7C00) + 0x0400 sets the half's top bit
-  }
-}
-
-// =================================================================== variant 3: three tiles in flight
-// Same arithmetic as mp_edge_tc_kernel, different resource plan:
+// Resource plan of mp_edge_tc3_kernel, three tiles in flight per SM:
 //  * the gathered x[col] rows are fetched by TMA (tile::gather4, 4 rows per instruction, 8 lanes per warp issue)
 //    straight into 128B-swizzled K-major shared-memory tiles and consumed by SS-mode MMAs (layers 1 and 3) - no
 //    per-thread loads, no register / TMEM staging of the widest operand;
@@ -1303,12 +1107,9 @@ int mpn_mp_forward_tc(const mpn_core_weights* w, const mpn_edge_layout* g, const
   MPN_CUDA(cudaFuncSetAttribute(tc::mp_edge_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM3_BYTES));
   MPN_CUDA(cudaMemsetAsync(m.sched, 0, 3 * (tc::MAX_STEPS + 8) * 4, s));
   const int sms = sm_count();
-  tc::pack_weights_kernel<<<16, 256, 0, s>>>(*w, m.wimg_out, m.wimg_in, m.wimg_node, 1, status); count_launch();
+  tc::pack_weights_kernel<<<16, 256, 0, s>>>(*w, m.wimg_out, m.wimg_in, m.wimg_node, status); count_launch();
   const unsigned ngrid = (unsigned)std::min<int64_t>(ceil_div(n * 32, 256), (int64_t)sms * 4);
-  const unsigned ngrid_node = (unsigned)std::min<int64_t>(ceil_div(n, 8 * tc::NODE_NB), (int64_t)sms * 2);
   const unsigned ngrid_node2 = (unsigned)std::min<int64_t>(ceil_div(ceil_div(n, tc::TS), 2), (int64_t)sms);
-  static const bool node_simt = getenv("MPN_NODE_SIMT") != nullptr;      // development switch: FFMA2 node kernel
-  static const float scale_target = getenv("MPN_SCALE_TARGET") ? (float)atof(getenv("MPN_SCALE_TARGET")) : tc::SCALE_TARGET;
   tc::prep_nodes_kernel<<<ngrid, 256, 0, s>>>(x_init, n, w->edge_w0, w->edge_b0, m.xi, m.xl[0], m.pinit, m.prow, m.xmax, status);
   count_launch();
   if (e > 0) {
@@ -1358,17 +1159,10 @@ int mpn_mp_forward_tc(const mpn_core_weights* w, const mpn_edge_layout* g, const
       if (profiling()) profile_mark(0, false, s);
     }
     if (profiling()) profile_mark(1, true, s);
-    if (node_simt) {
-      tc::node_tc_kernel<<<ngrid_node, 256, 0, s>>>(g->out_ptr, g->in_ptr, n, g->num_out,
-                                               (int32_t)ceil_div(g->num_out, chunk), chunk_shift, m.flow, m.part, w->node_w,
-                                               w->node_b, w->edge_w0, m.pinit, xl_next, m.prow,
-                                               step == num_steps ? x_out : nullptr, step, m.sched, m.amax, m.xmax, scale_target, w->node_agg, status);
-    } else {
-      tc::node_tc2_kernel<<<ngrid_node2, tc::NT2_THREADS, tc::NSMEM_BYTES, s>>>(
-          g->out_ptr, g->in_ptr, n, g->num_out, (int32_t)ceil_div(g->num_out, chunk), chunk_shift, m.flow, m.part,
-          m.wimg_node, m.pinit, reinterpret_cast<uint4*>(xl_next), m.prow, step == num_steps ? x_out : nullptr, step,
-          m.sched, m.amax, m.xmax, scale_target, w->node_agg, status);
-    }
+    tc::node_tc2_kernel<<<ngrid_node2, tc::NT2_THREADS, tc::NSMEM_BYTES, s>>>(
+        g->out_ptr, g->in_ptr, n, g->num_out, (int32_t)ceil_div(g->num_out, chunk), chunk_shift, m.flow, m.part,
+        m.wimg_node, m.pinit, reinterpret_cast<uint4*>(xl_next), m.prow, step == num_steps ? x_out : nullptr, step,
+        m.sched, m.amax, m.xmax, w->node_agg, status);
     count_launch();
     if (profiling()) profile_mark(1, false, s);
     MPN_LAUNCH_CHECK();

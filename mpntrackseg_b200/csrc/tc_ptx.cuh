@@ -31,17 +31,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
-// non-blocking probe: true once the phase with this parity has completed
-__device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity) {
-  uint32_t done;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(done)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return done != 0;
-}
-
 // ---------------------------------------------------------------- fences
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -73,10 +62,6 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8])
                "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
                : "memory");
 }
-__device__ __forceinline__ void tmem_st4(uint32_t taddr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(a), "r"(b), "r"(c), "r"(d)
-               : "memory");
-}
 
 // ---------------------------------------------------------------- MMA
 // Shared-memory matrix descriptor, K-major, no swizzle: 8x16B core matrices; LBO = byte distance
@@ -88,6 +73,11 @@ __device__ __forceinline__ uint64_t smem_desc_kmajor(uint32_t saddr, uint32_t lb
   d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
   d |= (uint64_t)1 << 46;   // descriptor version 1 (sm_100)
   return d;
+}
+// Byte offset of element (n, k16) inside one K = 16 step of such an operand ("slab"), laid out [n/8][k16/8][n%8][k16%8]:
+// 8-row x 16-B core matrices, the two K halves LBO = 128 B apart and the 8-row groups SBO = 256 B apart.
+__device__ __forceinline__ int slab_off(int n, int k16) {
+  return (n >> 3) * 256 + (k16 >> 3) * 128 + (n & 7) * 16 + (k16 & 7) * 2;
 }
 // Instruction descriptor, kind::f16: fp16 A/B (K-major), fp32 accumulate, M x N tile.
 __host__ __device__ constexpr uint32_t idesc_f16(int m, int n) {
@@ -142,12 +132,6 @@ __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
 }
-
-// 16-byte asynchronous global -> shared copy (LDGSTS), L2-only caching
-__device__ __forceinline__ void cp_async16(uint32_t saddr, const void* gptr) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(saddr), "l"(gptr) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 // one lane of the (converged) warp
 __device__ __forceinline__ bool elect_one() {
@@ -215,13 +199,10 @@ __device__ __forceinline__ void split2s(float a, float b, uint32_t& hi, uint32_t
   hi = *reinterpret_cast<const uint32_t*>(&h);
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
-__device__ __forceinline__ void split2s_relu(float a, float b, uint32_t& hi, uint32_t& lo) {
-  asm("cvt.rz.relu.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(b), "f"(a));
-  const float2 hf = __half22float2(*reinterpret_cast<const __half2*>(&hi));
-  asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"((b - hf.y) * LO_SCALE), "f"((a - hf.x) * LO_SCALE));
-}
-// The same on (a + ba, b + bb) with the packed fp32x2 pipe (FADD2 / FMUL2: one instruction per pair): 7 instructions per
-// pair instead of 10.  Every packed operation is the IEEE rn operation of its two lanes, so the result is bit-identical.
+// ReLU fused into the lifted split of (a + ba, b + bb), as in split2_relu: hi = fp16_rz(max(v, 0)),
+// lo' = fp16_rn(max((v - hi) * 2^LO_SHIFT, 0)).  The add, subtract and lift run on the packed fp32x2 pipe (FADD2 / FMUL2:
+// one instruction per pair): 7 instructions per pair instead of 10.  Every packed operation is the IEEE rn operation of
+// its two lanes, so the result is bit-identical to the scalar form.
 __device__ __forceinline__ unsigned long long pack2(float x, float y) {
   unsigned long long r;
   asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(x), "f"(y));
