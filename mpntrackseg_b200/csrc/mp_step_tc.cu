@@ -63,7 +63,9 @@ constexpr int NIMG_BYTES = (NOFF_F32 + DN * 4 + 127) / 128 * 128;
 
 // =================================================================== range bookkeeping
 // Per forward: sched[t] = s_t (exponent of the step's scale), amax[t] = float bits of the largest true activation
-// the edge kernel of step t saw, xmax[t] = largest |x_lat| consumed by step t (t = 1..num_steps; all zeroed at start).
+// the edge kernel of step t saw, xmax[t] = largest |x_lat| consumed by step t (t = 1..num_steps; all zeroed at start);
+// amax[0] = largest |x_init|, |e_init| (the constant rows, recorded by prep_nodes_kernel and split_edges_kernel);
+// fmax[t] = largest flow row sum (or granule partial) the edge kernel of step t wrote.
 constexpr int MAX_STEPS = 1000;
 // The lifted low halves keep 22 bits for any operand whose high half is a normal fp16 number (>= 2^-14), so the scale
 // can leave generous headroom at no cost in precision: the lagged maximum is brought to <= 2^6 (1024x headroom for the
@@ -78,7 +80,19 @@ constexpr int INIT_SHIFT = 8;                // the constant x_init / e_init row
 // order 1 (a quiet window batched with a loud one: its logit error triples at s = 19 and is 7x the bar at s = 22, on
 // a B200).  Such a step sets status bit 2, which sends engine 'auto' to the fp32 kernels like an fp16 overflow.
 constexpr int S_RESOLVED = 17;
+// The constant rows are stored x 2^-INIT_SHIFT once per forward, whatever the step scale (which never goes below 0), so
+// they have the same floor: below 2^-14 stored their absolute resolution is 2^-34 (2^-26 in true units).  They are
+// resolved as S_RESOLVED resolves rows of order 1 -- floor at most 2^-17 of the value -- when the largest stored
+// |x_init|, |e_init| is at least 2^(S_RESOLVED - 34); a smaller nonzero maximum sets status bit 2 (all-zero rows are exact).
+__device__ __forceinline__ bool init_rows_unresolved(float init_max) {
+  const float m = init_max * pow2i(-INIT_SHIFT);
+  return m > 0.f && m < pow2i(S_RESOLVED - 34);
+}
 constexpr int FLOW_SHIFT = 7;                // a flow vector sums up to ~100 messages: operand scale 2^-(s_t + 7)
+// Flows far below that (a flow MLP whose output layer is small next to the rest of the network) would leave their low
+// bits to fp16 subnormals in the node Linear's operand.  When the largest flow piece of the step lies below 2^-FLOW_LIFT
+// there, the node kernel lowers the flow scale so that it lands in [2^-5, 2^-4) (exact: powers of two, fp32 epilogue).
+constexpr int FLOW_LIFT = 10;
 // s_{t+1} from what is known when the node kernel of step t starts: the edge kernel's activation maximum of step t
 // and the node-state maxima of steps t and t-1 (their ratio predicts the growth of the state being produced).
 __device__ __forceinline__ int scale_for(float a_t, float x_t, float x_tm1) {
@@ -99,8 +113,12 @@ __device__ __forceinline__ void atomic_max_f32(uint32_t* addr, float v) {   // v
 // One image per direction (flow_out / flow_in); layers 1-2 and the classifier are shared.
 __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ img_out, uint8_t* __restrict__ img_in,
                                     uint8_t* __restrict__ img_node, int32_t* __restrict__ status) {
-  int bad = 0;                       // a weight whose fp16 image (x 2^INIT_SHIFT for the constant-row slabs) is not finite
-  auto fits = [&](float v) { if (!(fabsf(v) * pow2i(INIT_SHIFT) < 65000.f)) bad = 1; };
+  // bad: a weight whose fp16 image, times the largest factor its slab carries (2^INIT_SHIFT for the constant-row slabs,
+  // 1 elsewhere), is not finite; or a non-finite bias or fp32 tail weight
+  int bad = 0;
+  auto fits = [&](float v, float f) { if (!(fabsf(v) * f < 65000.f)) bad = 1; };
+  auto finite = [&](float v) { if (!isfinite(v)) bad = 1; };
+  const float init_f = pow2i(INIT_SHIFT);
   {
     auto putn = [&](int off_h, int off_l, int slab_bytes, int n, int k, float v) {
       const __half h = __float2half_rn(v);
@@ -110,12 +128,13 @@ __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ im
       *reinterpret_cast<__half*>(img_node + off_l + o) = l;
     };
     const int tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
-    for (int i = tid; i < DN * 2 * DN; i += nt) { fits(w.node_w[i]); putn(NOFF_NWH, NOFF_NWL, NW_SLAB, i / (2 * DN), i % (2 * DN), w.node_w[i]); }
+    for (int i = tid; i < DN * 2 * DN; i += nt) { fits(w.node_w[i], 1.f); putn(NOFF_NWH, NOFF_NWL, NW_SLAB, i / (2 * DN), i % (2 * DN), w.node_w[i]); }
     for (int i = tid; i < EH * DN; i += nt) {            // edge layer 0, input columns 32..63 (x_lat[row])
       const int n = i / DN, k = i % DN;
+      fits(w.edge_w0[n * 160 + 32 + k], 1.f);
       putn(NOFF_PWH, NOFF_PWL, PW_SLAB, n, k, w.edge_w0[n * 160 + 32 + k]);
     }
-    for (int i = tid; i < DN; i += nt) reinterpret_cast<float*>(img_node + NOFF_F32)[i] = w.node_b[i];
+    for (int i = tid; i < DN; i += nt) { finite(w.node_b[i]); reinterpret_cast<float*>(img_node + NOFF_F32)[i] = w.node_b[i]; }
   }
   for (int dir = 0; dir < 2; ++dir) {
     uint8_t* img = dir == 0 ? img_out : img_in;
@@ -123,8 +142,8 @@ __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ im
     const float* f1 = dir == 0 ? w.fout_w1 : w.fin_w1;
     const float* fb0 = dir == 0 ? w.fout_b0 : w.fin_b0;
     const float* fb1 = dir == 0 ? w.fout_b1 : w.fin_b1;
-    auto put = [&](int off_h, int off_l, int slab_bytes, int n, int k, float v) {
-      fits(v);
+    auto put = [&](int off_h, int off_l, int slab_bytes, int n, int k, float v, float f) {
+      fits(v, f);
       const __half h = __float2half_rn(v);
       const __half l = __float2half_rn((v - __half2float(h)) * LO_SCALE);
       const int o = (k >> 4) * slab_bytes + slab_off(n, k & 15);
@@ -133,12 +152,12 @@ __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ im
     };
     const int tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
     for (int i = tid; i < EH * 96; i += nt) {            // edge layer 0, input columns 64..159
-      const int n = i / 96, k = i % 96;
-      put(OFF_L1H, OFF_L1L, L1_SLAB, n, k, w.edge_w0[n * 160 + 64 + k]);
+      const int n = i / 96, k = i % 96, ks = k >> 4;     // K steps 0, 1 (x_init[col]) and 4 (e_init): constant rows
+      put(OFF_L1H, OFF_L1L, L1_SLAB, n, k, w.edge_w0[n * 160 + 64 + k], ks <= 1 || ks == 4 ? init_f : 1.f);
     }
     for (int i = tid; i < DE * EH; i += nt) {            // edge layer 1
       const int n = i / EH, k = i % EH;
-      put(OFF_L2H, OFF_L2L, L2_SLAB, n, k, w.edge_w1[n * EH + k]);
+      put(OFF_L2H, OFF_L2L, L2_SLAB, n, k, w.edge_w1[n * EH + k], 1.f);
     }
     for (int i = tid; i < FHP * 80; i += nt) {           // flow layer 0 (rows padded 56 -> 64)
       const int n = i / 80, k = i % 80;
@@ -146,11 +165,11 @@ __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ im
       // only the e' K step, columns 64..79)
       float v = n < FH ? f0[n * 80 + k] : 0.f;
       if (n >= FH && k >= 64) v = w.cls_w0[(n - FH) * DE + (k - 64)];
-      put(OFF_L3H, OFF_L3L, L3_SLAB, n, k, v);
+      put(OFF_L3H, OFF_L3L, L3_SLAB, n, k, v, k < DN ? init_f : 1.f);   // K steps 0, 1: x_init[col]
     }
     for (int i = tid; i < DN * FHP; i += nt) {           // flow layer 1 (K padded 56 -> 64)
       const int n = i / FHP, k = i % FHP;
-      put(OFF_L4H, OFF_L4L, L4_SLAB, n, k, k < FH ? f1[n * FH + k] : 0.f);
+      put(OFF_L4H, OFF_L4L, L4_SLAB, n, k, k < FH ? f1[n * FH + k] : 0.f, 1.f);
     }
     float* ft = reinterpret_cast<float*>(img + OFF_F32);
     for (int i = tid; i < F_COUNT; i += nt) {
@@ -162,6 +181,7 @@ __global__ void pack_weights_kernel(mpn_core_weights w, uint8_t* __restrict__ im
       else if (i < F_CW1) v = w.cls_b0[i - F_CB0];
       else if (i < F_CB1) v = w.cls_w1[i - F_CW1];
       else if (i == F_CB1) v = w.cls_b1[0];
+      finite(v);
       ft[i] = v;
     }
   }
@@ -183,19 +203,22 @@ __global__ void __launch_bounds__(256) prep_nodes_kernel(const float* __restrict
                                                          const float* __restrict__ w0, const float* __restrict__ b0,
                                                          __half* __restrict__ xi, __half* __restrict__ xl0,
                                                          float* __restrict__ pinit, float* __restrict__ prow,
-                                                         uint32_t* __restrict__ xmax, int32_t* __restrict__ status) {
+                                                         uint32_t* __restrict__ xmax, uint32_t* __restrict__ init_max,
+                                                         int32_t* __restrict__ status) {
   __shared__ float s_w[64 * EH];     // [i][o], i over W0 columns 0..63
   __shared__ float s_b[EH];
+  int ovf = 0;                       // also a non-finite W0[:, 0:64] or b0: they enter the hoisted row term in fp32, unchecked elsewhere
   for (int idx = threadIdx.x; idx < 64 * EH; idx += blockDim.x) {        // coalesced along a weight row
     const int o = idx / 64, i = idx - o * 64;
-    s_w[i * EH + o] = w0[o * 160 + i];
+    const float v = w0[o * 160 + i];
+    if (!isfinite(v)) ovf = 1;
+    s_w[i * EH + o] = v;
   }
-  for (int o = threadIdx.x; o < EH; o += blockDim.x) s_b[o] = b0[o];
+  for (int o = threadIdx.x; o < EH; o += blockDim.x) { s_b[o] = b0[o]; if (!isfinite(s_b[o])) ovf = 1; }
   __syncthreads();
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  int ovf = 0;
   float mx = 0.f;
   for (int64_t r = warp; r < n; r += nwarps) {
     const float v = x_init[r * DN + lane];
@@ -221,6 +244,7 @@ __global__ void __launch_bounds__(256) prep_nodes_kernel(const float* __restrict
     }
   }
   atomic_max_f32(xmax + 1, mx);                                         // the state consumed by step 1 (scale s_1 = 0)
+  atomic_max_f32(init_max, mx);
   if (ovf) atomicOr(status, 1);
 }
 
@@ -241,7 +265,8 @@ __global__ void __launch_bounds__(NT2_THREADS, 1) node_tc2_kernel(
     int32_t chunks_out, int chunk_shift, const float* __restrict__ flow, const float* __restrict__ part,
     const uint8_t* __restrict__ wimg, const float* __restrict__ pinit, uint4* __restrict__ xl_next,
     float* __restrict__ prow, float* __restrict__ x_out, int32_t step, int32_t* __restrict__ sched,
-    const uint32_t* __restrict__ amax, uint32_t* __restrict__ xmax, int32_t agg, int32_t* __restrict__ status) {
+    const uint32_t* __restrict__ amax, uint32_t* __restrict__ xmax, const uint32_t* __restrict__ fmax, int32_t agg,
+    int32_t* __restrict__ status) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
@@ -262,8 +287,17 @@ __global__ void __launch_bounds__(NT2_THREADS, 1) node_tc2_kernel(
   const int s_next = scale_for(a_t, x_t, x_tm1);
   const float sig_next = pow2i(-s_next);
   if (blockIdx.x == 0 && tid == 0) sched[step + 1] = s_next;
-  // the flow vectors enter the node Linear in the scale of the step that produced the messages, 2^-FLOW_SHIFT lower
-  const int s_flow = sched[step] + FLOW_SHIFT;
+  // the flow vectors enter the node Linear in the scale of the step that produced the messages, 2^-FLOW_SHIFT lower,
+  // or lifted (FLOW_LIFT)
+  int s_flow = sched[step] + FLOW_SHIFT;
+  {
+    const float f_op = __uint_as_float(fmax[step]) * pow2i(-s_flow);
+    if (f_op > 0.f && f_op < pow2i(-FLOW_LIFT)) {
+      int e;
+      frexpf(f_op, &e);                                                  // f_op in [2^(e-1), 2^e)
+      s_flow = max(s_flow + e + 4, -100);
+    }
+  }
   const float sig_flow = pow2i(-s_flow), inv_sig_flow = pow2i(s_flow);
 
   const int g = warp >> 2, wq = warp & 3;
@@ -454,8 +488,9 @@ __global__ void __launch_bounds__(NT2_THREADS, 1) node_tc2_kernel(
 
 // e (fp32 [E,16], slot order) -> split rows [hi(16) | lo(16)] halfs
 __global__ void split_edges_kernel(const float* __restrict__ e, int64_t num_edges, uint4* __restrict__ out,
-                                   int32_t* __restrict__ status) {
+                                   uint32_t* __restrict__ init_max, int32_t* __restrict__ status) {
   int ovf = 0;
+  float mx = 0.f;
   for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < num_edges; s += (int64_t)gridDim.x * blockDim.x) {
     const float4* p = reinterpret_cast<const float4*>(e + s * DE);
     uint32_t hi[8], lo[8];
@@ -465,13 +500,16 @@ __global__ void split_edges_kernel(const float* __restrict__ e, int64_t num_edge
       const float sc = pow2i(-INIT_SHIFT);
       split2s(v.x * sc, v.y * sc, hi[2 * q], lo[2 * q]);
       split2s(v.z * sc, v.w * sc, hi[2 * q + 1], lo[2 * q + 1]);
-      if (!(fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))) < 65000.f)) ovf = 1;
+      const float m = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));   // fmaxf drops NaN:
+      if (!(m < 65000.f) || isnan(v.x + v.y + v.z + v.w)) ovf = 1;                           // the sum keeps it
+      mx = fmaxf(mx, m);
     }
     out[s * 4 + 0] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
     out[s * 4 + 1] = make_uint4(hi[4], hi[5], hi[6], hi[7]);
     out[s * 4 + 2] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
     out[s * 4 + 3] = make_uint4(lo[4], lo[5], lo[6], lo[7]);
   }
+  atomic_max_f32(init_max, mx);
   if (ovf) atomicOr(status, 1);
 }
 
@@ -510,7 +548,8 @@ struct TcArgs {
   int32_t* status;
   int32_t step;              // 1-based step index
   const int32_t* sched;      // sched[t] = s_t, see "range bookkeeping"
-  uint32_t* amax;            // amax[step] receives the largest true activation of this launch
+  uint32_t* amax;            // amax[step] receives the largest true activation of this launch; amax[0]: constant rows
+  uint32_t* fmax;            // fmax[step] receives the largest flow piece (true value) this launch wrote
   int32_t agg;               // 0 sum, 1 mean (summed here, divided by the node kernel), 2 max
 };
 
@@ -572,6 +611,7 @@ __global__ void __launch_bounds__(NTHREADS3, 1) mp_edge_tc3_kernel(TcArgs a, con
 
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SM3_BAR);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + SM3_TMEM);
+  uint32_t* s_fmax = tmem_slot + 1;                                     // largest flow piece this CTA wrote (scaled)
   // this step's scale (uniform): operands are true values x sigma
   const int s_cur = a.sched[a.step];
   const int s_prev = a.step > 1 ? a.sched[a.step - 1] : INIT_SHIFT;   // step 1 reads e_init rows as the latent state
@@ -608,10 +648,12 @@ __global__ void __launch_bounds__(NTHREADS3, 1) mp_edge_tc3_kernel(TcArgs a, con
     // s_cur > INIT_SHIFT + 14: the slab factor 2^(INIT_SHIFT - s) is a subnormal fp16 number (or 0 beyond 2^-24) and the
     // constant-row terms lose bits / vanish; such steps are already flagged by S_RESOLVED
   }
-  if (s_cur > S_RESOLVED && blockIdx.x == 0 && tid == 0) atomicOr(a.status, 2);
+  if (blockIdx.x == 0 && tid == 0 && (s_cur > S_RESOLVED || (a.step == 1 && init_rows_unresolved(__uint_as_float(a.amax[0])))))
+    atomicOr(a.status, 2);
   if (tid == 0) {
     for (int i = 0; i < NG3; ++i) { mbar_init(&bars[i], 1); mbar_init(&bars[NG3 + i], 4); }
     mbar_fence_init();
+    *s_fmax = 0u;
   }
   if (warp == 0) tmem_alloc<512>(tmem_slot);
   fence_async_smem();
@@ -838,6 +880,7 @@ __global__ void __launch_bounds__(NTHREADS3, 1) mp_edge_tc3_kernel(TcArgs a, con
         const int32_t rq = rows[q];
         const bool starts_before = first_seg && r_prev == rq;
         const bool continues = q == cw - 1 && r_next == rq;
+        atomicMax(s_fmax, __float_as_uint(sum));                       // sum >= 0: integer order = float order
         if (!starts_before && !continues) a.flow[(int64_t)rq * 2 * DN + dir_off + f] = sum * inv_sigma;
         else a.part[(chunk_id * 2 + (first_seg ? 0 : 1)) * DN + f] = sum * inv_sigma;
         sum = 0.f;
@@ -999,6 +1042,10 @@ __global__ void __launch_bounds__(NTHREADS3, 1) mp_edge_tc3_kernel(TcArgs a, con
     cur = nxt; nxt = nn;
   }
   {
+    // __hmax2 drops NaN, so this sees an fp16 overflow (an inf or a value at the top of the range) but not a NaN.  It need
+    // not: every input, weight and bias is checked finite and inside the fp16 range before step 1 (prep_nodes_kernel,
+    // split_edges_kernel, pack_weights_kernel), and from such operands the edge kernel cannot produce a NaN before an
+    // activation has overflowed, which this test sees.
     const uint32_t w = *reinterpret_cast<const uint32_t*>(&vmax);
     if ((w & 0x7FFFu) >= 0x7BFFu || ((w >> 16) & 0x7FFFu) >= 0x7BFFu) atomicOr(a.status, 1);
     const float2 vm = __half22float2(vmax);
@@ -1006,6 +1053,7 @@ __global__ void __launch_bounds__(NTHREADS3, 1) mp_edge_tc3_kernel(TcArgs a, con
   }
   tc_fence_before();
   __syncthreads();
+  if (tid == 0 && *s_fmax != 0u) atomicMax(a.fmax + a.step, __float_as_uint(__uint_as_float(*s_fmax) * inv_sigma));
   if (warp == 0) tmem_dealloc<512>(tbase);
 }
 
@@ -1036,7 +1084,7 @@ struct TcWorkspace {
   uint4* ei; uint4* es;
   float* flow; float* part;
   uint8_t* wimg_out; uint8_t* wimg_in; uint8_t* wimg_node;
-  int32_t* sched; uint32_t* amax; uint32_t* xmax;      // range bookkeeping, MAX_STEPS + 8 entries each (contiguous)
+  int32_t* sched; uint32_t* amax; uint32_t* xmax; uint32_t* fmax;   // range bookkeeping, MAX_STEPS + 8 entries each (contiguous)
 };
 
 static int64_t carve(void* ws, int64_t n, int64_t e, TcWorkspace* out) {
@@ -1055,9 +1103,10 @@ static int64_t carve(void* ws, int64_t n, int64_t e, TcWorkspace* out) {
   w.wimg_out = cv.take<uint8_t>(IMG_BYTES);
   w.wimg_in = cv.take<uint8_t>(IMG_BYTES);
   w.wimg_node = cv.take<uint8_t>(NIMG_BYTES);
-  w.sched = cv.take<int32_t>(3 * (MAX_STEPS + 8));
+  w.sched = cv.take<int32_t>(4 * (MAX_STEPS + 8));
   w.amax = reinterpret_cast<uint32_t*>(w.sched) + (MAX_STEPS + 8);
   w.xmax = w.amax + (MAX_STEPS + 8);
+  w.fmax = w.xmax + (MAX_STEPS + 8);
   if (out) *out = w;
   return cv.off;
 }
@@ -1105,16 +1154,16 @@ int mpn_mp_forward_tc(const mpn_core_weights* w, const mpn_edge_layout* g, const
   tc::carve(ws, n, e > 0 ? e : 1, &m);
 
   MPN_CUDA(cudaFuncSetAttribute(tc::mp_edge_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM3_BYTES));
-  MPN_CUDA(cudaMemsetAsync(m.sched, 0, 3 * (tc::MAX_STEPS + 8) * 4, s));
+  MPN_CUDA(cudaMemsetAsync(m.sched, 0, 4 * (tc::MAX_STEPS + 8) * 4, s));
   const int sms = sm_count();
   tc::pack_weights_kernel<<<16, 256, 0, s>>>(*w, m.wimg_out, m.wimg_in, m.wimg_node, status); count_launch();
   const unsigned ngrid = (unsigned)std::min<int64_t>(ceil_div(n * 32, 256), (int64_t)sms * 4);
   const unsigned ngrid_node2 = (unsigned)std::min<int64_t>(ceil_div(ceil_div(n, tc::TS), 2), (int64_t)sms);
-  tc::prep_nodes_kernel<<<ngrid, 256, 0, s>>>(x_init, n, w->edge_w0, w->edge_b0, m.xi, m.xl[0], m.pinit, m.prow, m.xmax, status);
+  tc::prep_nodes_kernel<<<ngrid, 256, 0, s>>>(x_init, n, w->edge_w0, w->edge_b0, m.xi, m.xl[0], m.pinit, m.prow, m.xmax, m.amax, status);
   count_launch();
   if (e > 0) {
     const unsigned egrid = (unsigned)std::min<int64_t>(ceil_div(e, 256), (int64_t)sms * 8);
-    tc::split_edges_kernel<<<egrid, 256, 0, s>>>(e_init, e, m.ei, status); count_launch();
+    tc::split_edges_kernel<<<egrid, 256, 0, s>>>(e_init, e, m.ei, m.amax, status); count_launch();
   }
   MPN_LAUNCH_CHECK();
 
@@ -1152,7 +1201,7 @@ int mpn_mp_forward_tc(const mpn_core_weights* w, const mpn_edge_layout* g, const
       a.logits = (logits && step >= first_class_step) ? logits + (int64_t)(step - first_class_step) * e : nullptr;
       a.wimg_out = m.wimg_out; a.wimg_in = m.wimg_in;
       a.status = status;
-      a.step = step; a.sched = m.sched; a.amax = m.amax; a.agg = w->node_agg;
+      a.step = step; a.sched = m.sched; a.amax = m.amax; a.fmax = m.fmax; a.agg = w->node_agg;
       if (profiling()) profile_mark(0, true, s);
       tc::mp_edge_tc3_kernel<<<grid3, tc::NTHREADS3, tc::SMEM3_BYTES, s>>>(a, tm_xi, tm_xl[(step - 1) & 1]);
       count_launch();
@@ -1162,7 +1211,7 @@ int mpn_mp_forward_tc(const mpn_core_weights* w, const mpn_edge_layout* g, const
     tc::node_tc2_kernel<<<ngrid_node2, tc::NT2_THREADS, tc::NSMEM_BYTES, s>>>(
         g->out_ptr, g->in_ptr, n, g->num_out, (int32_t)ceil_div(g->num_out, chunk), chunk_shift, m.flow, m.part,
         m.wimg_node, m.pinit, reinterpret_cast<uint4*>(xl_next), m.prow, step == num_steps ? x_out : nullptr, step,
-        m.sched, m.amax, m.xmax, w->node_agg, status);
+        m.sched, m.amax, m.xmax, m.fmax, w->node_agg, status);
     count_launch();
     if (profiling()) profile_mark(1, false, s);
     MPN_LAUNCH_CHECK();
