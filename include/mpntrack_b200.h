@@ -281,6 +281,42 @@ int mpn_gather_cols(const float* src, int64_t lds, int64_t width, const int32_t*
 int mpn_segment_sum(const float* in, int64_t ld, int64_t in_off, int64_t width, const int32_t* ptr,
                     const int32_t* perm, int64_t nodes, int accumulate, float* out, int64_t ldo,
                     int64_t col_off, void* stream);
+/* mpn_segment_sum with a choice of reduction (the node_agg_fn of models/mpn.py:263-273): mode 0: sum; 1: mean (0 for an
+ * empty segment); 2: max, the first strictly larger value in ascending q (torch_scatter's scatter_max), 0 for an empty
+ * segment.  argmax (mode 2, may be NULL): int32 [nodes, width], the input row of each maximum, -1 for an empty
+ * segment. */
+int mpn_segment_reduce(const float* in, int64_t ld, int64_t in_off, int64_t width, const int32_t* ptr,
+                       const int32_t* perm, int64_t nodes, int accumulate, float* out, int64_t ldo,
+                       int64_t col_off, int mode, int32_t* argmax, void* stream);
+/* Backward of a mean (mode 1) / max (mode 2) mpn_segment_sum without perm, for the slots q in [q0, q1):
+ * out[q*ldo + f] = g[row[q]*ldg + f] / (ptr[row[q]+1] - ptr[row[q]])  (mean), or
+ * out[q*ldo + f] = argmax[row[q]*width + f] == q ? g[row[q]*ldg + f] : 0  (max: the whole gradient to one argmax). */
+int mpn_segment_grad(const float* g, int64_t ldg, const int32_t* row, const int32_t* ptr, const int32_t* argmax,
+                     int64_t q0, int64_t q1, int64_t width, int mode, float* out, int64_t ldo, void* stream);
+/* Linear -> BatchNorm1d (training mode) -> ReLU [-> Dropout] after the Linear: z [m, n] (row stride ldz) is the Linear
+ * output.  Per column the mean and the biased variance over the m rows (two passes, fixed order) go to stats[0:n] and
+ * (as 1/sqrt(var + eps)) stats[n:2n] (stats holds 4n floats; the backward uses the rest); running_mean / running_var
+ * move by momentum towards the mean and the unbiased variance and *num_batches_tracked grows by 1, as
+ * torch.nn.BatchNorm1d does.  y = ReLU(gamma (z - mean) / sqrt(var + eps) + beta), times keep / (1 - p) when p > 0
+ * (see mpn_dropout_forward for the mask; mask may be NULL).  m == 1 is an error (MPN_EINVAL); m == 0 only increments
+ * *num_batches_tracked. */
+int mpn_batchnorm_forward(const float* z, int64_t ldz, int64_t m, int64_t n, const float* gamma, const float* beta,
+                          float eps, float momentum, float* running_mean, float* running_var,
+                          int64_t* num_batches_tracked, float* stats, float p, uint64_t seed, const int64_t* counter,
+                          int call, float* y, int64_t ldy, uint8_t* mask, void* stream);
+/* Its backward from dL/dy (g) and the stored y: g' = (y > 0) g gscale (gscale = 1 / (1 - p)),
+ * ggamma += sum g' xhat, gbeta += sum g', gz = gamma / sqrt(var + eps) (g' - mean(g') - xhat mean(g' xhat)). */
+int mpn_batchnorm_backward(const float* z, int64_t ldz, const float* g, int64_t ldg, const float* y, int64_t ldy,
+                           int64_t m, int64_t n, const float* gamma, float* stats, float gscale, float* ggamma,
+                           float* gbeta, float* gz, int64_t ldgz, void* stream);
+/* In place on a ReLU output y [m, n]: y = y * keep / (1 - p), 0 < p < 1.  keep of element t = r*n + c is a Philox4x32-10
+ * draw keyed by seed, with counter (*counter, the number of the training forward) and call (the dropout call within
+ * it): independent of the launch configuration.  mask (may be NULL): uint8 [m, n] receives keep. */
+int mpn_dropout_forward(float* y, int64_t ldy, int64_t m, int64_t n, float p, uint64_t seed, const int64_t* counter,
+                        int call, uint8_t* mask, void* stream);
+/* out = y > 0 ? g * scale : 0  (ReLU + dropout backward from the stored output; scale = 1 / (1 - p)) */
+int mpn_dropout_backward(const float* g, int64_t ldg, const float* y, int64_t ldy, int64_t m, int64_t n, float scale,
+                         float* out, int64_t ldo, void* stream);
 /* g[i] = y[i] > 0 ? g[i] : 0 */
 int mpn_relu_mask(float* g, const float* y, int64_t n, void* stream);
 /* torch.optim.Adam step (configs/tracking_cfg.yaml:6-10: lr 1e-3, weight_decay 1e-4 as L2 term) on flat

@@ -70,6 +70,15 @@ SIGNATURES = {
     'mpn_colsum': (C.c_int, [c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, C.c_int, c_vp, c_vp]),
     'mpn_gather_cols': (C.c_int, [c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_i64, c_i64, c_vp]),
     'mpn_segment_sum': (C.c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_i64, C.c_int, c_vp, c_i64, c_i64, c_vp]),
+    'mpn_segment_reduce': (C.c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_i64, C.c_int, c_vp, c_i64, c_i64, C.c_int,
+                                     c_vp, c_vp]),
+    'mpn_segment_grad': (C.c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, C.c_int, c_vp, c_i64, c_vp]),
+    'mpn_batchnorm_forward': (C.c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_f32,
+                                        C.c_uint64, c_vp, C.c_int, c_vp, c_i64, c_vp, c_vp]),
+    'mpn_batchnorm_backward': (C.c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_f32, c_vp, c_vp,
+                                         c_vp, c_i64, c_vp]),
+    'mpn_dropout_forward': (C.c_int, [c_vp, c_i64, c_i64, c_i64, c_f32, C.c_uint64, c_vp, C.c_int, c_vp, c_vp]),
+    'mpn_dropout_backward': (C.c_int, [c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_f32, c_vp, c_i64, c_vp]),
     'mpn_relu_mask': (C.c_int, [c_vp, c_vp, c_i64, c_vp]),
     'mpn_adam_step': (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_f32, c_f32, c_f32, c_f32, c_i64, c_f32, c_vp]),
     'mpn_adam_step_dev': (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_f32, c_f32, c_f32, c_f32, c_vp, c_f32, c_vp]),

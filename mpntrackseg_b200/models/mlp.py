@@ -14,7 +14,8 @@ class MLP(nn.Module):
     Evaluation mode (what the tracker runs): BatchNorm1d is the affine map of its running statistics and is folded
     into the preceding Linear (W' = s W, b' = s (b - mean) + beta with s = gamma / sqrt(var + eps)); Dropout is the
     identity.  The fused kernels therefore see plain Linear + ReLU layers (``effective_linears``).  Training mode
-    with BatchNorm (batch statistics) or Dropout (random masks) is not built into the CUDA path and raises."""
+    with BatchNorm (batch statistics) or Dropout (random masks) is trained as part of ``MOTMPNet`` (training.py's
+    CoreTrainer); a standalone call of an ``MLP``, ``EdgeModel`` or ``TimeAwareNodeModel`` in that mode raises."""
 
     def __init__(self, input_dim, fc_dims, dropout_p=0.4, use_batchnorm=False):
         super().__init__()
@@ -39,8 +40,9 @@ class MLP(nn.Module):
 
     def _check_mode(self):
         if self.training and (self.use_batchnorm or self.dropout_p != 0):
-            raise NotImplementedError('BatchNorm / Dropout in training mode are not built into the CUDA path '
-                                      '(every shipped config has use_batchnorm: False, dropout_p: 0); call model.eval()')
+            raise NotImplementedError('BatchNorm / Dropout in training mode run only inside a MOTMPNet training forward '
+                                      '(model.train()(data), CoreTrainer); call eval() for a standalone MLP / EdgeModel / '
+                                      'TimeAwareNodeModel')
 
     def effective_linears(self):
         """[(weight, bias)] of the Linear layers as the kernels evaluate them (BatchNorm folded in)."""

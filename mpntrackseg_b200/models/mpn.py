@@ -394,11 +394,14 @@ class MOTMPNet(nn.Module):
     def forward(self, data, return_state=False):
         x, edge_index, edge_attr = data.x, data.edge_index, data.edge_attr
         x_ext = getattr(data, 'x_ext', None) if self.has_mask_branch else None
-        if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+        if self.training and ((torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()))
+                              or self._core_has_train_only_layers()):
             # training (pl_module.py:122-135): model.train() + autograd on.  The core network runs through the
             # deterministic fp32 training kernels with a hand-written backward; loss.backward() fills p.grad of the
-            # encoder / MPNet / classifier weights.  Evaluation-mode calls (model.eval(), with or without no_grad)
-            # always take the inference kernels below.
+            # encoder / MPNet / classifier weights.  A training-mode call under no_grad takes this path too when the
+            # core has BatchNorm or Dropout: batch statistics, running-statistic updates and fresh dropout masks, as
+            # torch runs such a module, without a backward.  Evaluation-mode calls (model.eval(), with or without
+            # no_grad) always take the inference kernels below.
             if return_state:
                 raise NotImplementedError('return_state is an inference-only option')
             tr = self.core_trainer()
@@ -423,6 +426,13 @@ class MOTMPNet(nn.Module):
         if return_state:
             out['node_state'], out['edge_state_slots'], out['layout'] = res[1], res[2], layout
         return out
+
+    def _core_has_train_only_layers(self):
+        """True when a core MLP has BatchNorm1d or Dropout, whose training-mode forward the inference kernels lack."""
+        return any(isinstance(m, MLP) and (m.use_batchnorm or m.dropout_p != 0)
+                   for m in (self.encoder.node_model, self.encoder.edge_model, self.MPNet.edge_model.edge_model,
+                             self.MPNet.node_model.flow_in_model, self.MPNet.node_model.flow_out_model,
+                             self.classifier.edge_model))
 
     def core_trainer(self):
         """The ``training.CoreTrainer`` bound to this model (built on first use: it re-homes the core parameters

@@ -6,8 +6,12 @@ reference: pl_module/pl_module.py:88-135 (_compute_loss, _train_val_step), scrip
 one summed all-reduce of a single flat gradient bucket), models/mpn.py:349-381 for the forward.
 
 The arithmetic runs in the deterministic fp32 kernels of csrc/train_ops.cu (mpn_gemm, mpn_colsum,
-mpn_gather_cols, mpn_segment_sum, mpn_adam_step) and csrc/loss.cu; torch only owns the buffers, does
-index bookkeeping (argsort of the column indices) and trivial elementwise adds of gradient buffers.
+mpn_gather_cols, mpn_segment_reduce, mpn_segment_grad, mpn_batchnorm_*, mpn_dropout_*, mpn_adam_step) and
+csrc/loss.cu; torch only owns the buffers, does index bookkeeping (argsort of the column indices, the dropout
+forward counter) and trivial elementwise adds of gradient buffers.  The model options of the reference MLPs are
+trained as the reference trains them: node_agg_fn sum / mean / max (max sends the gradient to one argmax, the lowest
+caller edge id among ties, like torch_scatter's scatter_max), BatchNorm1d with batch statistics over the rows of each
+call (running statistics updated in the module's buffers) and Dropout with Philox masks.
 Scope: the tracking loss of the core network (encoders, MPNet, classifier).  The mask branch / mask loss
 are not trained here.
 """
@@ -57,25 +61,86 @@ def gather_cols(src, idx, out, col_off):
                                 stream_ptr()), 'gather_cols')
 
 
-def segment_sum(inp, in_off, width, seg_ptr, perm, out, col_off, accumulate=False):
-    check(lib().mpn_segment_sum(ptr(inp), _ld(inp), in_off, width, ptr(seg_ptr), ptr(perm), out.shape[0], int(accumulate),
-                                ptr(out), _ld(out), col_off, stream_ptr()), 'segment_sum')
+AGG_MODES = {'sum': 0, 'mean': 1, 'max': 2}
+
+
+def segment_sum(inp, in_off, width, seg_ptr, perm, out, col_off, accumulate=False, mode='sum', argmax=None):
+    """out[:, col_off:col_off+width] (+)= the sum / mean / max of each segment; ``argmax`` (int32 [nodes, width], max only)
+    receives the input row of each maximum (-1 for an empty segment)."""
+    check(lib().mpn_segment_reduce(ptr(inp), _ld(inp), in_off, width, ptr(seg_ptr), ptr(perm), out.shape[0],
+                                   int(accumulate), ptr(out), _ld(out), col_off, AGG_MODES[mode], ptr(argmax),
+                                   stream_ptr()), 'segment_sum')
+
+
+def segment_grad(g, row, seg_ptr, argmax, q0, q1, mode, out):
+    """out[q] for the slots q in [q0, q1): the gradient of a mean / max ``segment_sum`` (without perm) from ``g``."""
+    check(lib().mpn_segment_grad(ptr(g), _ld(g), ptr(row), ptr(seg_ptr), ptr(argmax), q0, q1, out.shape[1],
+                                 AGG_MODES[mode], ptr(out), _ld(out), stream_ptr()), 'segment_grad')
+
+
+class _Dropout:
+    """Mask source of one training forward: call k of the forward numbered ``counter`` (a device int64) draws its mask
+    from Philox4x32 keyed by ``seed``.  ``masks`` (tests only) collects each call's uint8 mask under its layer key."""
+
+    def __init__(self, seed, counter, keep_masks=False):
+        self.seed, self.counter, self.calls = seed, counter, 0
+        self.masks = {} if keep_masks else None
+
+    def next(self, key, shape, device):
+        self.calls += 1
+        if self.masks is None:
+            return self.calls - 1, None
+        m = self.masks[key] = torch.empty(shape, dtype=torch.uint8, device=device)
+        return self.calls - 1, m
 
 
 class _Linear:
-    """y = act(x W^T + b) with its backward (ReLU folded in through the output mask)."""
+    """y = act(x W^T + b) with its backward (ReLU folded in through the output mask).  With ``bn`` (the BatchNorm1d
+    module and its parameter / gradient views) y = ReLU(BN(x W^T + b)) on batch statistics; with ``p`` > 0 the ReLU
+    output is followed by inverted dropout.  ``fwd`` returns (y, state); ``bwd`` takes that state back."""
 
-    def __init__(self, w, b, relu, gw, gb):
+    def __init__(self, w, b, relu, gw, gb, bn=None, p=0.0, key=None):
         self.w, self.b, self.relu, self.gw, self.gb = w, b, relu, gw, gb
+        self.bn, self.p, self.key = bn, float(p), key
 
-    def fwd(self, x):
-        return gemm(x, self.w, tb=True, bias=self.b, relu=self.relu)
+    def fwd(self, x, drop=None, out=None, tag=''):
+        if self.bn is None:
+            y = gemm(x, self.w, tb=True, bias=self.b, relu=self.relu, out=out)
+            if self.p:
+                call, mask = drop.next(self.key + tag, y.shape, y.device)
+                check(lib().mpn_dropout_forward(ptr(y), _ld(y), y.shape[0], y.shape[1], self.p, drop.seed,
+                                                ptr(drop.counter), call, ptr(mask), stream_ptr()), 'dropout')
+            return y, None
+        mod, gamma, beta = self.bn['mod'], self.bn['gamma'], self.bn['beta']
+        z = gemm(x, self.w, tb=True, bias=self.b)
+        if out is None:
+            out = torch.empty_like(z)
+        stats = torch.empty((4, z.shape[1]), dtype=torch.float32, device=z.device)
+        call, mask = drop.next(self.key + tag, z.shape, z.device) if self.p else (0, None)
+        check(lib().mpn_batchnorm_forward(ptr(z), _ld(z), z.shape[0], z.shape[1], ptr(gamma), ptr(beta), float(mod.eps),
+                                          float(mod.momentum), ptr(mod.running_mean), ptr(mod.running_var),
+                                          ptr(mod.num_batches_tracked), ptr(stats), self.p,
+                                          drop.seed if self.p else 0, ptr(drop.counter) if self.p else None, call,
+                                          ptr(out), _ld(out), ptr(mask), stream_ptr()), 'batchnorm')
+        return out, (z, stats)
 
-    def bwd(self, x, y, gy, need_gx=True):
-        mask = y if self.relu else None
-        gemm(gy, x, ta=True, mask=mask, out=self.gw, accumulate=True)         # gW += (gy*[y>0])^T x
-        colsum(gy, mask=mask, out=self.gb, accumulate=True)
-        return gemm(gy, self.w, mask=mask) if need_gx else None               # gx = (gy*[y>0]) W
+    def bwd(self, x, y, gy, state=None, need_gx=True, out=None, accumulate=False):
+        scale = 1.0 / (1.0 - self.p)
+        if self.bn is not None:                      # gradient w.r.t. the Linear output z: no mask left to apply
+            z, stats = state
+            gz, mask = torch.empty_like(z), None
+            check(lib().mpn_batchnorm_backward(ptr(z), _ld(z), ptr(gy), _ld(gy), ptr(y), _ld(y), z.shape[0], z.shape[1],
+                                               ptr(self.bn['gamma']), ptr(stats), scale, ptr(self.bn['ggamma']),
+                                               ptr(self.bn['gbeta']), ptr(gz), _ld(gz), stream_ptr()), 'batchnorm_backward')
+        elif self.p:
+            gz, mask = torch.empty_like(y), None
+            check(lib().mpn_dropout_backward(ptr(gy), _ld(gy), ptr(y), _ld(y), y.shape[0], y.shape[1], scale, ptr(gz),
+                                             _ld(gz), stream_ptr()), 'dropout_backward')
+        else:
+            gz, mask = gy, (y if self.relu else None)
+        gemm(gz, x, ta=True, mask=mask, out=self.gw, accumulate=True)         # gW += (gy*[y>0])^T x
+        colsum(gz, mask=mask, out=self.gb, accumulate=True)
+        return gemm(gz, self.w, mask=mask, out=out, accumulate=accumulate) if need_gx else None   # gx = (gy*[y>0]) W
 
 
 CORE_PREFIXES = ('encoder.', 'classifier.', 'MPNet.')
@@ -124,15 +189,18 @@ class AttnAggregate(torch.autograd.Function):
 class CoreTrainer:
     """Owns a flat parameter / gradient / Adam-state bucket for the core network of a ``MOTMPNet``."""
 
-    def __init__(self, model, lr=1e-3, weight_decay=1e-4, betas=(0.9, 0.999), eps=1e-8):
+    def __init__(self, model, lr=1e-3, weight_decay=1e-4, betas=(0.9, 0.999), eps=1e-8, seed=None):
+        """``seed`` keys the dropout masks (default ``torch.initial_seed()``); with the device-side forward counter it
+        fixes every mask, so two trainers with the same seed draw the same masks forward for forward."""
         self.model = model
-        from .models.mlp import MLP
+        from .models.mpn import _agg_name
+        self.agg = _agg_name(model.MPNet.node_model.node_agg_fn)
+        if self.agg not in AGG_MODES:
+            raise NotImplementedError(f'node_agg_fn {self.agg!r}: the training kernels aggregate by sum / mean / max')
         for name, mod in model.named_modules():
-            if isinstance(mod, MLP) and name.startswith(CORE_PREFIXES) and (mod.use_batchnorm or mod.dropout_p != 0):
-                raise NotImplementedError(f'{name}: BatchNorm / Dropout are not built into the training kernels '
-                                          '(the shipped configs train with use_batchnorm: False, dropout_p: 0)')
-        if model.MPNet.node_model.node_agg_fn != 'sum':
-            raise NotImplementedError("training kernels are built for node_agg_fn = 'sum'")
+            if name.startswith(CORE_PREFIXES) and isinstance(mod, torch.nn.BatchNorm1d) and mod.momentum is None:
+                raise NotImplementedError(f'{name}: BatchNorm1d with momentum=None (cumulative average) is not built '
+                                          'into the training kernels')
         self.named = OrderedDict((n, p) for n, p in model.named_parameters() if n.startswith(CORE_PREFIXES))
         dev = next(iter(self.named.values())).device
         total = sum(p.numel() for p in self.named.values())
@@ -150,19 +218,43 @@ class CoreTrainer:
             off += k
         self.lr, self.weight_decay, self.betas, self.eps = lr, weight_decay, betas, eps
         self.t_dev = torch.zeros(1, dtype=torch.int64, device=dev)        # Adam step number, kept on the device
+        self.seed = torch.initial_seed() if seed is None else int(seed)
+        self.fwd_dev = torch.zeros(1, dtype=torch.int64, device=dev)      # training forwards so far (dropout counter)
         self._prep_cache, self._graphed = {}, {}
         object.__setattr__(model, '_core_trainer', self)       # one flat bucket per model: MOTMPNet.forward reuses it under autograd
 
     # ---------------------------------------------------------------- helpers
-    def _lin(self, prefix, slot, relu):
+    def _lin(self, prefix, slot, relu, bn=None, p=0.0):
         w, b = self.named[f'{prefix}.{slot}.weight'], self.named[f'{prefix}.{slot}.bias']
-        return _Linear(w.data, b.data, relu, self.g[f'{prefix}.{slot}.weight'], self.g[f'{prefix}.{slot}.bias'].view(-1))
+        return _Linear(w.data, b.data, relu, self.g[f'{prefix}.{slot}.weight'], self.g[f'{prefix}.{slot}.bias'].view(-1),
+                       bn=bn, p=p, key=f'{prefix}.{slot}')
 
     def _mlp(self, prefix):
+        """The Linear layers of the MLP at ``prefix`` (models/mlp.py), each with the BatchNorm1d that follows it and the
+        dropout probability of its ReLU output."""
+        mlp = self.model.get_submodule(prefix)
+        layers = list(mlp.fc_layers)
         slots = sorted({int(n[len(prefix) + 1:].split('.')[1]) for n in self.named
-                        if n.startswith(prefix + '.fc_layers.') and n.endswith('.weight')})
-        return [self._lin(prefix + '.fc_layers', s, self.named[f'{prefix}.fc_layers.{s}.weight'].shape[0] != 1)
-                for s in slots]
+                        if n.startswith(prefix + '.fc_layers.') and self.named[n].dim() == 2})
+        out = []
+        for s in slots:
+            relu = self.named[f'{prefix}.fc_layers.{s}.weight'].shape[0] != 1
+            bn = None
+            if s + 1 < len(layers) and isinstance(layers[s + 1], torch.nn.BatchNorm1d):
+                k = f'{prefix}.fc_layers.{s + 1}'
+                bn = dict(mod=layers[s + 1], gamma=self.named[k + '.weight'].data, beta=self.named[k + '.bias'].data,
+                          ggamma=self.g[k + '.weight'], gbeta=self.g[k + '.bias'])
+            out.append(self._lin(prefix + '.fc_layers', s, relu, bn=bn, p=mlp.dropout_p if relu else 0.0))
+        return out
+
+    def _forward_state(self):
+        """Device state a training forward changes besides activations: BatchNorm running statistics and counters and the
+        dropout forward counter."""
+        bufs = [self.fwd_dev]
+        for name, mod in self.model.named_modules():
+            if name.startswith(CORE_PREFIXES) and isinstance(mod, torch.nn.BatchNorm1d):
+                bufs += [mod.running_mean, mod.running_var, mod.num_batches_tracked]
+        return bufs
 
     # ---------------------------------------------------------------- forward + backward
     def loss_and_grads(self, data, edge_labels, tracking_weight=1.0, zero_grad=True, prep=None):
@@ -191,9 +283,11 @@ class CoreTrainer:
         ptr_c[1:] = torch.cumsum(torch.bincount(scol.long(), minlength=n), 0).to(torch.int32)
         return dict(lay=lay, n=n, e=e, srow=srow, scol=scol, sedge=sedge, perm_c=perm_c, ptr_c=ptr_c)
 
-    def forward_core(self, data, prep=None, all_steps=False):
+    def forward_core(self, data, prep=None, all_steps=False, keep_masks=False):
         """Forward with stored activations.  Returns (logits [num_class_steps, E] in SLOT order, ctx); ``ctx['sedge']``
-        maps a slot to the caller's edge id."""
+        maps a slot to the caller's edge id.  BatchNorm layers normalise with the statistics of this call's rows and move
+        their running statistics; dropout draws the masks of the next forward number.  ``keep_masks`` (tests) stores
+        every dropout mask, in slot order, in ``ctx['masks']`` under '<Linear name>@<step>[.out|.in]'."""
         m = self.model
         x = data.x
         pooled = ops.avgpool(x) if x.dim() > 2 else x.contiguous()
@@ -214,15 +308,22 @@ class CoreTrainer:
                 raise NotImplementedError(f'the training kernels expect two-layer MLPs; the {what} has {len(mlp_)} layers')
         dn, de = node_lin.w.shape[0], edge_mlp[-1].w.shape[0]
         fh = flow['out'][0].w.shape[0]
+        if steps == 0:
+            raise NotImplementedError('training with num_enc_steps == 0')
+        drop = _Dropout(self.seed, self.fwd_dev, keep_masks)
+        if any(l.p for l in enc_n + enc_e + edge_mlp + flow['out'] + flow['in'] + cls):
+            self.fwd_dev.add_(1)
 
         # ---- encoders (activations kept)
-        acts_n = [pooled]
+        acts_n, st_n = [pooled], []
         for l in enc_n:
-            acts_n.append(l.fwd(acts_n[-1]))
+            y, st = l.fwd(acts_n[-1], drop)
+            acts_n.append(y); st_n.append(st)
         x0 = acts_n[-1]
-        acts_e = [ops.gather_rows(data.edge_attr.contiguous(), sedge) if e else data.edge_attr.new_empty((0, 6))]
+        acts_e, st_e = [ops.gather_rows(data.edge_attr.contiguous(), sedge) if e else data.edge_attr.new_empty((0, 6))], []
         for l in enc_e:
-            acts_e.append(l.fwd(acts_e[-1]))
+            y, st = l.fwd(acts_e[-1], drop)
+            acts_e.append(y); st_e.append(st)
         e0 = acts_e[-1]
 
         # ---- message-passing steps
@@ -233,32 +334,37 @@ class CoreTrainer:
             gather_cols(x0, srow, a, 0); gather_cols(xs, srow, a, dn)
             gather_cols(x0, scol, a, 2 * dn); gather_cols(xs, scol, a, 3 * dn)
             gather_cols(e0, None, a, 4 * dn); gather_cols(es, None, a, 4 * dn + de)
-            h = edge_mlp[0].fwd(a)
-            e2 = edge_mlp[1].fwd(h)
-            c1 = cls[0].fwd(e2)
-            lg = cls[1].fwd(c1)
+            tag = f'@{step}'
+            h, st_h = edge_mlp[0].fwd(a, drop, tag=tag)
+            e2, st_e2 = edge_mlp[1].fwd(h, drop, tag=tag)
+            c1, st_c1 = cls[0].fwd(e2, drop, tag=tag)
+            lg, _ = cls[1].fwd(c1)
             b = torch.empty((e, 2 * dn + de), dtype=torch.float32, device=dev)
             gather_cols(a[:, 2 * dn:4 * dn], None, b, 0); gather_cols(e2, None, b, 2 * dn)
             g_ = torch.empty((e, fh), dtype=torch.float32, device=dev)
             msg = torch.empty((e, dn), dtype=torch.float32, device=dev)
             f = torch.empty((n, 2 * dn), dtype=torch.float32, device=dev)
+            argmax = torch.empty((2, n, dn), dtype=torch.int32, device=dev) if self.agg == 'max' else None
+            st_flow = {}
             for name, s0, s1, coff in ranges:
-                if s1 > s0:
-                    gemm(b[s0:s1], flow[name][0].w, tb=True, bias=flow[name][0].b, relu=True, out=g_[s0:s1])
-                    gemm(g_[s0:s1], flow[name][1].w, tb=True, bias=flow[name][1].b, relu=True, out=msg[s0:s1])
-                segment_sum(msg, 0, dn, lay.out_ptr if name == 'out' else lay.in_ptr, None, f, coff)
-            xs_new = node_lin.fwd(f)
-            saved.append((a, h, e2, c1, b, g_, msg, f, xs_new))
+                # BatchNorm takes the statistics of this direction's rows and counts the call even when it has none
+                if s1 > s0 or flow[name][0].bn is not None:
+                    _, st0 = flow[name][0].fwd(b[s0:s1], drop, out=g_[s0:s1], tag=f'{tag}.{name}')
+                    _, st1 = flow[name][1].fwd(g_[s0:s1], drop, out=msg[s0:s1], tag=f'{tag}.{name}')
+                    st_flow[name] = (st0, st1)
+                segment_sum(msg, 0, dn, lay.out_ptr if name == 'out' else lay.in_ptr, None, f, coff, mode=self.agg,
+                            argmax=None if argmax is None else argmax[coff // dn])
+            xs_new, _ = node_lin.fwd(f)
+            saved.append(dict(a=a, h=h, e2=e2, c1=c1, b=b, g_=g_, msg=msg, f=f, xs_new=xs_new, argmax=argmax,
+                              st=(st_h, st_e2, st_c1), st_flow=st_flow))
             if all_steps or step >= first_cls:
                 logits.append(lg.view(-1))
                 logit_steps.append(step)
             xs, es = xs_new, e2
-        if steps == 0:
-            raise NotImplementedError('training with num_enc_steps == 0')
 
         ctx = dict(lay=lay, sedge=sedge, srow=srow, scol=scol, perm_c=perm_c, ptr_c=ptr_c, n=n, e=e, n_out=n_out,
-                   steps=steps, first_cls=first_cls, saved=saved, acts_n=acts_n, acts_e=acts_e, dn=dn, de=de,
-                   logit_steps=logit_steps)
+                   steps=steps, first_cls=first_cls, saved=saved, acts_n=acts_n, acts_e=acts_e, st_n=st_n, st_e=st_e,
+                   dn=dn, de=de, logit_steps=logit_steps, masks=drop.masks)
         return torch.stack(logits), ctx
 
     def backward_core(self, ctx, g_logits):
@@ -283,28 +389,31 @@ class CoreTrainer:
         gx0 = torch.zeros((n, dn), dtype=torch.float32, device=dev)
         ge0 = torch.zeros((e, de), dtype=torch.float32, device=dev)
         for step in range(steps, 0, -1):
-            a, h, e2, c1, b, g_, msg, f, xs_new = saved[step - 1]
+            sv = saved[step - 1]
+            a, h, e2, c1, b, g_, msg, f, xs_new = (sv[k] for k in ('a', 'h', 'e2', 'c1', 'b', 'g_', 'msg', 'f', 'xs_new'))
+            st_h, st_e2, st_c1 = sv['st']
             gf = node_lin.bwd(f, xs_new, gxs)                                           # [n, 2dn]
             gmsg = torch.empty((e, dn), dtype=torch.float32, device=dev)
             gb = torch.empty((e, 2 * dn + de), dtype=torch.float32, device=dev)
             for name, s0, s1, coff in ranges:
                 if s1 <= s0:
                     continue
-                gather_cols(gf[:, coff:coff + dn], srow[s0:s1], gmsg[s0:s1], 0)       # d flow[row] -> each message
+                if self.agg == 'sum':                                                   # d flow[row] -> each message
+                    gather_cols(gf[:, coff:coff + dn], srow[s0:s1], gmsg[s0:s1], 0)
+                else:
+                    segment_grad(gf[:, coff:coff + dn], srow, lay.out_ptr if name == 'out' else lay.in_ptr,
+                                 None if sv['argmax'] is None else sv['argmax'][coff // dn], s0, s1, self.agg, gmsg)
                 l0, l1 = flow[name]
-                gg = l1.bwd(g_[s0:s1], msg[s0:s1], gmsg[s0:s1])
-                gemm(gg, b[s0:s1], ta=True, mask=g_[s0:s1], out=l0.gw, accumulate=True)
-                colsum(gg, mask=g_[s0:s1], out=l0.gb, accumulate=True)
-                gemm(gg, l0.w, mask=g_[s0:s1], out=gb[s0:s1])
+                st0, st1 = sv['st_flow'][name]
+                gg = l1.bwd(g_[s0:s1], msg[s0:s1], gmsg[s0:s1], st1)
+                l0.bwd(b[s0:s1], g_[s0:s1], gg, st0, out=gb[s0:s1])
             ge2 = ge2_next + gb[:, 2 * dn:]                                             # e' feeds the flow MLPs and step+1
             if step in row_of:
                 gl = g_logits[row_of[step]].view(-1, 1)
                 gc1 = cls[1].bwd(c1, None, gl)
-                gemm(gc1, e2, ta=True, mask=c1, out=cls[0].gw, accumulate=True)
-                colsum(gc1, mask=c1, out=cls[0].gb, accumulate=True)
-                gemm(gc1, cls[0].w, mask=c1, out=ge2, accumulate=True)
-            gh = edge_mlp[1].bwd(h, e2, ge2)
-            ga = edge_mlp[0].bwd(a, h, gh)                                              # [e, 4dn+2de]
+                cls[0].bwd(e2, c1, gc1, st_c1, out=ge2, accumulate=True)
+            gh = edge_mlp[1].bwd(h, e2, ge2, st_e2)
+            ga = edge_mlp[0].bwd(a, h, gh, st_h)                                        # [e, 4dn+2de]
             gxs_new = torch.empty((n, dn), dtype=torch.float32, device=dev)
             for part, dst in ((0, gx0), (dn, gxs_new)):                                 # x_init part / x_latent part
                 acc = dst is gx0
@@ -321,10 +430,10 @@ class CoreTrainer:
         # ---- encoders
         g_act = gx0
         for i in range(len(enc_n) - 1, -1, -1):
-            g_act = enc_n[i].bwd(acts_n[i], acts_n[i + 1], g_act, need_gx=i > 0)
+            g_act = enc_n[i].bwd(acts_n[i], acts_n[i + 1], g_act, ctx['st_n'][i], need_gx=i > 0)
         g_act = ge0
         for i in range(len(enc_e) - 1, -1, -1):
-            g_act = enc_e[i].bwd(acts_e[i], acts_e[i + 1], g_act, need_gx=i > 0)
+            g_act = enc_e[i].bwd(acts_e[i], acts_e[i + 1], g_act, ctx['st_e'][i], need_gx=i > 0)
 
     # ---------------------------------------------------------------- autograd bridge
     def autograd_logits(self, data, all_steps=False):
@@ -380,6 +489,7 @@ class _GraphedStep(object):
         tr = self.trainer = trainer
         self.data, self.labels = data, edge_labels.to(data.edge_index.device, torch.float32).contiguous()
         self.prep = tr.prepare(data)
+        state = [t.clone() for t in tr._forward_state()]
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):                                   # warm-up off the capture (allocator, lazy inits)
@@ -387,6 +497,8 @@ class _GraphedStep(object):
                 tr.loss_and_grads(data, self.labels, tracking_weight, prep=self.prep)
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
+        for t, s in zip(tr._forward_state(), state):                    # the warm-up forwards do not count as steps
+            t.copy_(s)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             self.loss = tr.loss_and_grads(data, self.labels, tracking_weight, prep=self.prep)
