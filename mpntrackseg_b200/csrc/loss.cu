@@ -2,6 +2,7 @@
 //   pos_weight = (#edges - #positives) / #positives   (0 when there is no positive label)
 //   loss = weight * sum_steps mean_edges BCEWithLogits(logits_s, labels, pos_weight)
 // plus d loss / d logits (the seed of the backward pass).  Reductions are fixed-order (deterministic).
+// Per edge: term (1 - y) softplus(x) + pw y softplus(-x), gradient weight / E ((1 - y) sigmoid(x) - pw y sigmoid(-x)).
 #include <math.h>
 
 #include "common.cuh"
@@ -18,6 +19,14 @@ __device__ __forceinline__ double block_sum(double v, double* sm) {
   if (threadIdx.x == 0) for (int w = 0; w < LB / 32; ++w) t += sm[w];
   __syncthreads();
   return t;                                            // valid in thread 0
+}
+
+// softplus(x) = log(1 + e^x) and sigmoid(x) = 1 / (1 + e^-x), both accurate relative to their value for every x
+// (sigmoid(x) of a very negative x is e^x, not the difference 1 - sigmoid(-x), which rounds to 0 below x = -17)
+__device__ __forceinline__ float softplus(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
+__device__ __forceinline__ float sigmoid(float x) {
+  const float t = expf(-fabsf(x));                                 // no overflow: e^x / (1 + e^x) below 0
+  return x < 0.f ? t / (1.f + t) : 1.f / (1.f + t);
 }
 
 __global__ void __launch_bounds__(LB) label_partials_kernel(const float* __restrict__ labels, int64_t e,
@@ -47,13 +56,10 @@ __global__ void __launch_bounds__(LB) bce_partials_kernel(const float* __restric
   double s = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * LB + threadIdx.x; i < steps * e; i += (int64_t)gridDim.x * LB) {
     const float x = logits[i], y = labels[i % e];
-    const float lw = 1.f + (pw - 1.f) * y;
-    const float sp = log1pf(expf(-fabsf(x))) + fmaxf(-x, 0.f);      // softplus(-x)
-    s += (double)((1.f - y) * x + lw * sp);
-    if (grad != nullptr) {
-      const float sig_neg = 1.f / (1.f + expf(x));                  // sigmoid(-x)
-      grad[i] = weight * inv_e * ((1.f - y) - lw * sig_neg);
-    }
+    const float wn = 1.f - y, wp = pw * y;                           // weights of the negative / positive side
+    // (1 - y) sp(x) + pw y sp(-x): no term cancels, and a side of weight 0 adds 0 even where its softplus is inf
+    s += (double)((wn != 0.f ? wn * softplus(x) : 0.f) + (wp != 0.f ? wp * softplus(-x) : 0.f));
+    if (grad != nullptr) grad[i] = weight * inv_e * (wn * sigmoid(x) - wp * sigmoid(-x));
   }
   s = block_sum(s, sm);
   if (threadIdx.x == 0) partial[blockIdx.x] = s;

@@ -196,18 +196,20 @@ __device__ __forceinline__ bool dropout_keep(uint64_t seed, const int64_t* __res
 
 // Per-slice column partials over rows [r0, r1) in a fixed order (the layout of colsum_kernel):
 //   what 0: sum z;  1: sum (z - mean)^2;  2: sum g' and sum g' xhat  with g' = y > 0 ? g * gscale : 0,
-//   xhat = (z - mean) invstd.  partial: [slices][n] (what 2: a second [slices][n] block follows).
+//   xhat = (z - mean) invstd.  partial: [slices][n] (what 2: a second [slices][n] block follows).  The sums run in
+//   double: a thread adds up to rows_per_slice / 8 rows (977 at 10^6 rows), and an fp32 sum of that many equal values
+//   drifts by ~1e-5 of the mean, which a column of large offset turns into an error of the normalised output.
 __global__ void __launch_bounds__(256) bn_partial_kernel(const float* __restrict__ z, int64_t ldz,
                                                          const float* __restrict__ g, int64_t ldg,
                                                          const float* __restrict__ y, int64_t ldy,
                                                          const float* __restrict__ stats, float gscale, int64_t m,
                                                          int64_t n, int64_t rows_per_slice, int what,
-                                                         float* __restrict__ partial) {
-  __shared__ float part[2][8][33];
+                                                         double* __restrict__ partial) {
+  __shared__ double part[2][8][33];
   const int col = blockIdx.x * 32 + (threadIdx.x & 31), rgrp = threadIdx.x >> 5;
   const int64_t r0 = (int64_t)blockIdx.y * rows_per_slice;
   const int64_t r1 = r0 + rows_per_slice < m ? r0 + rows_per_slice : m;
-  float s0 = 0.f, s1 = 0.f;
+  double s0 = 0.0, s1 = 0.0;
   if (col < n) {
     const float mu = what > 0 ? stats[col] : 0.f, is = what == 2 ? stats[n + col] : 0.f;
     for (int64_t r = r0 + rgrp; r < r1; r += 8) {
@@ -225,7 +227,7 @@ __global__ void __launch_bounds__(256) bn_partial_kernel(const float* __restrict
   part[1][rgrp][threadIdx.x & 31] = s1;
   __syncthreads();
   if (rgrp == 0 && col < n) {
-    float t0 = 0.f, t1 = 0.f;
+    double t0 = 0.0, t1 = 0.0;
     for (int k = 0; k < 8; ++k) { t0 += part[0][k][threadIdx.x & 31]; t1 += part[1][k][threadIdx.x & 31]; }
     partial[(int64_t)blockIdx.y * n + col] = t0;
     if (what == 2) partial[((int64_t)gridDim.y + blockIdx.y) * n + col] = t1;
@@ -238,21 +240,22 @@ __global__ void __launch_bounds__(256) bn_partial_kernel(const float* __restrict
 //           unbiased one (torch.nn.BatchNorm1d), and *num_batches_tracked += 1 (also for m == 0, which changes nothing
 //           else);
 //   what 2: ggamma += sum g' xhat, gbeta += sum g', stats[2n:3n] / stats[3n:4n] = their means over the rows.
-__global__ void bn_finalize_kernel(const float* __restrict__ partial, int slices, int64_t m, int64_t n, int what,
+__global__ void bn_finalize_kernel(const double* __restrict__ partial, int slices, int64_t m, int64_t n, int what,
                                    float eps, float momentum, float* __restrict__ stats, float* __restrict__ running_mean,
                                    float* __restrict__ running_var, int64_t* __restrict__ num_batches_tracked,
                                    float* __restrict__ ggamma, float* __restrict__ gbeta) {
   if (what == 1 && num_batches_tracked != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *num_batches_tracked += 1;
   if (m == 0) return;
   for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (int64_t)gridDim.x * blockDim.x) {
-    float t0 = 0.f, t1 = 0.f;
-    for (int k = 0; k < slices; ++k) t0 += partial[(int64_t)k * n + c];
+    double d0 = 0.0, d1 = 0.0;
+    for (int k = 0; k < slices; ++k) d0 += partial[(int64_t)k * n + c];
     if (what == 2)
-      for (int k = 0; k < slices; ++k) t1 += partial[(int64_t)(slices + k) * n + c];
+      for (int k = 0; k < slices; ++k) d1 += partial[(int64_t)(slices + k) * n + c];
+    const float t0 = (float)d0, t1 = (float)d1;
     if (what == 0) {
-      stats[c] = t0 / (float)m;
+      stats[c] = (float)(d0 / (double)m);
     } else if (what == 1) {
-      const float var = t0 / (float)m;
+      const float var = (float)(d0 / (double)m);
       stats[n + c] = 1.f / sqrtf(var + eps);
       running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * stats[c];
       running_var[c] = (1.f - momentum) * running_var[c] + momentum * (var * (float)m / (float)(m - 1));
@@ -496,8 +499,8 @@ int mpn_batchnorm_forward(const float* z, int64_t ldz, int64_t m, int64_t n, con
   }
   keep_async_pool();
   const int64_t slices = bn_slices(m), rps = ceil_div(m, slices);
-  float* partial = nullptr;
-  MPN_CUDA(cudaMallocAsync(&partial, sizeof(float) * slices * n, s));
+  double* partial = nullptr;
+  MPN_CUDA(cudaMallocAsync(&partial, sizeof(double) * slices * n, s));
   const dim3 grid((unsigned)ceil_div(n, 32), (unsigned)slices);
   const unsigned fgrid = (unsigned)ceil_div(n, 256);
   for (int what = 0; what < 2; ++what) {              // mean, then the variance around it (two passes)
@@ -521,8 +524,8 @@ int mpn_batchnorm_backward(const float* z, int64_t ldz, const float* g, int64_t 
   cudaStream_t s = as_stream(stream);
   keep_async_pool();
   const int64_t slices = bn_slices(m), rps = ceil_div(m, slices);
-  float* partial = nullptr;
-  MPN_CUDA(cudaMallocAsync(&partial, sizeof(float) * 2 * slices * n, s));
+  double* partial = nullptr;
+  MPN_CUDA(cudaMallocAsync(&partial, sizeof(double) * 2 * slices * n, s));
   bn_partial_kernel<<<dim3((unsigned)ceil_div(n, 32), (unsigned)slices), 256, 0, s>>>(z, ldz, g, ldg, y, ldy, stats, gscale,
                                                                                      m, n, rps, 2, partial);
   bn_finalize_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, s>>>(partial, (int)slices, m, n, 2, 0.f, 0.f, stats, nullptr,
