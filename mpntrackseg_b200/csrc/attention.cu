@@ -69,9 +69,17 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_aggregate_kernel(
 // ------------------------------------------------------------------ backward (training through the mask branch)
 // Given G_dir[n] = d loss / d flow_dir[n]:
 //   d w_q     = < G_dir[n], z[col_q] >                        (one warp per neighbour, fixed-order tree)
-//   d logit_q = w_q (d w_q - sum_p w_p d w_p)                  (softmax backward; the 1e-12 in the denominator keeps this form)
+//   d logit_q = w_q (d w_q - S),  S = sum_p w_p d w_p          (softmax backward; the 1e-12 in the denominator keeps this form)
+//   except for the dominant slot q* (largest logit, lowest slot among ties), whose w -> 1 would cancel dw_q* - S:
+//   d logit_q* = w_q* (dw_q* W' - T'),  W' = sum_{p != q*} w_p,  T' = sum_{p != q*} w_p dw_p   (0 for a 1-slot segment)
+//   S, W', T' are summed in double by thread 0 in slot order.
 //   d z[c]    = sum over the slots q with col_q = c of w_q G_dir(q)[row_q]   (second kernel, slots of a column in slot order)
-__global__ void __launch_bounds__(ATT_THREADS) attn_backward_edge_kernel(
+__device__ __forceinline__ float attn_d_logit(float w, float dw, bool dominant, double S, double Wo, double To) {
+  return dominant ? (float)((double)w * ((double)dw * Wo - To)) : (float)((double)w * ((double)dw - S));
+}
+
+// 5 blocks per SM: 48 registers; the serial loop of thread 0 stays rolled, so nothing spills
+__global__ void __launch_bounds__(ATT_THREADS, 5) attn_backward_edge_kernel(
     const float* __restrict__ z, int64_t feat, const int32_t* __restrict__ slot_col, const int32_t* __restrict__ slot_edge,
     const int32_t* __restrict__ out_ptr, const int32_t* __restrict__ in_ptr, const float* __restrict__ logits,
     const float* __restrict__ g_in, const float* __restrict__ g_out, float* __restrict__ w_slot,
@@ -79,7 +87,8 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_backward_edge_kernel(
   __shared__ float s_w[ATT_MAX_DEG];
   __shared__ float s_dw[ATT_MAX_DEG];
   __shared__ float s_red[32];
-  __shared__ float s_dot;
+  __shared__ int s_qred[32];
+  __shared__ double s_S, s_Wo, s_To;
   const int64_t node = blockIdx.x >> 1;
   const int dir = blockIdx.x & 1;
   const int32_t* ptr = dir == 0 ? in_ptr : out_ptr;
@@ -97,15 +106,23 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_backward_edge_kernel(
   for (int w = 1; w < ATT_THREADS / 32; ++w) m = fmaxf(m, s_red[w]);
   __syncthreads();
   float sum = 0.f;
-  for (int q = tid; q < deg; q += ATT_THREADS) sum += expf(logits[slot_edge[s0 + q]] - m);
-  for (int d = 16; d > 0; d >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, d);
-  if (lane == 0) s_red[warp] = sum;
+  int qs = deg;                                           // the dominant slot: the first one whose logit is the max
+  for (int q = tid; q < deg; q += ATT_THREADS) {
+    const float l = logits[slot_edge[s0 + q]];
+    sum += expf(l - m);
+    if (l == m && qs == deg) qs = q;
+  }
+  for (int d = 16; d > 0; d >>= 1) {
+    sum += __shfl_xor_sync(0xffffffffu, sum, d);
+    qs = min(qs, __shfl_xor_sync(0xffffffffu, qs, d));
+  }
+  if (lane == 0) { s_red[warp] = sum; s_qred[warp] = qs; }
   __syncthreads();
   sum = 0.f;
-  for (int w = 0; w < ATT_THREADS / 32; ++w) sum += s_red[w];
+  for (int w = 0; w < ATT_THREADS / 32; ++w) { sum += s_red[w]; qs = min(qs, s_qred[w]); }
   const float inv = 1.f / (sum + 1e-12f);
-  float carry = 0.f;                                      // sum_p w_p dw_p over the passes (thread 0)
-  for (int pass = 0; pass < 2; ++pass) {                  // pass 0: the weighted mean of dw; pass 1: d logits
+  if (tid == 0) { s_S = 0.0; s_Wo = 0.0; s_To = 0.0; }   // accumulated by thread 0 over the chunks of pass 0
+  for (int pass = 0; pass < 2; ++pass) {                  // pass 0: S, W', T'; pass 1: d logits
     for (int q0 = 0; q0 < deg; q0 += ATT_MAX_DEG) {
       const int nq = deg - q0 < ATT_MAX_DEG ? deg - q0 : ATT_MAX_DEG;
       __syncthreads();
@@ -119,21 +136,29 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_backward_edge_kernel(
       }
       __syncthreads();
       if (pass == 0) {
-        if (tid == 0) { for (int q = 0; q < nq; ++q) carry = fmaf(s_w[q], s_dw[q], carry); }
+        if (tid == 0) {
+          double S = s_S, Wo = s_Wo, To = s_To;
+#pragma unroll 1
+          for (int q = 0; q < nq; ++q) {
+            const double wd = (double)s_w[q] * (double)s_dw[q];
+            S += wd;
+            if (q0 + q != qs) { Wo += (double)s_w[q]; To += wd; }
+          }
+          s_S = S; s_Wo = Wo; s_To = To;
+        }
       } else {
         for (int q = tid; q < nq; q += ATT_THREADS) {
           w_slot[s0 + q0 + q] = s_w[q];
-          d_logits[slot_edge[s0 + q0 + q]] = s_w[q] * (s_dw[q] - s_dot);
+          d_logits[slot_edge[s0 + q0 + q]] = attn_d_logit(s_w[q], s_dw[q], q0 + q == qs, s_S, s_Wo, s_To);
         }
       }
     }
     if (pass == 0) {
-      if (tid == 0) s_dot = carry;
       __syncthreads();
       if (deg <= ATT_MAX_DEG) {                           // one pass over the neighbours is enough: s_w / s_dw are still valid
         for (int q = tid; q < deg; q += ATT_THREADS) {
           w_slot[s0 + q] = s_w[q];
-          d_logits[slot_edge[s0 + q]] = s_w[q] * (s_dw[q] - s_dot);
+          d_logits[slot_edge[s0 + q]] = attn_d_logit(s_w[q], s_dw[q], q == qs, s_S, s_Wo, s_To);
         }
         break;
       }
