@@ -378,6 +378,37 @@ int64_t mpn_connected_components_workspace(int64_t num_nodes);
 int mpn_connected_components(const int64_t* row, const int64_t* col, const float* edge_vals, int64_t num_edges,
                              int64_t num_nodes, void* workspace, int64_t* labels, int64_t* h_num_components, void* stream);
 
+/* ------------------------------------------------------------------ MOTS output (after identity assignment)
+ * tracker/mpn_tracker.py:267-298 + :398-417: each node's mask pasted into its frame (torchvision's
+ * paste_masks_in_image), one owner per pixel within a frame, pycocotools RLE of every mask.  masks [N, M, M] fp32
+ * probabilities; boxes [N, 4] int64 (x0, y0, x1, y1) = torchvision's expand_boxes(box, (M + 2 padding) / M) truncated
+ * to integers (the caller computes them in its own dtype); the image is height x width with height * width <= 2^31 - 1.
+ * p_i(y, x) = the zero-padded (M + 2 padding)^2 mask resized to h = max(y1 - y0 + 1, 1) by w = max(x1 - x0 + 1, 1)
+ * with ATen's bilinear interpolation (align_corners = False), read at (y - y0, x - x0) inside the box clamped to the
+ * image, 0 elsewhere; evaluated in double. */
+
+/* out [N, H, W] fp32 = p_i(y, x): the dense paste, torchvision's paste_masks_in_image. */
+int mpn_paste_masks(const float* masks, int64_t num_nodes, int64_t mask_size, int32_t padding, const int64_t* boxes,
+                    int64_t height, int64_t width, float* out, void* stream);
+
+/* Run-length encoding of the masks.  Within a frame (frame [N] int64, non-decreasing) pixel (y, x) belongs to the
+ * node with the largest p_i(y, x), ties to the lower node index, NaN counting as -inf; node i's mask is the set of
+ * pixels it owns where p_i > threshold.  Its RLE is pycocotools' rleEncode of the column-major H x W image (counts
+ * start with the zeros, possibly 0) and its string rleToString's.  A node with an empty mask has no counts and no
+ * characters.  Two phases, like mpn_time_valid_pairs_count / _fill:
+ * _count writes area [N] (pixels of the mask) and the exclusive scans cnt_ptr / char_ptr [N+1] of each node's number of
+ * counts and of characters; h_totals (host) = {total counts, total characters}.  MPN_EINVAL if frame decreases.  SYNCS.
+ * _fill writes the int32 counts at cnt_ptr offsets and the characters (no terminator) at char_ptr offsets.
+ * workspace: mpn_mots_rle_workspace(N) bytes. */
+int64_t mpn_mots_rle_workspace(int64_t num_nodes);
+int mpn_mots_rle_count(const float* masks, int64_t num_nodes, int64_t mask_size, int32_t padding, const int64_t* boxes,
+                       const int64_t* frame, int64_t height, int64_t width, double threshold, void* workspace,
+                       int64_t* area, int64_t* cnt_ptr /*[N+1]*/, int64_t* char_ptr /*[N+1]*/, int64_t* h_totals /*[2]*/,
+                       void* stream);
+int mpn_mots_rle_fill(const float* masks, int64_t num_nodes, int64_t mask_size, int32_t padding, const int64_t* boxes,
+                      const int64_t* frame, int64_t height, int64_t width, double threshold, const int64_t* cnt_ptr,
+                      const int64_t* char_ptr, int32_t* counts, uint8_t* chars, void* stream);
+
 /* Diagnostics of the last mpn_mp_forward_tc run on `workspace` (same n, e): the scale exponents s_t and the maxima
  * they were derived from, entries [0, num_steps + 2) indexed by step (1-based).  h_* are HOST arrays and may be
  * NULL.  SYNCS. */

@@ -95,6 +95,12 @@ SIGNATURES = {
     'mpn_mp_tc_read_schedule': (C.c_int, [c_vp, c_i64, c_i64, c_i32, C.POINTER(c_i32), C.POINTER(c_f32), C.POINTER(c_f32), c_vp]),
     'mpn_mp_forward_tc': (C.c_int, [C.POINTER(CoreWeights), C.POINTER(EdgeLayout), c_vp, c_vp, c_i32, c_i32,
                                     c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'mpn_paste_masks': (C.c_int, [c_vp, c_i64, c_i64, c_i32, c_vp, c_i64, c_i64, c_vp, c_vp]),
+    'mpn_mots_rle_workspace': (c_i64, [c_i64]),
+    'mpn_mots_rle_count': (C.c_int, [c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_i64, c_i64, C.c_double, c_vp, c_vp, c_vp, c_vp,
+                                     c_i64p, c_vp]),
+    'mpn_mots_rle_fill': (C.c_int, [c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_i64, c_i64, C.c_double, c_vp, c_vp, c_vp, c_vp,
+                                    c_vp]),
 }
 
 _lib = None

@@ -59,34 +59,6 @@ constexpr int kScanItems = 8;                       // per thread
 constexpr int kScanChunk = kScanThreads * kScanItems;
 
 template <typename T>
-__device__ __forceinline__ T block_exclusive_scan(T v, T* smem /*[32]*/, T* total) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  T incl = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    T o = __shfl_up_sync(0xffffffffu, incl, d);
-    if (lane >= d) incl += o;
-  }
-  if (lane == 31) smem[warp] = incl;
-  __syncthreads();
-  if (warp == 0) {
-    T w = lane < (blockDim.x >> 5) ? smem[lane] : T(0);
-    T wi = w;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      T o = __shfl_up_sync(0xffffffffu, wi, d);
-      if (lane >= d) wi += o;
-    }
-    smem[lane] = wi - w;                            // exclusive warp offsets
-    if (lane == 31) *total = wi;
-  }
-  __syncthreads();
-  T res = smem[warp] + incl - v;
-  __syncthreads();
-  return res;
-}
-
-template <typename T>
 __global__ void scan_chunk_totals(const T* __restrict__ in, T* __restrict__ totals, int64_t n) {
   __shared__ T sm[32];
   __shared__ T tot;

@@ -50,6 +50,36 @@ void profile_mark(int kind, bool begin, cudaStream_t s);
 int exclusive_scan_i64(const int64_t* in, int64_t* out, int64_t n, cudaStream_t stream);
 int exclusive_scan_i32(const int32_t* in, int32_t* out, int64_t n, cudaStream_t stream);
 
+// Block-wide exclusive scan of one value per thread (blockDim.x a multiple of 32, at most 1024); *total gets the
+// block total.  Every thread of the block must call it; it ends with a barrier, so smem can be reused.
+template <typename T>
+__device__ __forceinline__ T block_exclusive_scan(T v, T* smem /*[32]*/, T* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  T incl = v;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    T o = __shfl_up_sync(0xffffffffu, incl, d);
+    if (lane >= d) incl += o;
+  }
+  if (lane == 31) smem[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    T w = lane < (blockDim.x >> 5) ? smem[lane] : T(0);
+    T wi = w;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      T o = __shfl_up_sync(0xffffffffu, wi, d);
+      if (lane >= d) wi += o;
+    }
+    smem[lane] = wi - w;                            // exclusive warp offsets
+    if (lane == 31) *total = wi;
+  }
+  __syncthreads();
+  T res = smem[warp] + incl - v;
+  __syncthreads();
+  return res;
+}
+
 // Bump allocator over a caller-provided workspace (256-byte aligned pieces).
 struct Carver {
   char* base;

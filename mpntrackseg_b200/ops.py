@@ -502,3 +502,75 @@ def connected_components(edge_index, edge_vals, num_nodes):
     check(lib().mpn_connected_components(ptr(ei[0]), ptr(ei[1]), ptr(v), e, n, ptr(ws), ptr(labels), C.byref(ncomp), stream_ptr()),
           'connected_components')
     return labels, ncomp.value
+
+
+# ------------------------------------------------------------------ MOTS output (tracker/mpn_tracker.py:267-298,398-417)
+def paste_boxes(boxes, mask_size, padding=1):
+    """[N, 4] int64 boxes of torchvision's ``expand_boxes(boxes, (M + 2 padding) / M).to(torch.int64)``
+    (roi_heads.py), computed with the same torch ops in the boxes' own dtype, so that the truncation toward zero sees
+    the same values."""
+    scale = float(mask_size + 2 * padding) / mask_size
+    w_half = (boxes[:, 2] - boxes[:, 0]) * 0.5
+    h_half = (boxes[:, 3] - boxes[:, 1]) * 0.5
+    x_c = (boxes[:, 2] + boxes[:, 0]) * 0.5
+    y_c = (boxes[:, 3] + boxes[:, 1]) * 0.5
+    w_half = w_half * scale
+    h_half = h_half * scale
+    return torch.stack((x_c - w_half, y_c - h_half, x_c + w_half, y_c + h_half), dim=1).to(torch.int64).contiguous()
+
+
+def _mots_inputs(masks, boxes, img_shape, padding):
+    if not torch.is_tensor(masks) or masks.dim() not in (3, 4) or (masks.dim() == 4 and masks.shape[1] != 1):
+        raise ValueError(f'masks must be [N, 1, M, M] or [N, M, M], got {tuple(getattr(masks, "shape", ()))}')
+    m = _req(masks.reshape(masks.shape[0], masks.shape[-2], masks.shape[-1]), torch.float32, 'masks')
+    n, mh, mw = m.shape
+    if mh != mw or mh == 0:
+        raise ValueError(f'masks must be square and non-empty, got {mh} x {mw}')
+    if not torch.is_tensor(boxes) or boxes.dtype not in (torch.float32, torch.float64):
+        raise TypeError('boxes: expected a float32 or float64 tensor')
+    b = _req(boxes, boxes.dtype, 'boxes')
+    if tuple(b.shape) != (n, 4):
+        raise ValueError(f'boxes must be [{n}, 4], got {tuple(b.shape)}')
+    h, w = int(img_shape[0]), int(img_shape[1])
+    if h < 1 or w < 1 or h * w >= 2 ** 31:
+        raise ValueError(f'image {h} x {w} must have 1 .. 2^31 - 1 pixels')
+    if padding < 0:
+        raise ValueError(f'padding must be >= 0, got {padding}')
+    return m, paste_boxes(b, mh, padding), n, mh, h, w
+
+
+def paste_masks_in_image(masks, boxes, img_shape, padding=1):
+    """[N, 1, H, W] fp32: torchvision's ``paste_masks_in_image`` (roi_heads.py) on the device.  masks [N, 1, M, M] fp32,
+    boxes [N, 4] (x1, y1, x2, y2) float32 / float64, img_shape (H, W).  A box with no pixel inside the image gives an
+    all-zero mask.  reference: tracker/mpn_tracker.py:267-298"""
+    m, ib, n, ms, h, w = _mots_inputs(masks, boxes, img_shape, padding)
+    out = torch.empty((n, 1, h, w), dtype=torch.float32, device=m.device)
+    check(lib().mpn_paste_masks(ptr(m), n, ms, int(padding), ptr(ib), h, w, ptr(out), stream_ptr()), 'paste_masks')
+    return out
+
+
+def mots_rle(masks, boxes, frame, img_shape, threshold=0.5):
+    """Run-length encoding of every node's pasted mask after the one-owner-per-pixel rule of its frame:
+    ``(area [N] int64, chars uint8, char_ptr [N+1] int64)``; node i's RLE string (pycocotools' ``rleToString`` format)
+    is ``chars[char_ptr[i]:char_ptr[i+1]]``, empty when its mask is.  masks [N, 1, M, M] or [N, M, M] fp32
+    probabilities, boxes [N, 4] (x1, y1, x2, y2) float32 / float64, frame [N] int64 non-decreasing, img_shape (H, W).
+    A pixel belongs to the node of its frame with the largest pasted probability (ties: lower index; NaN: -inf), and
+    to its mask where that probability is > threshold.  One host sync (the totals).  See DESIGN.md, MOTS output."""
+    padding = 1
+    m, ib, n, ms, h, w = _mots_inputs(masks, boxes, img_shape, padding)
+    f = _req(frame.reshape(-1), torch.int64, 'frame')
+    if f.numel() != n:
+        raise ValueError(f'frame has {f.numel()} entries for {n} masks')
+    dev = m.device
+    ws = _bytes(lib().mpn_mots_rle_workspace(n), dev)
+    area = torch.empty(n, dtype=torch.int64, device=dev)
+    cnt_ptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    char_ptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    totals = (C.c_int64 * 2)()
+    check(lib().mpn_mots_rle_count(ptr(m), n, ms, int(padding), ptr(ib), ptr(f), h, w, float(threshold), ptr(ws), ptr(area),
+                                   ptr(cnt_ptr), ptr(char_ptr), totals, stream_ptr()), 'mots_rle_count')
+    counts = torch.empty(max(totals[0], 1), dtype=torch.int32, device=dev)
+    chars = torch.empty(max(totals[1], 1), dtype=torch.uint8, device=dev)
+    check(lib().mpn_mots_rle_fill(ptr(m), n, ms, int(padding), ptr(ib), ptr(f), h, w, float(threshold), ptr(cnt_ptr),
+                                  ptr(char_ptr), ptr(counts), ptr(chars), stream_ptr()), 'mots_rle_fill')
+    return area, chars[:totals[1]], char_ptr

@@ -126,3 +126,24 @@ def make_params(model_params, seed=0, gain=1.0, core_only=False, dtype=torch.flo
         scale = gain if name.endswith('weight') else 1.0
         out[name] = ((torch.rand(shape, generator=g, dtype=torch.float64) * 2 - 1) * b * scale).to(dtype)
     return out
+
+
+def make_mots_sequence(frames=600, per_frame=20, height=1080, width=1920, mask_size=56, seed=0):
+    """A MOTS-shaped sequence for the mask output stage: ``per_frame`` pedestrian-shaped boxes (height 60-400 px,
+    width 0.35-0.5 of it, some partly outside the image) in each of ``frames`` frames, and smooth 56 x 56 masks (a
+    logistic ellipse per node).  Returns (masks [N,1,M,M] fp32, boxes [N,4] float64 (x1, y1, x2, y2), frame [N] int64)."""
+    g = torch.Generator().manual_seed(int(seed))
+    n = frames * per_frame
+    frame = torch.arange(1, frames + 1, dtype=torch.int64).repeat_interleave(per_frame)
+    bh = 60.0 + 340.0 * torch.rand(n, generator=g, dtype=torch.float64)
+    bw = bh * (0.35 + 0.15 * torch.rand(n, generator=g, dtype=torch.float64))
+    x1 = width * torch.rand(n, generator=g, dtype=torch.float64) - 0.5 * bw
+    y1 = (height - 0.8 * bh) * torch.rand(n, generator=g, dtype=torch.float64) - 0.1 * bh
+    boxes = torch.stack((x1, y1, x1 + bw, y1 + bh), dim=1)
+    u = (torch.arange(mask_size, dtype=torch.float32) + 0.5) / mask_size
+    cu, cv = 0.5 + 0.1 * torch.randn(2, n, 1, 1, generator=g)
+    su, sv = 0.25 + 0.15 * torch.rand(2, n, 1, 1, generator=g)
+    sharp = 3.0 + 6.0 * torch.rand(n, 1, 1, generator=g)
+    r2 = ((u.view(1, 1, -1) - cu) / su) ** 2 + ((u.view(1, -1, 1) - cv) / sv) ** 2
+    masks = torch.sigmoid(sharp * (1.0 - r2)).unsqueeze(1).contiguous()
+    return masks, boxes, frame

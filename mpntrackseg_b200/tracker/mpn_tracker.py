@@ -4,7 +4,8 @@
 hot path -- ``_predict_edges_and_masks`` (one window: KNN prune -> network -> sigmoid -> scatter back) and
 ``_evaluate_graph_in_batches`` (all overlapping windows of a sequence, per-edge averaging, directed ->
 undirected merge, pruning at 0.5).  reference: tracker/mpn_tracker.py:96-210, utils/graph.py:165-207.
-Dataset loading, rounding (projectors) and id assignment (:212-260) are outside this path.
+Dataset loading is outside this path; rounding, id assignment (:212-260) and the MOTS result (:267-298, :398-417) run on
+the device after it.
 
 B200 design of ``_evaluate_graph_in_batches`` (same results, different schedule):
   * every node of the sequence is encoded ONCE (avg-pool + 2048->128->32 on tcgen05) instead of once per
@@ -306,9 +307,41 @@ class MPNTracker(object):
         from .. import ops
         go = self.full_graph.graph_obj
         labels, _ = ops.connected_components(go.edge_index, (go.edge_preds == 1).float(), go.num_nodes)
+        self.ped_ids = labels
         df = getattr(self.full_graph, 'graph_df', None)
         if df is not None and hasattr(df, 'copy') and not isinstance(df, dict):
             assert len(labels) == df.shape[0], "Ped Ids Label format is wrong"
             self.final_projected_output = df.copy()
             self.final_projected_output['ped_id'] = labels.cpu().numpy()
         return labels
+
+    # ------------------------------------------------------------------ MOTS result
+    def save_mots_results(self, path, class_id=2, threshold=0.5):
+        """Writes the tracker's MOTS result: one line ``"<frame> <id> <class_id> <H> <W> <rle>"`` per node with a
+        non-empty mask, sorted by frame, then node index (reference: tracker/mpn_tracker.py:267-298, :398-417).  Each
+        node's averaged mask ``graph_obj.node_preds`` is pasted into its box (``graph_df`` columns bb_left, bb_top,
+        bb_width, bb_height, frame) of the ``seq_info_dict`` frame_height x frame_width image; within a frame every pixel
+        goes to the node with the largest probability, and to its mask where that is > threshold.  id = the node's
+        ``_assign_ped_ids`` label.  Runs after ``_assign_ped_ids``.  Returns (lines written, nodes whose mask is
+        empty and were skipped)."""
+        from ..utils.mots import encode_mots_masks, write_mots_txt
+        mg = self.full_graph
+        go = mg.graph_obj
+        node_preds = getattr(go, 'node_preds', None)
+        if node_preds is None:
+            raise RuntimeError('save_mots_results: the sequence graph has no node_preds (evaluate it with the mask '
+                               'branch: node features x_ext and a model with the mask modules)')
+        labels = getattr(self, 'ped_ids', None)
+        if labels is None:
+            raise RuntimeError('save_mots_results: call _assign_ped_ids first')
+        dev = node_preds.device
+        df = mg.graph_df
+        col = lambda c: np.asarray(df[c].values if hasattr(df[c], 'values') else df[c])
+        left, top = col('bb_left').astype(np.float64), col('bb_top').astype(np.float64)
+        boxes = np.stack((left, top, left + col('bb_width').astype(np.float64), top + col('bb_height').astype(np.float64)), 1)
+        frame = col('frame').astype(np.int64)
+        h, w = int(mg.seq_info_dict['frame_height']), int(mg.seq_info_dict['frame_width'])
+        strings = encode_mots_masks(node_preds.float(), torch.from_numpy(boxes).to(dev), torch.from_numpy(frame).to(dev),
+                                    (h, w), threshold)
+        written = write_mots_txt(path, frame, labels.cpu().numpy(), class_id, h, w, strings)
+        return written, len(strings) - written
