@@ -152,8 +152,12 @@ int mpn_edge_layout_build(const int64_t* edge_index /*[2,E]*/, int64_t num_edges
 
 /* ------------------------------------------------------------------ model: encoders */
 
-/* models/mpn.py:351-352  AdaptiveAvgPool2d((1,1)) + view: x[N,C,HW] -> out[N,C]. */
-int mpn_avgpool(const float* x, int64_t n, int64_t c, int64_t hw, float* out, void* stream);
+/* models/mpn.py:351-352  AdaptiveAvgPool2d((1,1)) + view: x[N,C,HW] -> out[N,C], for `windows` windows at once:
+ * window i reads x[i] [n[i],C,HW] and writes the next n[i] rows of out (out [sum n, C]).  x and n are host arrays.
+ * The windows whose maps are 16-byte aligned (HW/4 a power of two up to 32) are pooled by one launch per 64
+ * windows; the others by one scalar launch each. */
+int mpn_avgpool(const float* const* x, const int64_t* n, int64_t windows, int64_t c, int64_t hw, float* out,
+                void* stream);
 
 /* models/mlp.py:12-23  one Linear(+ReLU) layer: out[M,O] = act(in[M,K] @ W[O,K]^T + b). */
 int mpn_linear(const float* in, int64_t m, int64_t k, const float* w, const float* b,

@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'lib', 'libmpntrack_b200.so')
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 c_i64, c_i32, c_f32, c_vp = C.c_int64, C.c_int32, C.c_float, C.c_void_p
 c_i64p = C.POINTER(C.c_int64)
@@ -53,7 +53,7 @@ SIGNATURES = {
                                       c_vp, c_vp, c_vp, c_vp, c_i64p, c_i64p, c_vp]),
     'mpn_edge_layout_workspace': (c_i64, [c_i64, c_i64]),
     'mpn_edge_layout_build': (C.c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64p, c_vp]),
-    'mpn_avgpool': (C.c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_vp]),
+    'mpn_avgpool': (C.c_int, [C.POINTER(c_vp), c_i64p, c_i64, c_i64, c_i64, c_vp, c_vp]),
     'mpn_linear': (C.c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_i64, C.c_int, c_vp, c_vp]),
     'mpn_node_encoder_tc_workspace': (c_i64, [c_i64]),
     'mpn_node_encoder_tc': (C.c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),

@@ -1,5 +1,7 @@
 // Encoders: global average pool, generic Linear(+ReLU) layer (fp32 SIMT tiled GEMM),
 // row gather, and the fused edge-feature MLP in slot order.
+#include <algorithm>
+
 #include "common.cuh"
 #include "mlp_regs.cuh"
 
@@ -8,33 +10,52 @@ namespace mpn {
 constexpr unsigned kFull = 0xffffffffu;
 
 // ------------------------------------------------------------------ average pool
-// x[n*c][hw] -> out[n*c].  GROUP = hw/4 lanes cooperate on one channel (float4 each).
+// x[n*c][hw] -> out[n*c] for any number of windows in one launch.  GROUP = hw/4 lanes cooperate on one channel
+// (float4 each).  The windows' rows are cut into chunks of POOL_UNROLL * 32 float4 (2 KB: every load of a warp
+// covers 512 contiguous bytes); the chunks of all windows form one list, and each block takes the next
+// POOL_BLOCK_CHUNKS of it.  POOL_UNROLL independent 16-byte loads per thread are issued before any of them is
+// consumed: the kernel is a pure HBM stream and needs the bytes in flight.
+// The blocks are short (128 KB of maps, some 10-20 us at the HBM rate per SM): the pool runs on its own stream
+// beside the window-graph build, whose kernels have the higher stream priority, so a build kernel waits for the pool
+// blocks on an SM to end, never for the whole pool.
+constexpr int POOL_THREADS = 256, POOL_UNROLL = 4, POOL_BLOCK_CHUNKS = 64, POOL_MAX_WINDOWS = 64;
+
+struct PoolWindow {
+  const float4* x;          // the window's maps, 16-byte aligned
+  int64_t rows;             // n * c
+  int64_t out_row;          // first output element of the window
+  int32_t chunk_end;        // one past the window's last chunk in the launch's chunk list
+};
+struct PoolTable {          // passed by value: the table lives in the kernel's parameter space, no copy to the device
+  PoolWindow w[POOL_MAX_WINDOWS];
+  int count;
+};
+
 template <int GROUP>
-__global__ void avgpool_vec_kernel(const float4* __restrict__ x, int64_t rows, float inv_hw_unused,
-                                   int hw, float* __restrict__ out) {
-  constexpr int ROWS_PER_WARP = 32 / GROUP;
+__global__ void __launch_bounds__(POOL_THREADS) avgpool_kernel(const __grid_constant__ PoolTable t, int hw,
+                                                               float* __restrict__ out) {
+  constexpr int ROWS_PER_WARP = 32 / GROUP, CHUNK_ROWS = ROWS_PER_WARP * POOL_UNROLL;
   const int lane = threadIdx.x & 31;
-  const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  // UNROLL independent 16-byte loads per thread are issued before any of them is consumed: the kernel is a pure
-  // HBM stream and needs the bytes in flight (one load per thread left it at 87 % of the measured peak)
-  constexpr int UNROLL = 4;
-  const int64_t stride = nwarps * ROWS_PER_WARP;
-  for (int64_t r0 = warp * ROWS_PER_WARP; r0 < rows; r0 += UNROLL * stride) {
-    float4 v[UNROLL];
+  const int chunks = t.w[t.count - 1].chunk_end;
+  const int end = min(chunks, (int)(blockIdx.x + 1) * POOL_BLOCK_CHUNKS);
+  int w = 0, first = 0;                                 // window of chunk ch and its first chunk
+  for (int ch = blockIdx.x * POOL_BLOCK_CHUNKS + (threadIdx.x >> 5); ch < end; ch += POOL_THREADS / 32) {
+    while (ch >= t.w[w].chunk_end) first = t.w[w++].chunk_end;
+    const int64_t r0 = (int64_t)(ch - first) * CHUNK_ROWS;
+    const int valid = (int)min((int64_t)CHUNK_ROWS, t.w[w].rows - r0);    // rows of this chunk
+    const float4* src = t.w[w].x + r0 * GROUP + lane;
+    float4 v[POOL_UNROLL];
 #pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      const int64_t ru = r0 + u * stride;
-      v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (ru + lane / GROUP < rows) v[u] = __ldcs(x + ru * GROUP + lane);      // streaming: read once
-    }
+    for (int u = 0; u < POOL_UNROLL; ++u)
+      v[u] = valid == CHUNK_ROWS || u * ROWS_PER_WARP + lane / GROUP < valid ? __ldcs(src + u * 32)  // streaming
+                                                                            : make_float4(0.f, 0.f, 0.f, 0.f);
+    float* dst = out + t.w[w].out_row + r0 + lane / GROUP;
 #pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      const int64_t r = r0 + u * stride + lane / GROUP;
+    for (int u = 0; u < POOL_UNROLL; ++u) {
       float s = (v[u].x + v[u].y) + (v[u].z + v[u].w);
 #pragma unroll
       for (int d = GROUP / 2; d > 0; d >>= 1) s += __shfl_xor_sync(kFull, s, d);
-      if (r < rows && (lane % GROUP) == 0) out[r] = s / (float)hw;
+      if ((lane % GROUP) == 0 && u * ROWS_PER_WARP + lane / GROUP < valid) dst[u * ROWS_PER_WARP] = s / (float)hw;
     }
   }
 }
@@ -145,6 +166,14 @@ __global__ void gather_rows_kernel(const float* __restrict__ in, const int32_t* 
   }
 }
 
+template <int GROUP>
+static int launch_avgpool(const PoolTable& t, int64_t hw, float* out, cudaStream_t s) {
+  const unsigned grid = (unsigned)ceil_div(t.w[t.count - 1].chunk_end, POOL_BLOCK_CHUNKS);
+  avgpool_kernel<GROUP><<<grid, POOL_THREADS, 0, s>>>(t, (int)hw, out); count_launch();
+  MPN_LAUNCH_CHECK();
+  return MPN_OK;
+}
+
 static inline unsigned grid_for(int64_t n, int threads, int per_sm = 8) {
   int64_t want = ceil_div(n > 0 ? n : 1, threads);
   int64_t cap = (int64_t)sm_count() * per_sm;
@@ -157,31 +186,52 @@ using namespace mpn;
 
 extern "C" {
 
-int mpn_avgpool(const float* x, int64_t n, int64_t c, int64_t hw, float* out, void* stream) {
-  MPN_CHECK_ARG(n >= 0 && c > 0 && hw > 0, "avgpool: bad sizes");
-  const int64_t rows = n * c;
-  if (rows == 0) return MPN_OK;
-  MPN_CHECK_ARG(x && out, "avgpool: null pointer");
+int mpn_avgpool(const float* const* x, const int64_t* n, int64_t windows, int64_t c, int64_t hw, float* out,
+                void* stream) {
+  MPN_CHECK_ARG(windows >= 0 && c > 0 && hw > 0 && (windows == 0 || (x && n)), "avgpool: bad sizes");
   cudaStream_t s = as_stream(stream);
   const int64_t vec = hw / 4;
-  const bool vec_ok = (hw % 4 == 0) && vec >= 1 && vec <= 32 && (vec & (vec - 1)) == 0 &&
-                      (reinterpret_cast<uintptr_t>(x) % 16 == 0);
-  if (vec_ok) {
-    const unsigned grid = grid_for(rows * vec, 256, 16);
-    const float4* x4 = reinterpret_cast<const float4*>(x);
+  const bool vec_hw = (hw % 4 == 0) && vec >= 1 && vec <= 32 && (vec & (vec - 1)) == 0;
+  const int64_t chunk_rows = POOL_UNROLL * (32 / std::max<int64_t>(vec, 1));
+  PoolTable t;
+  t.count = 0;
+  int64_t out_row = 0;
+  // one launch per POOL_MAX_WINDOWS vector-path windows; a window off 16-byte alignment takes the scalar kernel
+  auto flush = [&]() -> int {
+    if (t.count == 0) return MPN_OK;
+    int rc = MPN_OK;
     switch (vec) {
-      case 1: avgpool_vec_kernel<1><<<grid, 256, 0, s>>>(x4, rows, 0.f, (int)hw, out); count_launch(); break;
-      case 2: avgpool_vec_kernel<2><<<grid, 256, 0, s>>>(x4, rows, 0.f, (int)hw, out); count_launch(); break;
-      case 4: avgpool_vec_kernel<4><<<grid, 256, 0, s>>>(x4, rows, 0.f, (int)hw, out); count_launch(); break;
-      case 8: avgpool_vec_kernel<8><<<grid, 256, 0, s>>>(x4, rows, 0.f, (int)hw, out); count_launch(); break;
-      case 16: avgpool_vec_kernel<16><<<grid, 256, 0, s>>>(x4, rows, 0.f, (int)hw, out); count_launch(); break;
-      default: avgpool_vec_kernel<32><<<grid, 256, 0, s>>>(x4, rows, 0.f, (int)hw, out); count_launch(); break;
+      case 1: rc = launch_avgpool<1>(t, hw, out, s); break;
+      case 2: rc = launch_avgpool<2>(t, hw, out, s); break;
+      case 4: rc = launch_avgpool<4>(t, hw, out, s); break;
+      case 8: rc = launch_avgpool<8>(t, hw, out, s); break;
+      case 16: rc = launch_avgpool<16>(t, hw, out, s); break;
+      default: rc = launch_avgpool<32>(t, hw, out, s); break;
     }
-  } else {
-    avgpool_scalar_kernel<<<grid_for(rows, 256), 256, 0, s>>>(x, rows, (int)hw, out); count_launch();
+    t.count = 0;
+    return rc;
+  };
+  for (int64_t i = 0; i < windows; ++i) {
+    MPN_CHECK_ARG(n[i] >= 0, "avgpool: window %lld has %lld rows", (long long)i, (long long)n[i]);
+    const int64_t rows = n[i] * c;
+    if (rows == 0) continue;
+    MPN_CHECK_ARG(x[i] && out, "avgpool: null pointer");
+    if (vec_hw && reinterpret_cast<uintptr_t>(x[i]) % 16 == 0) {
+      const int64_t prev = t.count ? t.w[t.count - 1].chunk_end : 0;
+      MPN_CHECK_ARG(prev + ceil_div(rows, chunk_rows) < INT32_MAX - POOL_BLOCK_CHUNKS, "avgpool: more than 2^31 chunks in one launch");
+      t.w[t.count++] = PoolWindow{reinterpret_cast<const float4*>(x[i]), rows, out_row,
+                                   (int32_t)(prev + ceil_div(rows, chunk_rows))};
+      if (t.count == POOL_MAX_WINDOWS) {
+        const int rc = flush();
+        if (rc != MPN_OK) return rc;
+      }
+    } else {
+      avgpool_scalar_kernel<<<grid_for(rows, 256), 256, 0, s>>>(x[i], rows, (int)hw, out + out_row); count_launch();
+      MPN_LAUNCH_CHECK();
+    }
+    out_row += rows;
   }
-  MPN_LAUNCH_CHECK();
-  return MPN_OK;
+  return flush();
 }
 
 int mpn_linear(const float* in, int64_t m, int64_t k, const float* w, const float* b, int64_t o,

@@ -221,6 +221,14 @@ class GraphBatch(object):
     def __init__(self, xs, node_ptr, edge_index, edge_attr, pair_ptr, reid_emb_dists=None):
         self.xs, self.node_ptr, self.pair_ptr = xs, list(node_ptr), list(pair_ptr)
         self.edge_index, self.edge_attr, self.reid_emb_dists = edge_index, edge_attr, reid_emb_dists
+        self._pool = None           # (xs it was pooled from, [N, C] pooled buffer, event of the side stream)
+
+    def pooled_xs(self):
+        """(pooled [N, C] buffer, event that marks it ready) of the node-feature pool ``build_graph_batch`` started on a
+        side stream, or None when there is none or ``xs`` has been replaced since.  Wait on the event before reading."""
+        if self._pool is None or self._pool[0] is not self.xs:
+            return None
+        return self._pool[1], self._pool[2]
 
     @property
     def num_graphs(self):
@@ -265,8 +273,33 @@ def build_graph_batch(table, node_ptr, dataset_params, fps, inference_mode=False
     """Same as ``build_window_graphs`` for a detection table that is already ONE set of columns (the way
     the reference holds a sequence's ``graph_df``): ``table`` maps ``frame, bb_height, bb_width, feet_x,
     feet_y`` to [N_total] tensors, ``reid`` to [N_total,256] and ``x`` to the node features (one tensor
-    or a list with one tensor per window); window g owns rows ``node_ptr[g]:node_ptr[g+1]``."""
+    or a list with one tensor per window); window g owns rows ``node_ptr[g]:node_ptr[g+1]``.
+
+    When ``x`` holds CUDA fp32 feature maps ([n, C, H, W], the same C, H, W for every window), their average pool
+    is enqueued first, on a side stream, and the graph build runs on a stream of higher priority, so that the pool
+    fills the GPU around the build's kernels and host synchronisations; ``MOTMPNet.forward_batch`` waits for the
+    pool before the node encoder.  ``table['x']`` is therefore read at once: it
+    must be ready on the current stream when this is called, as any argument of a kernel on that stream."""
     dev = device or torch.device('cuda')
+    pool = _start_pool(table['x'])
+    if pool is None:
+        return _build(table, node_ptr, dataset_params, fps, inference_mode, max_frame_dist, dev, engine)
+    # the build runs on a stream of higher priority than the pool's: the pool is cut into short blocks, so a build
+    # kernel gets its SMs as soon as the pool blocks on them end, and the pool fills the GPU while the host waits
+    cur = torch.cuda.current_stream()
+    build = _stream('build', priority=-1)
+    build.wait_stream(cur)
+    with torch.cuda.stream(build):
+        batch = _build(table, node_ptr, dataset_params, fps, inference_mode, max_frame_dist, dev, engine)
+    cur.wait_stream(build)
+    for t in (batch.edge_index, batch.edge_attr, batch.reid_emb_dists):
+        if t is not None:
+            t.record_stream(cur)
+    batch._pool = (table['x'],) + pool
+    return batch
+
+
+def _build(table, node_ptr, dataset_params, fps, inference_mode, max_frame_dist, dev, engine):
     col = lambda name, dt: table[name].to(dev, dt).view(-1)
     frame = col('frame', torch.int64)
     reid = table['reid'].to(dev, torch.float32)
@@ -285,3 +318,36 @@ def build_graph_batch(table, node_ptr, dataset_params, fps, inference_mode=False
         attr = attr[:, wanted].contiguous()
     return GraphBatch(table['x'], node_ptr, edge_index, attr, pair_ptr,
                       torch.cat((dist, dist)) if inference_mode else None)
+
+
+_STREAMS = {}
+
+
+def _stream(name, priority=0):
+    """One cached stream per (purpose, device) of the current device."""
+    key = (name, torch.cuda.current_device())
+    if key not in _STREAMS:
+        _STREAMS[key] = torch.cuda.Stream(priority=priority)
+    return _STREAMS[key]
+
+
+def _start_pool(x):
+    """Enqueue the pool of the node-feature maps ``x`` (a tensor or a list of per-window tensors) on a side stream of
+    the current device: (pooled [N, C] buffer, event recorded after it), or None for inputs that are not CUDA fp32
+    maps of one shape per node (pooled features, CPU tensors, no windows), which the node encoder pools itself."""
+    xs = list(x) if isinstance(x, (list, tuple)) else [x]
+    if not xs or not all(torch.is_tensor(t) and t.is_cuda and t.dtype == torch.float32 and t.dim() >= 3 and
+                         t.shape[1:] == xs[0].shape[1:] and t.device.index == torch.cuda.current_device() for t in xs):
+        return None
+    cur = torch.cuda.current_stream()
+    side = _stream('pool')
+    pooled = torch.empty((sum(t.shape[0] for t in xs), xs[0].shape[1]), dtype=torch.float32, device=cur.device)
+    side.wait_stream(cur)                       # the maps are ready on the current stream, and the buffer is allocated
+    for t in xs:                                # neither is reused before the side stream is done with it, even if the
+        t.record_stream(side)                   # caller drops its maps right after build_graph_batch
+    pooled.record_stream(side)
+    with torch.cuda.stream(side):
+        ops.avgpool_windows(xs, out=pooled)
+        done = torch.cuda.Event()
+        done.record(side)
+    return pooled, done

@@ -376,6 +376,7 @@ class MOTMPNet(nn.Module):
             xs = list(batch.xs) if isinstance(batch.xs, (list, tuple)) else [batch.xs]
             edge_index, edge_attr, n = batch.edge_index, batch.edge_attr, batch.num_nodes
             spans = None
+            pooled = None if encoded else batch.pooled_xs()
         else:
             xs, eis, eas, spans, off, eo = [], [], [], [], 0, 0
             for g in graphs:
@@ -385,10 +386,10 @@ class MOTMPNet(nn.Module):
                 spans.append((eo, eo + g.edge_index.shape[1]))
                 off += g.x.shape[0]
                 eo += g.edge_index.shape[1]
-            edge_index, edge_attr, n, batch = torch.cat(eis, dim=1), torch.cat(eas), off, None
+            edge_index, edge_attr, n, batch, pooled = torch.cat(eis, dim=1), torch.cat(eas), off, None, None
         layout = ops.edge_layout(edge_index, n)
         first_class_step = self.num_enc_steps - self.num_class_steps + 1
-        logits = self._core(xs, edge_attr, layout, first_class_step, encoded=encoded)[0]
+        logits = self._core(xs, edge_attr, layout, first_class_step, encoded=encoded, pooled=pooled)[0]
         return BatchOutput(logits, batch, spans)
 
     def forward(self, data, return_state=False):
@@ -452,18 +453,23 @@ class MOTMPNet(nn.Module):
         c = tr.last_ctx
         return self._mask_branch(x_ext, c['lay'], logits, first_class_step, train_ctx=c)
 
-    def _core(self, xs, edge_attr, layout, first_needed, want_state=False, encoded=False):
+    def _core(self, xs, edge_attr, layout, first_needed, want_state=False, encoded=False, pooled=None):
         """Encoders + step loop.  The tensor-core kernels report fp16-range overflow through one status
-        word that is read once at the end (a single host sync); 'auto' then reruns on the fp32 kernels."""
+        word that is read once at the end (a single host sync); 'auto' then reruns on the fp32 kernels.
+        pooled: (the pooled [N, C] node features of ``xs``, event that marks them ready) when the pool already runs
+        on another stream; the edge encoder, which does not need them, is enqueued before the wait."""
         engine = self.engine or ops.default_engine()
         cw, keep = self.core_weights()
         for eng in ((engine,) if engine != 'auto' else ('auto', 'fp32')):
             status = torch.zeros(2, dtype=torch.int32, device=edge_attr.device) if eng != 'fp32' else None
+            e0 = self.encode_edges(edge_attr, layout)
             if encoded:
                 x0 = xs[0] if len(xs) == 1 else torch.cat(xs)
+            elif pooled is not None:
+                torch.cuda.current_stream().wait_event(pooled[1])
+                x0 = self.encode_pooled(pooled[0], engine=eng, status=None if status is None else status[0:1])
             else:
                 x0 = self.encode_nodes_list(xs, engine=eng, status=None if status is None else status[0:1])
-            e0 = self.encode_edges(edge_attr, layout)
             res = ops.mp_forward(cw, layout, x0, e0, self.num_enc_steps, first_needed, want_state=want_state,
                                  engine=eng, status=None if status is None else status[1:2])
             res = res if want_state else (res,)

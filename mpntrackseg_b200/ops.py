@@ -214,11 +214,32 @@ def avgpool(x, out=None):
             return x.reshape(n, c)
         out.copy_(x.reshape(n, c))
         return out
+    return avgpool_windows([x], out)
+
+
+def avgpool_windows(xs, out=None):
+    """Every window's maps [N_i, C, H, W] -> one [sum N_i, C] buffer, window i in rows sum(N_<i):sum(N_<=i), in one
+    launch (per 64 windows).  Each row is what ``avgpool`` gives for it, bit for bit."""
+    xs = [_req(x, torch.float32, 'x') for x in xs]
+    if not xs:
+        raise ValueError('avgpool_windows: no windows')
+    c, spatial = xs[0].shape[1], xs[0].shape[2:]
+    if any(x.dim() < 3 or x.shape[1] != c or x.shape[2:] != spatial for x in xs):
+        raise ValueError('avgpool_windows: every window must be [N_i, C, H, W] with the same C, H, W')
+    hw = 1
+    for s in spatial:
+        hw *= s
+    n_tot = sum(x.shape[0] for x in xs)
     if out is None:
-        out = torch.empty((n, c), dtype=torch.float32, device=x.device)
-    elif not (out.is_contiguous() and tuple(out.shape) == (n, c) and out.dtype == torch.float32):
+        out = torch.empty((n_tot, c), dtype=torch.float32, device=xs[0].device)
+    elif not (out.is_contiguous() and tuple(out.shape) == (n_tot, c) and out.dtype == torch.float32):
         raise ValueError('avgpool: out must be a contiguous fp32 [N, C] tensor')
-    check(lib().mpn_avgpool(ptr(x), n, c, hw, ptr(out), stream_ptr()), 'avgpool')
+    if hw == 1:
+        torch.cat([x.reshape(x.shape[0], c) for x in xs], out=out)
+        return out
+    g = len(xs)
+    check(lib().mpn_avgpool((C.c_void_p * g)(*[x.data_ptr() for x in xs]), (C.c_int64 * g)(*[x.shape[0] for x in xs]),
+                            g, c, hw, ptr(out), stream_ptr()), 'avgpool')
     return out
 
 
