@@ -219,15 +219,6 @@ typedef struct {
  * flow sums, tile partials). */
 int64_t mpn_mp_workspace(int64_t num_nodes, int64_t num_edges);
 
-/* models/mpn.py:33-54 MetaLayer.forward as ONE step on explicit latent states:
- *   mode 3: edge update then node update; mode 1: EdgeModel.forward only (:67-69, writes
- *   e_out); mode 2: TimeAwareNodeModel.forward only (:83-99, e_lat is taken as the already
- *   updated edge features, writes x_out).  logits (original edge order, may be NULL) gets
- *   classifier(e') (:114).  All edge tensors are in slot order. e_out may alias e_lat. */
-int mpn_mp_step(const mpn_core_weights* h_w, const mpn_edge_layout* h_g, const float* x_init,
-                const float* x_lat, const float* e_init, const float* e_lat, int32_t mode,
-                void* workspace, float* e_out, float* x_out, float* logits, void* stream);
-
 /* models/mpn.py:364-381  the step loop: num_steps x { reattach, MetaLayer.forward
  * (EdgeModel :67-69, TimeAwareNodeModel :83-99), classifier :114 }.
  *   x_init [N,dn], e_init [E,de] (slot order)   -- encoder outputs (models/mpn.py:355-360)

@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'lib', 'libmpntrack_b200.so')
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 c_i64, c_i32, c_f32, c_vp = C.c_int64, C.c_int32, C.c_float, C.c_void_p
 c_i64p = C.POINTER(C.c_int64)
@@ -61,8 +61,6 @@ SIGNATURES = {
     'mpn_edge_encoder': (C.c_int, [c_vp, c_vp, c_i64, C.POINTER(c_i32), c_i32, C.POINTER(c_vp),
                                    C.POINTER(c_vp), c_vp, c_vp]),
     'mpn_mp_workspace': (c_i64, [c_i64, c_i64]),
-    'mpn_mp_step': (C.c_int, [C.POINTER(CoreWeights), C.POINTER(EdgeLayout), c_vp, c_vp, c_vp, c_vp, c_i32,
-                              c_vp, c_vp, c_vp, c_vp, c_vp]),
     'mpn_mp_forward': (C.c_int, [C.POINTER(CoreWeights), C.POINTER(EdgeLayout), c_vp, c_vp, c_i32, c_i32,
                                  c_vp, c_vp, c_vp, c_vp, c_vp]),
     'mpn_gemm': (C.c_int, [c_vp, c_i64, C.c_int, c_vp, c_i64, c_vp, c_i64, C.c_int, c_vp, C.c_int, C.c_int, c_vp, c_i64,

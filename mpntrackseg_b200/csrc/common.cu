@@ -152,7 +152,7 @@ extern "C" {
 
 const char* mpn_last_error(void) { return mpn::g_err; }
 
-int mpn_abi_version(void) { return 3; }
+int mpn_abi_version(void) { return 4; }
 
 long long mpn_launch_count(void) { return mpn::g_launches.load(); }
 

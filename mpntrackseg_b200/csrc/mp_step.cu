@@ -55,17 +55,16 @@ struct StepArgs {
   float* flow;                                  // [N, 2*DN]  (flow_in | flow_out)
   float* part;                                  // [tiles, 2, DN]
   float* logits;                                // row of the logits output for this step or NULL
-  int do_edge;                                  // 0: e' := e_cur (node update only)
-  int do_node;                                  // 0: skip flow messages / aggregation
   int agg;                                      // 0 sum, 1 mean (sums here, divided in the node kernel), 2 max
 };
 
-template <int N4>
+// RO: read through the read-only path (__ldg).  Such loads of one address may be merged by the compiler.
+template <int N4, bool RO = true>
 __device__ __forceinline__ void load_vec(float (&dst)[N4 * 4], const float* __restrict__ src) {
   const float4* p = reinterpret_cast<const float4*>(src);
 #pragma unroll
   for (int q = 0; q < N4; ++q) {
-    const float4 v = __ldg(p + q);
+    const float4 v = RO ? __ldg(p + q) : p[q];
     dst[4 * q] = v.x; dst[4 * q + 1] = v.y; dst[4 * q + 2] = v.z; dst[4 * q + 3] = v.w;
   }
 }
@@ -121,31 +120,27 @@ __global__ void __launch_bounds__(TS) mp_edge_kernel(StepArgs a, mpn_core_weight
 #pragma unroll
     for (int i = 0; i < DN; ++i) msg[i] = 0.f;
     if (valid) {
+      // ---- edge MLP layer 0: stream the 6 input blocks through the accumulators
+      float h[EH];
+      load_bias<EH>(h, smem + W::OFF_EB0);
+      float v[DN];
+      const float* wt = smem + W::OFF_EW0;
+      load_vec<DN / 4>(v, a.x_init + (int64_t)r * DN); dense_acc<DN, EH>(h, v, wt, 0);
+      load_vec<DN / 4>(v, a.x_lat + (int64_t)r * DN);  dense_acc<DN, EH>(h, v, wt, DN);
+      load_vec<DN / 4>(v, a.x_init + (int64_t)c * DN); dense_acc<DN, EH>(h, v, wt, 2 * DN);
+      load_vec<DN / 4>(v, a.x_lat + (int64_t)c * DN);  dense_acc<DN, EH>(h, v, wt, 3 * DN);
+      float ev[DE];
+      load_vec<DE / 4>(ev, a.e_init + slot * DE);      dense_acc<DE, EH>(h, ev, wt, 4 * DN);
+      load_vec<DE / 4>(ev, a.e_cur + slot * DE);       dense_acc<DE, EH>(h, ev, wt, 4 * DN + DE);
+      relu_inplace(h);
+      // ---- edge MLP layer 1
       float e2[DE];
-      if (!a.do_edge) {
-        load_vec<DE / 4>(e2, a.e_cur + slot * DE);
-      } else {
-        // ---- edge MLP layer 0: stream the 6 input blocks through the accumulators
-        float h[EH];
-        load_bias<EH>(h, smem + W::OFF_EB0);
-        float v[DN];
-        const float* wt = smem + W::OFF_EW0;
-        load_vec<DN / 4>(v, a.x_init + (int64_t)r * DN); dense_acc<DN, EH>(h, v, wt, 0);
-        load_vec<DN / 4>(v, a.x_lat + (int64_t)r * DN);  dense_acc<DN, EH>(h, v, wt, DN);
-        load_vec<DN / 4>(v, a.x_init + (int64_t)c * DN); dense_acc<DN, EH>(h, v, wt, 2 * DN);
-        load_vec<DN / 4>(v, a.x_lat + (int64_t)c * DN);  dense_acc<DN, EH>(h, v, wt, 3 * DN);
-        float ev[DE];
-        load_vec<DE / 4>(ev, a.e_init + slot * DE);      dense_acc<DE, EH>(h, ev, wt, 4 * DN);
-        load_vec<DE / 4>(ev, a.e_cur + slot * DE);       dense_acc<DE, EH>(h, ev, wt, 4 * DN + DE);
-        relu_inplace(h);
-        // ---- edge MLP layer 1
-        load_bias<DE>(e2, smem + W::OFF_EB1);
-        dense_acc<EH, DE>(e2, h, smem + W::OFF_EW1);
-        relu_inplace(e2);
-        float4* dst = reinterpret_cast<float4*>(a.e_next + slot * DE);
+      load_bias<DE>(e2, smem + W::OFF_EB1);
+      dense_acc<EH, DE>(e2, h, smem + W::OFF_EW1);
+      relu_inplace(e2);
+      float4* dst = reinterpret_cast<float4*>(a.e_next + slot * DE);
 #pragma unroll
-        for (int q = 0; q < DE / 4; ++q) dst[q] = make_float4(e2[4 * q], e2[4 * q + 1], e2[4 * q + 2], e2[4 * q + 3]);
-      }
+      for (int q = 0; q < DE / 4; ++q) dst[q] = make_float4(e2[4 * q], e2[4 * q + 1], e2[4 * q + 2], e2[4 * q + 3]);
       // ---- classifier
       if (a.logits != nullptr) {
         float ch[CH];
@@ -157,22 +152,19 @@ __global__ void __launch_bounds__(TS) mp_edge_kernel(StepArgs a, mpn_core_weight
         for (int i = 0; i < CH; ++i) lg = fmaf(ch[i], smem[W::OFF_CW1 + i], lg);
         a.logits[a.slot_edge[slot]] = lg;
       }
-      // ---- flow MLP of this tile's direction on [x_init[c] | x_lat[c] | e']
-      if (a.do_node) {
-        float g[FH];
-        load_bias<FH>(g, smem + W::OFF_FB0);
-        float v[DN];
-        const float* wt = smem + W::OFF_FW0;
-        load_vec<DN / 4>(v, a.x_init + (int64_t)c * DN); dense_acc<DN, FH>(g, v, wt, 0);
-        load_vec<DN / 4>(v, a.x_lat + (int64_t)c * DN);  dense_acc<DN, FH>(g, v, wt, DN);
-        dense_acc<DE, FH>(g, e2, wt, 2 * DN);
-        relu_inplace(g);
-        load_bias<DN>(msg, smem + W::OFF_FB1);
-        dense_acc<FH, DN>(msg, g, smem + W::OFF_FW1);
-        relu_inplace(msg);
-      }
+      // ---- flow MLP of this tile's direction on [x_init[c] | x_lat[c] | e']; x[c] is read again with plain loads:
+      //      merged with the edge MLP's reads, it would stay live across layer 1 and the classifier (+58 registers)
+      float g[FH];
+      load_bias<FH>(g, smem + W::OFF_FB0);
+      const float* wf = smem + W::OFF_FW0;
+      load_vec<DN / 4, false>(v, a.x_init + (int64_t)c * DN); dense_acc<DN, FH>(g, v, wf, 0);
+      load_vec<DN / 4, false>(v, a.x_lat + (int64_t)c * DN);  dense_acc<DN, FH>(g, v, wf, DN);
+      dense_acc<DE, FH>(g, e2, wf, 2 * DN);
+      relu_inplace(g);
+      load_bias<DN>(msg, smem + W::OFF_FB1);
+      dense_acc<FH, DN>(msg, g, smem + W::OFF_FW1);
+      relu_inplace(msg);
     }
-    if (!a.do_node) continue;                               // uniform across the CTA
 #pragma unroll
     for (int i = 0; i < DN; ++i) s_msg[tid * W::MSG_LD + i] = msg[i];
     __syncthreads();
@@ -339,8 +331,7 @@ static int check_core(const mpn_core_weights* w, const mpn_edge_layout* g, const
 // One launch pair. e_next may alias e_cur. logits_row: this step's row of the output or NULL.
 static int launch_step(const mpn_core_weights* w, const mpn_edge_layout* g, const MpWorkspace& m,
                        const float* x_init, const float* x_cur, const float* e_init, const float* e_cur,
-                       float* e_next, float* x_next, float* logits_row, int do_edge, int do_node,
-                       cudaStream_t s) {
+                       float* e_next, float* x_next, float* logits_row, cudaStream_t s) {
   using W = Shipped;
   const int64_t n = g->num_nodes, e = g->num_edges;
   MPN_CUDA(cudaFuncSetAttribute(mp_edge_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -356,12 +347,12 @@ static int launch_step(const mpn_core_weights* w, const mpn_edge_layout* g, cons
     a.slot_row = g->slot_row; a.slot_col = g->slot_col; a.slot_edge = g->slot_edge;
     a.num_edges = e; a.num_out = g->num_out; a.tiles_out = tiles_out; a.tiles_in = tiles_in;
     a.x_init = x_init; a.x_lat = x_cur; a.e_init = e_init; a.e_cur = e_cur; a.e_next = e_next;
-    a.flow = m.flow; a.part = m.part; a.logits = logits_row; a.do_edge = do_edge; a.do_node = do_node; a.agg = w->node_agg;
+    a.flow = m.flow; a.part = m.part; a.logits = logits_row; a.agg = w->node_agg;
     if (profiling()) profile_mark(0, true, s);
     mp_edge_kernel<W><<<grid, TS, W::SMEM_BYTES, s>>>(a, *w); count_launch();
     if (profiling()) profile_mark(0, false, s);
   }
-  if (n > 0 && do_node) {
+  if (n > 0) {
     const unsigned ngrid = (unsigned)std::min<int64_t>(ceil_div(n * 32, 256), (int64_t)sm_count() * 8);
     if (profiling()) profile_mark(1, true, s);
     mp_node_kernel<W><<<ngrid, 256, 0, s>>>(g->out_ptr, g->in_ptr, n, g->num_out, tiles_out, m.flow,
@@ -375,22 +366,6 @@ static int launch_step(const mpn_core_weights* w, const mpn_edge_layout* g, cons
 }  // namespace mpn
 
 extern "C" {
-
-int mpn_mp_step(const mpn_core_weights* w, const mpn_edge_layout* g, const float* x_init,
-                const float* x_lat, const float* e_init, const float* e_lat, int32_t mode, void* ws,
-                float* e_out, float* x_out, float* logits, void* stream) {
-  int rc = check_core(w, g, "mp_step");
-  if (rc) return rc;
-  MPN_CHECK_ARG(mode >= 1 && mode <= 3, "mp_step: mode must be 1 (edge), 2 (node) or 3 (both)");
-  MPN_CHECK_ARG(ws != nullptr, "mp_step: null workspace");
-  const int do_edge = mode & 1, do_node = (mode >> 1) & 1;
-  MPN_CHECK_ARG(!do_edge || e_out || g->num_edges == 0, "mp_step: e_out is required when the edge update runs");
-  MPN_CHECK_ARG(!do_node || x_out || g->num_nodes == 0, "mp_step: x_out is required when the node update runs");
-  MpWorkspace m;
-  carve_workspace(ws, g->num_nodes > 0 ? g->num_nodes : 1, g->num_edges > 0 ? g->num_edges : 1, 32, 16, &m);
-  return launch_step(w, g, m, x_init, x_lat, e_init, e_lat, e_out, x_out, logits, do_edge, do_node,
-                     as_stream(stream));
-}
 
 int mpn_mp_forward(const mpn_core_weights* w, const mpn_edge_layout* g, const float* x_init,
                    const float* e_init, int32_t num_steps, int32_t first_class_step, void* ws,
@@ -423,7 +398,7 @@ int mpn_mp_forward(const mpn_core_weights* w, const mpn_edge_layout* g, const fl
     float* x_next = (step == num_steps && x_out) ? x_out : m.x_lat[step & 1];
     float* e_next = (step == num_steps && e_out) ? e_out : m.e_state;
     float* row = (logits && step >= first_class_step) ? logits + (int64_t)(step - first_class_step) * e : nullptr;
-    rc = launch_step(w, g, m, x_init, x_cur, e_init, e_cur, e_next, x_next, row, 1, 1, s);
+    rc = launch_step(w, g, m, x_init, x_cur, e_init, e_cur, e_next, x_next, row, s);
     if (rc) return rc;
     x_cur = x_next;
     e_cur = e_next;

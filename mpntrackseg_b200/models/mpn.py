@@ -29,32 +29,6 @@ def _core_weight_tensors(edge_mlp, flow_in, flow_out, node_lin, cls_mlp):
             'cls_w0': c0w, 'cls_b0': c0b, 'cls_w1': c1w, 'cls_b1': c1b}
 
 
-class _NullClassifier(nn.Module):
-    """Zero classifier used when MetaLayer is called standalone (no logits wanted)."""
-
-    def __init__(self, de, device):
-        super().__init__()
-        self.l0 = nn.Linear(de, 8).to(device)
-        self.l1 = nn.Linear(8, 1).to(device)
-
-    def linears(self):
-        return [self.l0, self.l1]
-
-    def effective_linears(self):
-        return [(self.l0.weight, self.l0.bias), (self.l1.weight, self.l1.bias)]
-
-
-def _zeros_like_core(dn, de, edge_h, flow_h, device):
-    """Placeholder tensors for the parts of ``mpn_core_weights`` a single sub-model does not own (the C
-    struct is one block; mpn_mp_step's mode selects which weights are read)."""
-    z = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=device)
-    return {'edge_w0': z(edge_h, 4 * dn + 2 * de), 'edge_b0': z(edge_h), 'edge_w1': z(de, edge_h), 'edge_b1': z(de),
-            'fin_w0': z(flow_h, 2 * dn + de), 'fin_b0': z(flow_h), 'fin_w1': z(dn, flow_h), 'fin_b1': z(dn),
-            'fout_w0': z(flow_h, 2 * dn + de), 'fout_b0': z(flow_h), 'fout_w1': z(dn, flow_h), 'fout_b1': z(dn),
-            'node_w': z(dn, 2 * dn), 'node_b': z(dn),
-            'cls_w0': z(8, de), 'cls_b0': z(8), 'cls_w1': z(1, 8), 'cls_b1': z(1)}
-
-
 def _agg_name(node_agg_fn):
     """'sum' | 'mean' | 'max' from the model's ``node_agg_fn`` (the reference stores a lambda around the torch_scatter
     function; here the config string is kept and the kernels switch on it).  reference: models/mpn.py:263-273"""
@@ -65,49 +39,46 @@ def _agg_name(node_agg_fn):
     raise NotImplementedError('node_agg_fn must be one of the strings the reference accepts (sum / mean / max)')
 
 
-def _split_reattached(x, edge_attr, dn, de):
-    if x.shape[1] != 2 * dn or edge_attr.shape[1] not in (de, 2 * de):
-        raise NotImplementedError('the fused step is built for reattach_initial_nodes/edges = True '
-                                  f'(x [N,{2 * dn}], edge_attr [E,{2 * de}])')
-    return x[:, :dn].contiguous(), x[:, dn:].contiguous()
+def _layout(edge_index, x, edge_attr):
+    """Slot layout of ``edge_index`` over the rows of ``x``; its build rejects self-loops and node ids outside [0, N)
+    (ValueError) before anything gathers by them."""
+    layout = ops.edge_layout(edge_index, x.shape[0])
+    if edge_attr.shape[0] != layout.num_edges:
+        raise ValueError(f'edge_attr has {edge_attr.shape[0]} rows for {layout.num_edges} edges')
+    return layout
 
 
 class EdgeModel(nn.Module):
     """Edge update e' = MLP(cat[x[row], x[col], e]).  reference: models/mpn.py:59-69
-    ``forward(node_feats [N,64], edge_index [2,E], edge_attr [E,32]) -> [E,16]`` in the caller's edge order;
-    runs the fused edge kernel in its edge-only mode (mpn_mp_step mode 1)."""
+    ``forward(node_feats [N,64], edge_index [2,E], edge_attr [E,32]) -> [E,16]`` in the caller's edge order."""
 
     def __init__(self, edge_model):
         super().__init__()
         self.edge_model = edge_model
 
     def forward(self, node_feats, edge_index, edge_attr):
-        (e0w, e0b), (e1w, e1b) = self.edge_model.effective_linears()
-        de, edge_h = e1w.shape[0], e0w.shape[0]
-        dn = (e0w.shape[1] - 2 * de) // 4
-        named = _zeros_like_core(dn, de, edge_h, 56, e0w.device)
-        named.update(edge_w0=e0w, edge_b0=e0b, edge_w1=e1w, edge_b1=e1b)
-        cw, keep = ops.core_weights(named)
-        xi, xl = _split_reattached(node_feats, edge_attr, dn, de)
-        if edge_attr.shape[1] != 2 * de:
-            raise NotImplementedError(f'EdgeModel expects edge_attr [E,{2 * de}] (reattach_initial_edges = True)')
-        layout = ops.edge_layout(edge_index, node_feats.shape[0])
-        e = layout.num_edges
-        if e == 0:
-            return edge_attr.new_zeros((0, de))
-        ea = ops.gather_rows(edge_attr, layout.slot_edge[:e])
-        e_new, _, _ = ops.mp_step(cw, layout, xi, xl, ea[:, :de].contiguous(), ea[:, de:].contiguous(), mode=1)
+        lins = self.edge_model.linears()
+        de = lins[-1].out_features
+        dn = (lins[0].in_features - 2 * de) // 4
+        if node_feats.shape[1] != 2 * dn or edge_attr.shape[1] != 2 * de:
+            raise NotImplementedError('the edge model is built for reattach_initial_nodes/edges = True '
+                                      f'(x [N,{2 * dn}], edge_attr [E,{2 * de}])')
+        layout = _layout(edge_index, node_feats, edge_attr)
+        e, slot_edge = layout.num_edges, layout.slot_edge[:layout.num_edges]
+        h = torch.cat((ops.gather_rows(node_feats, layout.slot_row[:e]), ops.gather_rows(node_feats, layout.slot_col[:e]),
+                       ops.gather_rows(edge_attr, slot_edge)), dim=1)
+        e_new = self.edge_model(h)
         out = torch.empty_like(e_new)
-        out[layout.slot_edge[:e].long()] = e_new
-        del keep
+        out[slot_edge.long()] = e_new                            # back to the caller's edge order
         return out
 
 
 class TimeAwareNodeModel(nn.Module):
     """Time-aware node update.  reference: models/mpn.py:71-99
     ``forward(x [N,64], edge_index [2,E], edge_attr [E,16]) -> [N,32]`` where ``edge_attr`` holds the already
-    updated edge features (models/mpn.py:52); runs the fused kernels in their node-only mode (mpn_mp_step mode 2).
-    ``node_agg_fn`` is the reference's name for the aggregation ('sum' | 'mean' | 'max' or its lambda)."""
+    updated edge features (models/mpn.py:52).  ``node_agg_fn`` is the reference's name for the aggregation
+    ('sum' | 'mean' | 'max' or its lambda).  The messages of the flow_out group (row < col) and of the flow_in group are
+    computed in slot order, where each node's edges of one group are contiguous, and reduced per node in that order."""
 
     def __init__(self, flow_in_model, flow_out_model, node_model, node_agg_fn):
         super().__init__()
@@ -117,66 +88,51 @@ class TimeAwareNodeModel(nn.Module):
         self.node_agg_fn = node_agg_fn
 
     def forward(self, x, edge_index, edge_attr):
-        (i0w, i0b), (i1w, i1b) = self.flow_in_model.effective_linears()
-        de = edge_attr.shape[1]
-        dn, flow_h = i1w.shape[0], i0w.shape[0]
-        if i0w.shape[1] != 2 * dn + de:
-            raise NotImplementedError(f'TimeAwareNodeModel expects x [N,{2 * dn}] and edge_attr [E,{i0w.shape[1] - 2 * dn}]')
-        (o0w, o0b), (o1w, o1b) = self.flow_out_model.effective_linears()
-        named = _zeros_like_core(dn, de, 80, flow_h, i0w.device)
-        named.update(fin_w0=i0w, fin_b0=i0b, fin_w1=i1w, fin_b1=i1b, fout_w0=o0w, fout_b0=o0b, fout_w1=o1w, fout_b1=o1b,
-                     node_w=self.node_model[0].weight, node_b=self.node_model[0].bias)
-        cw, keep = ops.core_weights(named, node_agg=_agg_name(self.node_agg_fn))
+        lins = self.flow_in_model.linears()
+        lin0, dn = lins[0], lins[-1].out_features
+        if lin0.in_features != 2 * dn + edge_attr.shape[1]:
+            raise NotImplementedError(f'TimeAwareNodeModel expects x [N,{2 * dn}] and '
+                                      f'edge_attr [E,{lin0.in_features - 2 * dn}]')
         if x.shape[1] != 2 * dn:
             raise NotImplementedError(f'TimeAwareNodeModel expects x [N,{2 * dn}] (reattach_initial_nodes = True)')
-        layout = ops.edge_layout(edge_index, x.shape[0])
-        e = layout.num_edges
-        ea = ops.gather_rows(edge_attr, layout.slot_edge[:e]) if e else edge_attr
-        _, x_new, _ = ops.mp_step(cw, layout, x[:, :dn].contiguous(), x[:, dn:].contiguous(), ea, ea, mode=2)
-        del keep
-        return x_new
+        agg = _agg_name(self.node_agg_fn)
+        if agg not in ops.NODE_AGG:
+            raise ValueError(f"node_agg_fn can only be 'max', 'mean' or 'sum', got {agg!r}")
+        layout = _layout(edge_index, x, edge_attr)
+        e, n_out = layout.num_edges, layout.num_out
+        h = torch.cat((ops.gather_rows(x, layout.slot_col[:e]), ops.gather_rows(edge_attr, layout.slot_edge[:e])), dim=1)
+        msg = torch.cat((self.flow_out_model(h[:n_out]), self.flow_in_model(h[n_out:])))
+        flow = torch.empty((x.shape[0], 2 * dn), dtype=torch.float32, device=x.device)
+        ops.segment_sum(msg, 0, dn, layout.in_ptr, None, flow, 0, mode=agg)      # cat(flow_in, flow_out), models/mpn.py:97
+        ops.segment_sum(msg, 0, dn, layout.out_ptr, None, flow, dn, mode=agg)
+        lin = self.node_model[0]
+        return ops.linear(flow, lin.weight, lin.bias, relu=True)
 
 
 class MetaLayer(nn.Module):
-    """One message-passing step ``forward(x, edge_index, edge_attr) -> (x', edge_attr')`` with
-    x = [x_init | x_latent], edge_attr = [e_init | e_latent] in the caller's edge order.
-    reference: models/mpn.py:11-57"""
+    """One message-passing step ``forward(x, edge_index, edge_attr) -> (x', edge_attr')``: the edge model, then the
+    node model on the updated edge features, x = [x_init | x_latent], edge_attr = [e_init | e_latent] in the caller's
+    edge order.  reference: models/mpn.py:11-57"""
 
     def __init__(self, edge_model=None, node_model=None):
         super().__init__()
         self.edge_model = edge_model
         self.node_model = node_model
-        self._null_cls = None
 
-    def _weights(self, classifier=None):
+    def _weights(self, classifier):
         em, nm = self.edge_model, self.node_model
         if em is None or nm is None:
             raise NotImplementedError('the fused step needs both an EdgeModel and a TimeAwareNodeModel')
-        if classifier is None:
-            if self._null_cls is None:
-                dev = em.edge_model.linears()[0].weight.device
-                self._null_cls = [_NullClassifier(em.edge_model.linears()[-1].out_features, dev)]
-                self._null_cls[0].eval()
-            classifier = self._null_cls[0]
         named = _core_weight_tensors(em.edge_model, nm.flow_in_model, nm.flow_out_model,
                                      nm.node_model[0], classifier)
         return ops.core_weights(named, node_agg=_agg_name(nm.node_agg_fn))
 
     def forward(self, x, edge_index, edge_attr):
-        cw, keep = self._weights()
-        dn, de = cw.dn, cw.de
-        if x.shape[1] != 2 * dn or edge_attr.shape[1] != 2 * de:
-            raise NotImplementedError('fused step is built for reattach_initial_nodes/edges = True '
-                                      f'(x [N,{2 * dn}], edge_attr [E,{2 * de}])')
-        layout = ops.edge_layout(edge_index, x.shape[0])
-        e = layout.num_edges
-        ea = ops.gather_rows(edge_attr, layout.slot_edge[:e]) if e else edge_attr
-        e_new, x_new, _ = ops.mp_step(cw, layout, x[:, :dn].contiguous(), x[:, dn:].contiguous(),
-                                      ea[:, :de].contiguous(), ea[:, de:].contiguous(), mode=3)
-        out_e = torch.empty_like(e_new)
-        out_e[layout.slot_edge[:e].long()] = e_new          # back to the caller's edge order
-        del keep
-        return x_new, out_e
+        if self.edge_model is not None:
+            edge_attr = self.edge_model(x, edge_index, edge_attr)
+        if self.node_model is not None:
+            x = self.node_model(x, edge_index, edge_attr)
+        return x, edge_attr
 
     def __repr__(self):
         return '{}(edge_model={}, node_model={})'.format(self.__class__.__name__, self.edge_model, self.node_model)
@@ -454,14 +410,15 @@ class MOTMPNet(nn.Module):
         return self._mask_branch(x_ext, c['lay'], logits, first_class_step, train_ctx=c)
 
     def _core(self, xs, edge_attr, layout, first_needed, want_state=False, encoded=False, pooled=None):
-        """Encoders + step loop.  The tensor-core kernels report fp16-range overflow through one status
-        word that is read once at the end (a single host sync); 'auto' then reruns on the fp32 kernels.
+        """Encoders + step loop.  The tensor-core kernels report fp16-range overflow through one status word per
+        kernel family (mpn_mp_forward_tc clears its own at the start), read once at the end (a single host sync); 'auto'
+        then reruns on the fp32 kernels (``ops.tc_or_fp32``).
         pooled: (the pooled [N, C] node features of ``xs``, event that marks them ready) when the pool already runs
         on another stream; the edge encoder, which does not need them, is enqueued before the wait."""
         engine = self.engine or ops.default_engine()
         cw, keep = self.core_weights()
-        for eng in ((engine,) if engine != 'auto' else ('auto', 'fp32')):
-            status = torch.zeros(2, dtype=torch.int32, device=edge_attr.device) if eng != 'fp32' else None
+
+        def run(eng, status=None):
             e0 = self.encode_edges(edge_attr, layout)
             if encoded:
                 x0 = xs[0] if len(xs) == 1 else torch.cat(xs)
@@ -472,18 +429,13 @@ class MOTMPNet(nn.Module):
                 x0 = self.encode_nodes_list(xs, engine=eng, status=None if status is None else status[0:1])
             res = ops.mp_forward(cw, layout, x0, e0, self.num_enc_steps, first_needed, want_state=want_state,
                                  engine=eng, status=None if status is None else status[1:2])
-            res = res if want_state else (res,)
-            if status is None or not (ops.STRICT_TC_STATUS or eng == 'auto'):
-                break
-            flags = status.tolist()                                    # the one host sync
-            if not any(flags):
-                break
-            if eng == 'tc':
-                raise OverflowError('a value left the fp16 range on the tensor-core path, or the step scale passed the '
-                                    'split operands\' resolution; use engine="fp32"')
-            import warnings
-            warnings.warn('mpntrackseg_b200: value outside the fp16 range (or step scale beyond the split operands\' '
-                          'resolution), rerunning the forward on the fp32 kernels')
+            return res if want_state else (res,)
+
+        res = ops.tc_or_fp32(engine, lambda status: run(engine, status), lambda: run('fp32'),
+                             'a value left the fp16 range on the tensor-core path, or the step scale passed the '
+                             'split operands\' resolution; use engine="fp32"',
+                             'mpntrackseg_b200: value outside the fp16 range (or step scale beyond the split operands\' '
+                             'resolution), rerunning the forward on the fp32 kernels')
         del keep
         return res
 

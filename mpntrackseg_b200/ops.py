@@ -15,10 +15,6 @@ from . import _cabi
 from ._cabi import CoreWeights, EdgeLayout, check, lib, ptr, stream_ptr
 
 
-# engine='tc' also checks the overflow status (one 4-byte device read) unless this is cleared
-STRICT_TC_STATUS = True
-
-
 def _req(t, dtype, name):
     if not torch.is_tensor(t):
         raise TypeError(f'{name}: expected a torch tensor, got {type(t).__name__}')
@@ -31,6 +27,12 @@ def _req(t, dtype, name):
         raise RuntimeError(f'{name}: tensor lives on {t.device} but the current device is cuda:{torch.cuda.current_device()}; '
                            f'call under torch.cuda.device({t.device.index})')
     return t if t.is_contiguous() else t.contiguous()
+
+
+def _ld(t):
+    if t.dim() != 2 or t.stride(1) != 1:
+        raise ValueError('expected a 2-D tensor with unit column stride')
+    return t.stride(0)
 
 
 def _bytes(n, device):
@@ -269,25 +271,27 @@ def node_encoder(x, weights, biases, engine=None, status=None):
     ws_ = [_req(w, torch.float32, 'weight') for w in weights]
     bs_ = [_req(b, torch.float32, 'bias') for b in biases]
     n, k0 = x.shape
-    fits = (len(ws_) == 2 and ws_[0].shape[0] == 128 and ws_[1].shape[0] == 32 and k0 % 64 == 0 and k0 >= 64
-            and x.data_ptr() % 16 == 0)
-    if fits and engine in ('auto', 'tc') and n > 0:
+
+    def tc(st):
         out = torch.empty((n, 32), dtype=torch.float32, device=x.device)
         ws = _bytes(lib().mpn_node_encoder_tc_workspace(k0), x.device)
-        deferred = status is not None
-        if status is None:
-            status = torch.zeros(1, dtype=torch.int32, device=x.device)
         check(lib().mpn_node_encoder_tc(ptr(x), n, k0, ptr(ws_[0]), ptr(bs_[0]), 128, ptr(ws_[1]), ptr(bs_[1]), 32,
-                                        ptr(ws), ptr(out), ptr(status), stream_ptr()), 'node_encoder_tc')
-        if deferred or (engine == 'tc' and not STRICT_TC_STATUS) or int(status.item()) == 0:
-            return out
-        if engine == 'tc':
-            raise OverflowError('node_encoder_tc: non-finite node features or encoder weights; use engine="fp32"')
-        warnings.warn('mpntrackseg_b200: non-finite node features or encoder weights, rerunning the encoder on the fp32 kernels')
-    h = x
-    for w, b in zip(ws_, bs_):
-        h = linear(h, w, b, relu=w.shape[0] != 1)
-    return h
+                                        ptr(ws), ptr(out), ptr(st), stream_ptr()), 'node_encoder_tc')
+        return out
+
+    def fp32():
+        h = x
+        for w, b in zip(ws_, bs_):
+            h = linear(h, w, b, relu=w.shape[0] != 1)
+        return h
+
+    fits = (len(ws_) == 2 and ws_[0].shape[0] == 128 and ws_[1].shape[0] == 32 and k0 % 64 == 0 and k0 >= 64
+            and x.data_ptr() % 16 == 0)
+    if not fits or n == 0:
+        return fp32()
+    return tc_or_fp32(engine, tc, fp32, 'node_encoder_tc: non-finite node features or encoder weights; use engine="fp32"',
+                      'mpntrackseg_b200: non-finite node features or encoder weights, rerunning the encoder on the fp32 kernels',
+                      status=status)
 
 
 def gather_rows(inp, idx):
@@ -297,6 +301,14 @@ def gather_rows(inp, idx):
     out = torch.empty((rows, width), dtype=torch.float32, device=inp.device)
     check(lib().mpn_gather_rows(ptr(inp), ptr(idx), rows, width, ptr(out), stream_ptr()), 'gather_rows')
     return out
+
+
+def segment_sum(inp, in_off, width, seg_ptr, perm, out, col_off, accumulate=False, mode='sum', argmax=None):
+    """out[:, col_off:col_off+width] (+)= the sum / mean / max of each segment; ``argmax`` (int32 [nodes, width], max only)
+    receives the input row of each maximum (-1 for an empty segment)."""
+    check(lib().mpn_segment_reduce(ptr(inp), _ld(inp), in_off, width, ptr(seg_ptr), ptr(perm), out.shape[0],
+                                   int(accumulate), ptr(out), _ld(out), col_off, NODE_AGG[mode], ptr(argmax),
+                                   stream_ptr()), 'segment_sum')
 
 
 def edge_encoder(edge_attr, layout, weights, biases):
@@ -360,6 +372,29 @@ def default_engine():
     return eng
 
 
+def tc_or_fp32(engine, tc, fp32, overflow, rerun, status=None):
+    """The one tensor-core / fp32 policy.  ``tc(status)`` enqueues the tensor-core work, which sets a word of the zeroed
+    int32 device tensor ``status`` (two words: one per kernel family for a caller that runs both) when a value left the
+    fp16 range; ``fp32()`` computes on the fp32 kernels.  engine 'fp32' runs ``fp32()``.  Otherwise a caller's
+    ``status`` is only handed to ``tc`` (the caller reads it: no host sync, no fallback here); without one, the status
+    is read once: all 0 returns the tensor-core result, else engine 'tc' raises OverflowError(overflow) and 'auto'
+    warns ``rerun`` and returns ``fp32()``."""
+    if engine not in ENGINES:
+        raise ValueError(f'engine must be one of {ENGINES}, got {engine!r}')
+    if engine == 'fp32':
+        return fp32()
+    if status is not None:
+        return tc(status)
+    status = torch.zeros(2, dtype=torch.int32, device='cuda')
+    out = tc(status)
+    if status.view(torch.int64).item() == 0:                      # both words in the one host sync
+        return out
+    if engine == 'tc':
+        raise OverflowError(overflow)
+    warnings.warn(rerun)
+    return fp32()
+
+
 LAST_TC_SCHEDULE = {}     # filled by mp_forward(..., debug=True): {'sched': [...], 'amax': [...], 'xmax': [...]} by step
 
 
@@ -384,47 +419,31 @@ def mp_forward(cw, layout, x_init, e_init, num_steps, first_class_step, want_sta
     x_out = torch.empty((n, cw.dn), dtype=torch.float32, device=dev) if want_state else None
     e_out = torch.empty((e, cw.de), dtype=torch.float32, device=dev) if want_state else None
     g = layout.c_struct()
-    use_tc = engine in ('auto', 'tc') and num_steps >= 1 and n > 0
-    if use_tc:
+    result = (logits, x_out, e_out) if want_state else logits
+
+    def tc(st):
         ws = _bytes(lib().mpn_mp_tc_workspace(n, e), dev)
-        deferred = status is not None
-        if status is None:
-            status = torch.zeros(1, dtype=torch.int32, device=dev)
         check(lib().mpn_mp_forward_tc(C.byref(cw), C.byref(g), ptr(x_init), ptr(e_init), int(num_steps), int(first),
-                                      ptr(ws), ptr(logits), ptr(x_out), ptr(e_out), ptr(status), stream_ptr()),
+                                      ptr(ws), ptr(logits), ptr(x_out), ptr(e_out), ptr(st), stream_ptr()),
               'mp_forward_tc')
         if debug:
             hs, ha, hx = (C.c_int32 * (num_steps + 2))(), (C.c_float * (num_steps + 2))(), (C.c_float * (num_steps + 2))()
             check(lib().mpn_mp_tc_read_schedule(ptr(ws), n, e, int(num_steps), hs, ha, hx, stream_ptr()), 'mp_tc_read_schedule')
             LAST_TC_SCHEDULE.update(sched=list(hs), amax=list(ha), xmax=list(hx))
-        if deferred or (engine == 'tc' and not STRICT_TC_STATUS):
-            return (logits, x_out, e_out) if want_state else logits
-        if int(status.item()) == 0:
-            return (logits, x_out, e_out) if want_state else logits
-        if engine == 'tc':
-            raise OverflowError('mp_forward_tc: an activation left the fp16 range, or the step scale passed the split '
-                                'operands\' resolution; use engine="fp32"')
-        warnings.warn('mpntrackseg_b200: activation outside the fp16 range (or step scale beyond the split operands\' '
-                      'resolution), rerunning the message-passing steps on the fp32 kernels')
-    ws = _bytes(lib().mpn_mp_workspace(n, e), dev)
-    check(lib().mpn_mp_forward(C.byref(cw), C.byref(g), ptr(x_init), ptr(e_init), int(num_steps), int(first),
-                               ptr(ws), ptr(logits), ptr(x_out), ptr(e_out), stream_ptr()), 'mp_forward')
-    return (logits, x_out, e_out) if want_state else logits
+        return result
 
+    def fp32():
+        ws = _bytes(lib().mpn_mp_workspace(n, e), dev)
+        check(lib().mpn_mp_forward(C.byref(cw), C.byref(g), ptr(x_init), ptr(e_init), int(num_steps), int(first),
+                                   ptr(ws), ptr(logits), ptr(x_out), ptr(e_out), stream_ptr()), 'mp_forward')
+        return result
 
-def mp_step(cw, layout, x_init, x_lat, e_init, e_lat, mode=3, want_logits=False):
-    """One MetaLayer step on explicit states (edge tensors in slot order).  models/mpn.py:33-54"""
-    n, e, dev = layout.num_nodes, layout.num_edges, x_init.device
-    args = [_req(t, torch.float32, nm) for t, nm in ((x_init, 'x_init'), (x_lat, 'x_lat'),
-                                                      (e_init, 'e_init'), (e_lat, 'e_lat'))]
-    ws = _bytes(lib().mpn_mp_workspace(n, e), dev)
-    e_out = torch.empty((e, cw.de), dtype=torch.float32, device=dev) if mode & 1 else None
-    x_out = torch.empty((n, cw.dn), dtype=torch.float32, device=dev) if mode & 2 else None
-    logits = torch.empty(e, dtype=torch.float32, device=dev) if want_logits else None
-    g = layout.c_struct()
-    check(lib().mpn_mp_step(C.byref(cw), C.byref(g), *[ptr(t) for t in args], int(mode), ptr(ws), ptr(e_out),
-                            ptr(x_out), ptr(logits), stream_ptr()), 'mp_step')
-    return e_out, x_out, logits
+    if num_steps < 1 or n == 0:
+        return fp32()
+    return tc_or_fp32(engine, tc, fp32, 'mp_forward_tc: an activation left the fp16 range, or the step scale passed the '
+                      'split operands\' resolution; use engine="fp32"',
+                      'mpntrackseg_b200: activation outside the fp16 range (or step scale beyond the split operands\' '
+                      'resolution), rerunning the message-passing steps on the fp32 kernels', status=status)
 
 
 def attn_aggregate(z, layout, logits):

@@ -22,15 +22,10 @@ import torch
 
 from . import ops
 from ._cabi import check, lib, ptr, stream_ptr
+from .ops import NODE_AGG, _ld, segment_sum
 
 
 # ------------------------------------------------------------------ thin wrappers
-def _ld(t):
-    if t.dim() != 2 or t.stride(1) != 1:
-        raise ValueError('expected a 2-D tensor with unit column stride')
-    return t.stride(0)
-
-
 def gemm(a, b, ta=False, tb=False, bias=None, relu=False, mask=None, out=None, accumulate=False):
     """out = act(op(a) @ op(b) + bias) (+ out).  mask: a is multiplied by (mask > 0) elementwise."""
     m = a.shape[1] if ta else a.shape[0]
@@ -61,21 +56,10 @@ def gather_cols(src, idx, out, col_off):
                                 stream_ptr()), 'gather_cols')
 
 
-AGG_MODES = {'sum': 0, 'mean': 1, 'max': 2}
-
-
-def segment_sum(inp, in_off, width, seg_ptr, perm, out, col_off, accumulate=False, mode='sum', argmax=None):
-    """out[:, col_off:col_off+width] (+)= the sum / mean / max of each segment; ``argmax`` (int32 [nodes, width], max only)
-    receives the input row of each maximum (-1 for an empty segment)."""
-    check(lib().mpn_segment_reduce(ptr(inp), _ld(inp), in_off, width, ptr(seg_ptr), ptr(perm), out.shape[0],
-                                   int(accumulate), ptr(out), _ld(out), col_off, AGG_MODES[mode], ptr(argmax),
-                                   stream_ptr()), 'segment_sum')
-
-
 def segment_grad(g, row, seg_ptr, argmax, q0, q1, mode, out):
     """out[q] for the slots q in [q0, q1): the gradient of a mean / max ``segment_sum`` (without perm) from ``g``."""
     check(lib().mpn_segment_grad(ptr(g), _ld(g), ptr(row), ptr(seg_ptr), ptr(argmax), q0, q1, out.shape[1],
-                                 AGG_MODES[mode], ptr(out), _ld(out), stream_ptr()), 'segment_grad')
+                                 NODE_AGG[mode], ptr(out), _ld(out), stream_ptr()), 'segment_grad')
 
 
 class _Dropout:
@@ -195,7 +179,7 @@ class CoreTrainer:
         self.model = model
         from .models.mpn import _agg_name
         self.agg = _agg_name(model.MPNet.node_model.node_agg_fn)
-        if self.agg not in AGG_MODES:
+        if self.agg not in NODE_AGG:
             raise NotImplementedError(f'node_agg_fn {self.agg!r}: the training kernels aggregate by sum / mean / max')
         for name, mod in model.named_modules():
             if name.startswith(CORE_PREFIXES) and isinstance(mod, torch.nn.BatchNorm1d) and mod.momentum is None:

@@ -263,7 +263,7 @@ def test_hub_forward_is_deterministic_and_order_invariant(engine):
 
 
 def test_edge_and_node_model_operators_on_hub_graphs():
-    """EdgeModel / TimeAwareNodeModel as standalone operators (fp32 kernels) on the hub graph."""
+    """EdgeModel / TimeAwareNodeModel / MetaLayer as standalone operators (fp32 kernels) on the hub graph."""
     ei, n = hub_graph(HUB_DEGREES, offset=1, seed=12, duplicates=10)
     assert max_direction_degree(ei, n) > ATT_MAX_DEG
     for agg in ('sum', 'mean', 'max'):
@@ -278,8 +278,27 @@ def test_edge_and_node_model_operators_on_hub_graphs():
             x_ref = mpn_ref.node_update(p64(P), x.double(), ei, e_ref, agg)
             e_new = model.MPNet.edge_model(x.to(dev()), ei.to(dev()), ea.to(dev()))
             x_new = model.MPNet.node_model(x.to(dev()), ei.to(dev()), e_ref.float().to(dev()))
+            x_step, e_step = model.MPNet(x.to(dev()), ei.to(dev()), ea.to(dev()))
         assert_rows_close(e_new, e_ref, f'edge_model {agg}')
         assert_rows_close(x_new, x_ref, f'node_model {agg}')
+        assert_rows_close(e_step, e_ref, f'MetaLayer edge {agg}')
+        assert_rows_close(x_step, x_ref, f'MetaLayer node {agg}')
+    # an id >= N, a negative id, a self-loop or an edge_attr of another length raises before anything gathers by them
+    xd, ead, ed = x.to(dev()), ea.to(dev()), e_ref.float().to(dev())
+    for col in (n, -1, int(ei[0, 0])):
+        bad = ei.clone()
+        bad[1, 0] = col
+        bad = bad.to(dev())
+        for call in (lambda: model.MPNet.edge_model(xd, bad, ead), lambda: model.MPNet(xd, bad, ead),
+                     lambda: model.MPNet.node_model(xd, bad, ed)):
+            with torch.no_grad(), pytest.raises(ValueError, match='self-loops or out of range'):
+                call()
+    ei_d = ei.to(dev())
+    for call in (lambda: model.MPNet.edge_model(xd, ei_d, ead[1:]), lambda: model.MPNet(xd, ei_d, ead[1:]),
+                 lambda: model.MPNet.node_model(xd, ei_d, ed[1:])):
+        with torch.no_grad(), pytest.raises(ValueError, match='rows for'):
+            call()
+    torch.cuda.synchronize()
 
 
 # ================================================================== 3. mixed-magnitude batches
@@ -501,7 +520,7 @@ def test_colsum_segment_sum_and_gather_cols_against_fp64():
     for acc in (False, True):
         out0 = torch.randn(lens.numel(), 50, generator=g)
         out = out0.clone().to(dev())
-        training.segment_sum(inp.to(dev()), 4, 33, ptr.to(dev()), perm.to(dev()), out, 9, accumulate=acc)
+        ops.segment_sum(inp.to(dev()), 4, 33, ptr.to(dev()), perm.to(dev()), out, 9, accumulate=acc)
         ref = out0.double().clone()
         seg = torch.repeat_interleave(torch.arange(lens.numel()), lens)
         vals = inp.double()[perm.long(), 4:37]

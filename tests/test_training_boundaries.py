@@ -417,7 +417,7 @@ def segment_case(width, seed, ties=False):
 
 
 def run_segment(v, seg_ptr, perm, in_off, width, mode, accumulate, prev):
-    from mpntrackseg_b200.training import segment_sum
+    from mpntrackseg_b200.ops import segment_sum
     nodes = seg_ptr.numel() - 1
     col_off = 2
     out = torch.full((nodes, width + 4), 7.0, device=dev())
@@ -489,7 +489,8 @@ def test_segment_max_and_argmax_bit_exact(width, permuted, ties):
 def test_segment_grad_of_a_flow_in_slot_range(width):
     """Slots [0, q0) form the flow_out groups, [q0, q1) the flow_in groups (q0 > 0): max sends g to the argmax slot
     exactly, mean divides it by the segment size."""
-    from mpntrackseg_b200.training import segment_grad, segment_sum
+    from mpntrackseg_b200.ops import segment_sum
+    from mpntrackseg_b200.training import segment_grad
     g_ = torch.Generator().manual_seed(9)
     nodes = 6
     out_len, in_len = torch.tensor([2, 0, 3, 1, 1025, 0]), torch.tensor([1, 30000, 0, 2, 3, 1])
